@@ -16,6 +16,7 @@ bounds) and the CUDA-core FFMA mode are measured in the same run and reported un
 `--precision bf16|fp32` makes one of those the headline instead.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16x3|bf16|fp32] [--scaling weak|strong]
+                  [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -193,10 +194,11 @@ def run_reference(args):
     batch = O.make_ppo_batch(o, n_cpu, pool=512, seed=1)
     params = [p.clone() for p in o.actor_ft] + [p.clone() for p in o.critic]
     m = [torch.zeros_like(p) for p in params]; v = [torch.zeros_like(p) for p in params]
+    last_metrics = [None]
 
     def step(i):
         oo = O.Oracle(o.d, o.h, o.actor, params[:12], params[12:])
-        _, ga, gc = oo.ppo_grads(*batch)
+        last_metrics[0], ga, gc = oo.ppo_grads(*batch)
         O.adamw_keras(params, ga + gc, m, v, i + 1, 1e-4, o.h.beta1, o.h.beta2, o.h.adam_eps, o.h.weight_decay)
 
     for i in range(args.warmup):
@@ -206,6 +208,9 @@ def run_reference(args):
         step(args.warmup + i)
     dt = time.perf_counter() - t0
     val = n_cpu * args.steps / dt
+    if args.dump_outputs:
+        save_outputs(args.dump_outputs, {"ppo_metrics": [float(x) for x in last_metrics[0]],
+                                         "actor_ft_weights": O.flatten_params(params[:12]), "critic_weights": O.flatten_params(params[12:])})
     # sampling half of the metric on the CPU, for the "sampling" block
     obs, x_T, noise = O.make_rollout_inputs(o, N_ENVS, seed=3)
     o.sample(obs, x_T, noise)
@@ -260,6 +265,15 @@ def traffic_from_profiles(kernel_key):
     except Exception:
         pass
     return None, None
+
+
+def save_outputs(out_dir, arrays):
+    """--dump-outputs: what the timed PPO update hands its caller, i.e. the 8 metrics of the last timed step and the weights
+    the updates left (fine-tuned actor, critic), as out_dir/<name>.npy in fp32 (about 3 MB).  Weights, batches and seeds
+    are fixed, so two builds run with the same arguments can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def run_ours(args):
@@ -380,10 +394,17 @@ def run_ours(args):
 
     clk = Clocks(local); clk.start()
     dev_step = step_fn(e)
+    last_metrics = [None]
+
+    def timed_step(i):
+        last_metrics[0] = dev_step(i)
     l0 = e.launch_count()
-    ms_dev = timed(dev_step, args.steps, args.warmup)
+    ms_dev = timed(timed_step, args.steps, args.warmup)
     launches = e.launch_count() - l0
     launches_per_step = launches // (args.steps + args.warmup)
+    if args.dump_outputs and rank == 0:
+        save_outputs(args.dump_outputs, {"ppo_metrics": last_metrics[0].cpu().numpy(), "actor_ft_weights": e.get_weights(L.NET_ACTOR_FT),
+                                         "critic_weights": e.get_weights(L.NET_CRITIC)})
 
     # ---- e2e (a): host minibatch through dppo_ppo_step_host (H2D of the 18.6 MB minibatch + D2H of the metrics every step)
     def e2e_host_step(i):
@@ -696,7 +717,11 @@ def main():
                     help="weak: 50 000 rows per GPU; strong: the reference's 50 000-row minibatch (and 4096-row pre-train batch) sharded over the ranks")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-hopper", action="store_true", help="skip the hopper-shape block (configs[0] / [3])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed update's metrics and the weights it left as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
