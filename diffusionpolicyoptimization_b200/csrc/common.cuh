@@ -172,12 +172,9 @@ struct dppo_handle {
     int64_t tc_launches = 0;
     int w0p_dirty[4] = {1, 1, 1, 1};  // ActorDerived::w0p is stale (rebuilt on demand by the FFMA layer-0 GEMM)
     int w23_dirty[4] = {1, 1, 1, 1};     // folded output-layer tables (ActorDerived::w23 / b23) need a rebuild
-    int chain_cg = 2;                 // fused chain kernel: 2 = CTA pairs (tcgen05 cta_group::2), 1 = single CTAs (DPPO_CHAIN_CG=1)
     int peer_two_shot = -1;           // DPPO_PEER_TWO_SHOT=0/1 (default: two-shot from 4 ranks)
     float* peer_gsum[8] = {nullptr};
-    int overlap_chains = 1;           // DPPO_OVERLAP_CHAINS=0: actor and critic chains back to back on one stream
     cudaStream_t aux_stream = nullptr; cudaEvent_t aux_ev[3] = {nullptr, nullptr, nullptr};
-    int dw_pair = 1;                  // DPPO_DW_PAIR=0: weight-gradient GEMM on single CTAs instead of CTA pairs
     float grad_clip_norm = 0.f;       // dppo_set_grad_clip_norm: per-variable tf.clip_by_norm before AdamW (<= 0: off)
     int deterministic = 0;            // DPPO_DETERMINISTIC=1: fixed-order split-K reductions instead of red.global.add
     int chain_dbg_idx = 0;

@@ -265,9 +265,6 @@ static int dppo_create_impl(const dppo_cfg* cfg, int device, dppo_handle** out, 
     { const char* tv = getenv("DPPO_PEER_TIMEOUT_S"); double sec = tv ? atof(tv) : 600.0; if (!(sec > 0)) sec = 600.0;
       h->peer_timeout_cycles = (long long)(sec * 1e3 * (double)prop.clockRate); }
     { const char* dv = getenv("DPPO_DETERMINISTIC"); h->deterministic = (dv && dv[0] == '1') ? 1 : 0; }
-    { const char* cv = getenv("DPPO_CHAIN_CG"); h->chain_cg = (cv && cv[0] == '1') ? 1 : 2; }
-    { const char* pv = getenv("DPPO_DW_PAIR"); h->dw_pair = (pv && pv[0] == '0') ? 0 : 1; }
-    { const char* ov = getenv("DPPO_OVERLAP_CHAINS"); h->overlap_chains = (ov && ov[0] == '0') ? 0 : 1; }
     const size_t nA = g.ao.n, nC = g.co.n;
     const size_t total = 3 * nA + nC;
     CUDA_TRY(cudaMalloc(&h->params, total * sizeof(float)));
@@ -1083,10 +1080,7 @@ extern "C" int dppo_ppo_step_host(dppo_handle* h, const float* obs, const float*
     int* d_inds = (int*)p; p += b_n; float* d_ret = (float*)p; p += b_n; float* d_val = (float*)p; p += b_n; float* d_adv = (float*)p; p += b_n;
     float* d_met = (float*)p;
     // tensor mode: chunked pipeline - the H2D copy of chunk c+1 (copy stream) overlaps the compute of chunk c
-    int chunk_rows = (tc_eligible(h, N) && fc_ok(h) && fc_critic_ok(h) && !h->deterministic) ? tc_ppo_pipeline_chunk_rows(h, N) : 0;
-    static int env_chunk = -2, env_lead = -2;          // dev knobs: DPPO_HOST_CHUNK_ROWS (0 = no pipeline), DPPO_HOST_LEAD_ROWS
-    if (env_chunk == -2) { const char* v = getenv("DPPO_HOST_CHUNK_ROWS"); env_chunk = v ? atoi(v) : -1; const char* l = getenv("DPPO_HOST_LEAD_ROWS"); env_lead = l ? atoi(l) : -1; }
-    if (chunk_rows > 0 && env_chunk >= 0) chunk_rows = env_chunk >= N ? 0 : env_chunk;
+    const int chunk_rows = (tc_eligible(h, N) && fc_ok(h) && fc_critic_ok(h) && !h->deterministic) ? tc_ppo_pipeline_chunk_rows(h, N) : 0;
     if (chunk_rows > 0) {
         if (!obs || !prev || !nxt || !inds || !returns || !oldvalues || !advantages || !oldlogp || N_global < N) DPPO_FAIL(-1, "dppo_ppo_step_host: bad arguments");
         if (adv_std < 0.f && N_global != N) DPPO_FAIL(-1, "dppo_ppo_step_host: global advantage statistics are required when rows are sharded");
@@ -1099,7 +1093,7 @@ extern "C" int dppo_ppo_step_host(dppo_handle* h, const float* obs, const float*
         CUDA_TRY(cudaEventRecord(h->copy_ev[8], s));
         CUDA_TRY(cudaStreamWaitEvent(cs, h->copy_ev[8], 0));
         // a short first chunk (a third of a wave-sized one) gets the GPU going while the bulk of the minibatch is still on the link
-        const int lead = env_lead >= 0 ? (env_lead & ~127) : (((chunk_rows / 3) + 127) & ~127);
+        const int lead = ((chunk_rows / 3) + 127) & ~127;
         DPPO_TRY(tc_ppo_begin(h, s, N, chunk_rows, N_global, lead));
         const int CR = tc_plan(h).chunk_rows, nchunks = tc_plan(h).nchunks;
         if (nchunks > 8) DPPO_FAIL(-7, "dppo_ppo_step_host: too many pipeline chunks");
@@ -1330,7 +1324,7 @@ extern "C" int dppo_debug_mma_probe(dppo_handle* h, int grid, int mode, int iter
     CUDA_TRY(cudaSetDevice(h->device));
     if (!tc_shapes_ok(h)) DPPO_FAIL(-7, "tensor path unavailable");
     CUtensorMap wm;
-    DPPO_TRY(fc::weight_map(&wm, h->tc->net[DPPO_NET_ACTOR].w1, h->g.H, h->g.H, h->g.H, 1));
+    DPPO_TRY(tc::make_map(&wm, h->tc->net[DPPO_NET_ACTOR].w1, h->g.H, h->g.H, h->g.H, fc::WK, 64));      // four [32 k][64 n] boxes fill one 16 KB probe stage
     long long* d = nullptr;
     CUDA_TRY(cudaMalloc(&d, (size_t)grid * 2 * sizeof(long long)));
     CUDA_TRY(cudaMemset(d, 0, (size_t)grid * 2 * sizeof(long long)));

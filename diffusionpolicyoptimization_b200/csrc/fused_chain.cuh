@@ -1,6 +1,5 @@
-// Fused residual-MLP layer chain on tcgen05 (sm_100a).  A persistent CTA PAIR (cluster of 2, cta_group::2; CG = 1 is
-// the single-CTA variant) walks 256-row tiles - 128 rows per CTA - and runs EVERY layer of the chain for its tile with
-// the activations resident on chip.
+// Fused residual-MLP layer chain on tcgen05 (sm_100a).  A persistent CTA PAIR (cluster of 2, cta_group::2) walks
+// 256-row tiles - 128 rows per CTA - and runs EVERY layer of the chain for its tile with the activations resident on chip.
 //
 //   shared memory  X   [128][H] bf16   the current activation, stored as H/64 K-major 128B-swizzled tiles
 //   (per CTA)                          (exactly the image TMA would produce), i.e. directly the A operand
@@ -10,7 +9,7 @@
 //                  H0  [128][64] bf16  the packed layer-0 input tile [x | obs | onehot(t) | 1 | 0]
 //                                      (TMA-loaded, or rebuilt in place by the sampler every denoising step)
 //                  W   4 x 16 KB ring  this CTA's half of every weight tile: [64 k][128 n] (MN-major, TMA from L2);
-//                                      the pair's MMA reads both halves ([32 k][256 n] per stage when CG = 1)
+//                                      the pair's MMA reads both halves
 //   tensor memory  512 columns         the whole [128][H] fp32 accumulator of one layer
 //
 //   warp 0     TMA producer (weight ring, H0 / gate tiles); loads report to the LEADER CTA's mbarriers
@@ -257,10 +256,10 @@ __device__ __forceinline__ void build_h0_half(uint32_t h0_addr, int rloc, int ha
     }
 }
 
-template <int H, bool TIMING, int CG>
+template <int H, bool TIMING>
 __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constant__ Maps maps, const Params p) {
     constexpr int XT = H / 64;
-    constexpr int WKE = WK * CG;                                // k-rows per ring stage: a stage is [WKE][256 / CG] = 16 KB per CTA
+    constexpr int WKE = WK * 2;                                 // k-rows per ring stage: a stage is [WKE][128] = 16 KB per CTA
     constexpr int MPS = WKE / 16;                               // tcgen05.mma (K = 16) per stage
     constexpr int X_BYTES = XT * 16384;
     extern __shared__ uint8_t smem_raw[];
@@ -285,33 +284,28 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int ntiles = (p.rows + FBM - 1) / FBM;
-    const uint32_t rank = CG == 2 ? cluster_ctarank() : 0u;     // rank inside the CTA pair (leader = 0)
-    const int pair0 = blockIdx.x / CG, npairs = gridDim.x / CG, ptiles = (ntiles + CG - 1) / CG;
+    const uint32_t rank = cluster_ctarank();                     // rank inside the CTA pair (leader = 0)
+    const int pair0 = blockIdx.x / 2, npairs = gridDim.x / 2, ptiles = (ntiles + 1) / 2;
     const bool sampler = p.final_mode == FINAL_SAMPLE;
     const int nsteps = sampler ? p.T : 1;
 
     if (warp == 0 && lane == 0) {
         for (int i = 0; i < NMAPS; ++i) tma_prefetch_desc(&maps.m[i]);
-        for (int i = 0; i < NSTAGE; ++i) { mbar_init(&w_full[i], CG); mbar_init(&w_empty[i], 1); }
-        mbar_init(h0_full, CG); mbar_init(h0_empty, 1);
-        mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1); mbar_init(&xready[0], 8 * CG); mbar_init(&xready[1], 8 * CG);
+        for (int i = 0; i < NSTAGE; ++i) { mbar_init(&w_full[i], 2); mbar_init(&w_empty[i], 1); }
+        mbar_init(h0_full, 2); mbar_init(h0_empty, 1);
+        mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1); mbar_init(&xready[0], 16); mbar_init(&xready[1], 16);
         for (int i = 0; i < 4; ++i) mbar_init(&xfree[i], 1);
         mbar_init(g_full, 1); mbar_init(g_empty, 8);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (CG == 2) cluster_sync_all();                            // barriers of both CTAs initialised before anything remote
+    cluster_sync_all();                                         // barriers of both CTAs initialised before anything remote
     if (warp == 1) {
-        if (CG == 1) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     tcgen05_fence_before();
     __syncthreads();
-    if (CG == 2) cluster_sync_all();
+    cluster_sync_all();
     tcgen05_fence_after();
     const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);    // warp-uniform for the compiler
 
@@ -324,17 +318,12 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
             const uint32_t w_addr = smem_u32(sW);
             const uint32_t wfull_addr = smem_u32(w_full), wempty_addr = smem_u32(w_empty);
             for (int pt = pair0; pt < ptiles; pt += npairs) {
-                const int tile = pt * CG + (int)rank;
+                const int tile = pt * 2 + (int)rank;
                 if (p.h0_from_tma) {
                     mbar_wait(h0_empty, h0_phase ^ 1);
-                    if (elect_one()) {
-                        if (CG == 1) {
-                            mbar_expect_tx(h0_full, H0_BYTES);
-                            tma_load_2d(sH0, &maps.m[0], h0_full, 0, tile * FBM);
-                        } else {   // own rows, but the arrival and the bytes go to the leader's barrier
-                            mbar_expect_tx_cluster(mapa_rank0(smem_u32(h0_full)), H0_BYTES);
-                            tma_load_2d_pair(smem_u32(sH0), &maps.m[0], smem_u32(h0_full), 0, tile * FBM);
-                        }
+                    if (elect_one()) {   // own rows, but the arrival and the bytes go to the leader's barrier
+                        mbar_expect_tx_cluster(mapa_rank0(smem_u32(h0_full)), H0_BYTES);
+                        tma_load_2d_pair(smem_u32(sH0), &maps.m[0], smem_u32(h0_full), 0, tile * FBM);
                     }
                     __syncwarp();
                     h0_phase ^= 1;
@@ -346,7 +335,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                         const int n_cur = L.n < 256 ? L.n : 256, nhc = L.n / n_cur;
                         const int kx = L.a_src >= 1 ? H / WKE : 0, kh = L.a_src != 1 ? 64 / WKE : 0;
                         const CUtensorMap* wm = &maps.m[L.wmap];
-                        const int n_mine = n_cur / CG;                     // this CTA's share of the B tile's columns
+                        const int n_mine = n_cur / 2;                      // this CTA's share of the B tile's columns
                         const uint32_t tx = (uint32_t)(WKE * n_mine * 2);
                         const int nbox = n_mine / 64;
                         if (HASG && L.gate_load_map >= 0) {
@@ -368,13 +357,8 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                                 else mbar_wait_addr(wempty_addr + stage * 8, phase ^ 1);
                                 if (elect_one()) {
                                     const uint32_t dst = w_addr + stage * STAGE_BYTES;
-                                    if (CG == 1) {
-                                        mbar_expect_tx_addr(full_bar, tx);
-                                        for (int j = 0; j < nbox; ++j) tma_load_2d_addr(dst + j * (WKE * 128), wm, full_bar, col + j * 64, krow);
-                                    } else {
-                                        mbar_expect_tx_cluster(mapa_rank0(full_bar), tx);
-                                        for (int j = 0; j < nbox; ++j) tma_load_2d_pair(dst + j * (WKE * 128), wm, full_bar, col + j * 64, krow);
-                                    }
+                                    mbar_expect_tx_cluster(mapa_rank0(full_bar), tx);
+                                    for (int j = 0; j < nbox; ++j) tma_load_2d_pair(dst + j * (WKE * 128), wm, full_bar, col + j * 64, krow);
                                 }
                                 __syncwarp();
                                 krow += WKE;
@@ -408,7 +392,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                         const Layer& L = p.L[net][l];
                         const int n_cur = L.n < 256 ? L.n : 256, nhc = L.n / n_cur;
                         const int kx = L.a_src >= 1 ? H / WKE : 0, kh = L.a_src != 1 ? 64 / WKE : 0;
-                        const uint32_t idesc = make_idesc(FBM * CG, n_cur, false, true);
+                        const uint32_t idesc = make_idesc(FBM * 2, n_cur, false, true);
                         const bool h0_rel = L.h0_last && p.h0_from_tma;
                         // xready[0]: the previous epilogue wrote X tiles [0, XT/2) (or H0) and drained the first accumulator half;
                         // xready[1]: tiles [XT/2, XT) and the second half.  The second wait is deferred to the first stage that needs it.
@@ -423,7 +407,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                             uint32_t accf = 0u;
                             uint32_t a_lo = kx ? a_lo_x : a_lo_h0;
                             if (last_half_of_two && kx == 0) {            // this layer never reads X: the epilogue may overwrite it at once
-                                if (elect_one()) { for (int j = 0; j < XT / 2; ++j) { if (CG == 1) tcgen05_commit(&xfree[j]); else tcgen05_commit_pair(smem_u32(&xfree[j])); } }
+                                if (elect_one()) { for (int j = 0; j < XT / 2; ++j) tcgen05_commit_pair(smem_u32(&xfree[j])); }
                                 __syncwarp();
                             }
                             for (int s = 0; s < kx + kh; ++s) {
@@ -437,35 +421,26 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                                 tcgen05_fence_after();
                                 const uint32_t b_lo = b_lo_0 + (uint32_t)stage * (STAGE_BYTES >> 4);
                                 // the stage that finishes X tile j (j < XT/2) in the last n-half frees it for the epilogue
-                                const bool free_tile = last_half_of_two && s < S_HALF && s < kx && (CG == 2 || (s & 1));
-                                const int tile_j = CG == 2 ? s : (s >> 1);
+                                const bool free_tile = last_half_of_two && s < S_HALF && s < kx;
                                 if (elect_one()) {
-                                    if (CG == 1) {
-                                        umma_bf16_split(tmem_d, a_lo, b_lo, desc_hi, idesc, accf);
-                                        umma_bf16_split(tmem_d, a_lo + 2u, b_lo + (2048u >> 4), desc_hi, idesc, 1u);
-                                        tcgen05_commit_addr(wempty_addr + stage * 8);
-                                        if (free_tile) tcgen05_commit(&xfree[tile_j]);
-                                    } else {
-                                        umma_bf16_split_pair(tmem_d, a_lo, b_lo, desc_hi, idesc, accf);
-                                        umma_bf16_split_pair(tmem_d, a_lo + 2u, b_lo + (2048u >> 4), desc_hi, idesc, 1u);
-                                        umma_bf16_split_pair(tmem_d, a_lo + 4u, b_lo + (4096u >> 4), desc_hi, idesc, 1u);
-                                        umma_bf16_split_pair(tmem_d, a_lo + 6u, b_lo + (6144u >> 4), desc_hi, idesc, 1u);
-                                        tcgen05_commit_pair(wempty_addr + stage * 8);
-                                        if (free_tile) tcgen05_commit_pair(smem_u32(&xfree[tile_j]));
-                                    }
+                                    umma_bf16_split_pair(tmem_d, a_lo, b_lo, desc_hi, idesc, accf);
+                                    umma_bf16_split_pair(tmem_d, a_lo + 2u, b_lo + (2048u >> 4), desc_hi, idesc, 1u);
+                                    umma_bf16_split_pair(tmem_d, a_lo + 4u, b_lo + (4096u >> 4), desc_hi, idesc, 1u);
+                                    umma_bf16_split_pair(tmem_d, a_lo + 6u, b_lo + (6144u >> 4), desc_hi, idesc, 1u);
+                                    tcgen05_commit_pair(wempty_addr + stage * 8);
+                                    if (free_tile) tcgen05_commit_pair(smem_u32(&xfree[s]));
                                 }
                                 __syncwarp();
                                 accf = 1u;
-                                // CG = 1: next 32 columns of A (+64 B inside a 128-byte row, then the next 64-column tile); CG = 2: next tile
-                                if (CG == 1) a_lo += (s & 1) ? (16384u >> 4) - 4u : 4u; else a_lo += (16384u >> 4);
+                                a_lo += (16384u >> 4);                            // next 64-column tile of A
                                 if (++stage == NSTAGE) { stage = 0; phase ^= 1; }
                             }
-                            if (elect_one()) { if (CG == 1) tcgen05_commit(&acc_full[nh]); else tcgen05_commit_pair(smem_u32(&acc_full[nh])); }
+                            if (elect_one()) tcgen05_commit_pair(smem_u32(&acc_full[nh]));
                             __syncwarp();
                         }
                         if (!xr1_waited) mbar_wait(&xready[1], xr_phase);
                         xr_phase ^= 1;
-                        if (h0_rel) { if (elect_one()) { if (CG == 1) tcgen05_commit(h0_empty); else tcgen05_commit_pair(smem_u32(h0_empty)); } __syncwarp(); }
+                        if (h0_rel) { if (elect_one()) tcgen05_commit_pair(smem_u32(h0_empty)); __syncwarp(); }
                     }
                 }
             }
@@ -481,9 +456,8 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
         const bool store_thread = (warp == 2 && lane == 0);
         uint32_t gfull_phase = 0;
         // xready lives in the leader CTA: its MMA warp needs both CTAs' epilogues
-        const uint32_t xr0 = CG == 2 ? mapa_rank0(smem_u32(&xready[0])) : smem_u32(&xready[0]);
-        const uint32_t xr1 = CG == 2 ? mapa_rank0(smem_u32(&xready[1])) : smem_u32(&xready[1]);
-        auto arrive_xr = [&](uint32_t a) { if (CG == 2) mbar_arrive_cluster(a); else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a) : "memory"); };
+        const uint32_t xr0 = mapa_rank0(smem_u32(&xready[0]));
+        const uint32_t xr1 = mapa_rank0(smem_u32(&xready[1]));
         const int etid = threadIdx.x - 64;                       // 0..255
         uint32_t acc_phase[2] = {0u, 0u}, xf_phase = 0u;
         int bias_buf = 0;
@@ -495,7 +469,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
         float csum[2][2] = {};                                   // column sums: thread etid (< H/2) owns columns 2*etid, 2*etid+1
         long long t_acc = 0, t_gen = 0, t_fin = 0;
         for (int pt = pair0; pt < ptiles; pt += npairs) {
-            const int tile = pt * CG + (int)rank;
+            const int tile = pt * 2 + (int)rank;
             const int row = tile * FBM + rloc;
             const bool valid = row < p.rows;
             const float* obs_row = p.obs + (size_t)(valid ? row : 0) * p.Do;
@@ -520,9 +494,9 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                 build_h0_half(h0_addr, rloc, half, x, obs_row, A, p.Do, p.T, p.T - 1, valid);
                 fence_async_smem();
                 __syncwarp();
-                if (lane == 0) { arrive_xr(xr0); arrive_xr(xr1); }
+                if (lane == 0) { mbar_arrive_cluster(xr0); mbar_arrive_cluster(xr1); }
             } else if (first) {
-                if (lane == 0) { arrive_xr(xr0); arrive_xr(xr1); }   // "TMEM is free" for the very first layer
+                if (lane == 0) { mbar_arrive_cluster(xr0); mbar_arrive_cluster(xr1); }   // "TMEM is free" for the very first layer
             }
             first = false;
             for (int step = 0; step < nsteps; ++step) {
@@ -735,7 +709,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                                 tma_store_commit();
                             }
                             __syncwarp();
-                            if (lane == 0) { arrive_xr((two_half && hph == 1) ? xr1 : xr0); if (!two_half) arrive_xr(xr1); }
+                            if (lane == 0) { mbar_arrive_cluster((two_half && hph == 1) ? xr1 : xr0); if (!two_half) mbar_arrive_cluster(xr1); }
                         }
                         if (two_half) xf_phase ^= 1;
                         if (L.colsum_slot >= 0) {
@@ -765,7 +739,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                         tmem_ld16(tmem_base + lane_base + (uint32_t)(half * 16), r);
                         tcgen05_fence_before();
                         // eps / log-prob modes touch neither X nor H0 from here on: hand TMEM back before the math
-                        if (!sampler) { __syncwarp(); if (lane == 0) { arrive_xr(xr0); arrive_xr(xr1); } }
+                        if (!sampler) { __syncwarp(); if (lane == 0) { mbar_arrive_cluster(xr0); mbar_arrive_cluster(xr1); } }
                         epi_barrier();                                  // sb (bias) visible
                         const int abase = half * 16;
                         float eps[16];
@@ -826,7 +800,7 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
                         }
                         __syncwarp();
                         // the sampler's last step hands over to the next tile's prologue instead
-                        if (lane == 0 && sampler && step + 1 < nsteps) { arrive_xr(xr0); arrive_xr(xr1); }
+                        if (lane == 0 && sampler && step + 1 < nsteps) { mbar_arrive_cluster(xr0); mbar_arrive_cluster(xr1); }
                         if (TIMING) t_fin += clock64() - c_epi;
                     }
                 }
@@ -841,50 +815,44 @@ __global__ void __launch_bounds__(FTHREADS, 1) chain_kernel(const __grid_constan
     }
     tcgen05_fence_before();
     __syncthreads();
-    if (CG == 2) cluster_sync_all();        // the peer may still be signalling our barriers / reading our B halves
+    cluster_sync_all();                     // the peer may still be signalling our barriers / reading our B halves
     if (warp == 1) {
         tcgen05_fence_after();
-        if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
     }
 }
 
 // ------------------------------------------------------------------ host side
-// weight operand [K][N] bf16 row-major (leading dimension ld): box [WK * cg k][64 n]
-static int weight_map(CUtensorMap* m, const void* base, uint64_t K, uint64_t N, uint64_t ld, int cg) { return make_map(m, base, K, N, ld, WK * cg, 64); }
+// weight operand [K][N] bf16 row-major (leading dimension ld): box [2 WK k][64 n]
+static int weight_map(CUtensorMap* m, const void* base, uint64_t K, uint64_t N, uint64_t ld) { return make_map(m, base, K, N, ld, WK * 2, 64); }
 // row tile source / destination [rows][cols] bf16 row-major: box [128 rows][64 cols]
 static int rowtile_map(CUtensorMap* m, const void* base, uint64_t rows, uint64_t cols) { return make_map(m, base, rows, cols, cols, FBM, 64); }
 
-// number of CTAs a chain launch uses (cg = 2: CTA pairs, an even grid)
-static int chain_grid(const dppo_handle* h, int rows, int cg) {
+// number of CTAs a chain launch uses (CTA pairs: an even grid)
+static int chain_grid(const dppo_handle* h, int rows) {
     const int ntiles = (rows + FBM - 1) / FBM;
-    if (cg == 1) return ntiles < h->sm_count ? ntiles : h->sm_count;
     const int pairs = (ntiles + 1) / 2, maxp = h->sm_count / 2;
     return 2 * (pairs < maxp ? pairs : maxp);
 }
 
-template <int H, int CG>
+template <int H>
 static int launch_chain_t(dppo_handle* h, cudaStream_t s, const Maps& maps, const Params& p, double flops) {
-    auto kern = p.dbg ? chain_kernel<H, true, CG> : chain_kernel<H, false, CG>;
+    auto kern = p.dbg ? chain_kernel<H, true> : chain_kernel<H, false>;
     static bool attr_set_dev[64] = {};      // function attributes are per device
     bool& attr_set = attr_set_dev[h->device & 63];
     if (!attr_set) {
-        CUDA_TRY(cudaFuncSetAttribute(chain_kernel<H, true, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem_bytes<H>()));
-        CUDA_TRY(cudaFuncSetAttribute(chain_kernel<H, false, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem_bytes<H>()));
+        CUDA_TRY(cudaFuncSetAttribute(chain_kernel<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem_bytes<H>()));
+        CUDA_TRY(cudaFuncSetAttribute(chain_kernel<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem_bytes<H>()));
         attr_set = true;
     }
-    const int grid = chain_grid(h, p.rows, CG);
+    const int grid = chain_grid(h, p.rows);
     prof_begin(h, s);
-    if (CG == 1) {
-        kern<<<grid, FTHREADS, chain_smem_bytes<H>(), s>>>(maps, p);
-    } else {
-        cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1; cfg.blockDim = dim3(FTHREADS); cfg.gridDim = dim3(grid); cfg.dynamicSmemBytes = chain_smem_bytes<H>(); cfg.stream = s;
-        cudaError_t le = cudaLaunchKernelEx(&cfg, kern, maps, p);
-        if (le != cudaSuccess) DPPO_FAIL(-3, "fused chain (CTA pair) launch failed: %s", cudaGetErrorString(le));
-    }
+    cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1; cfg.blockDim = dim3(FTHREADS); cfg.gridDim = dim3(grid); cfg.dynamicSmemBytes = chain_smem_bytes<H>(); cfg.stream = s;
+    cudaError_t le = cudaLaunchKernelEx(&cfg, kern, maps, p);
+    if (le != cudaSuccess) DPPO_FAIL(-3, "fused chain (CTA pair) launch failed: %s", cudaGetErrorString(le));
     prof_end(h, s, flops, H == 512 ? 0 : 3);      // the two instantiations are different kernels: time them separately
     h->launches++; h->tc_launches++; h->fused_launches++;
     cudaError_t e = cudaGetLastError();
@@ -892,9 +860,8 @@ static int launch_chain_t(dppo_handle* h, cudaStream_t s, const Maps& maps, cons
     return 0;
 }
 static int launch_chain(dppo_handle* h, cudaStream_t s, int H, const Maps& maps, const Params& p, double flops) {
-    const int cg = h->chain_cg;
-    if (H == 512) return cg == 2 ? launch_chain_t<512, 2>(h, s, maps, p, flops) : launch_chain_t<512, 1>(h, s, maps, p, flops);
-    if (H == 256) return cg == 2 ? launch_chain_t<256, 2>(h, s, maps, p, flops) : launch_chain_t<256, 1>(h, s, maps, p, flops);
+    if (H == 512) return launch_chain_t<512>(h, s, maps, p, flops);
+    if (H == 256) return launch_chain_t<256>(h, s, maps, p, flops);
     DPPO_FAIL(-7, "fused chain: unsupported hidden width %d", H);
 }
 

@@ -1,11 +1,13 @@
 // Grouped weight-gradient GEMM on CTA pairs (cta_group::2):  out_p[M_p][N_p] += X_p^T D_p  for up to 10 problems, ONE launch.
 //
-// Same contract as tc::dw_group_kernel (tc_gemm.cuh): all problems reduce over the same rows, X_p [rows][M_p] and
-// D_p [rows][N_p] are bf16 row-major (both operands MN-major), partial tiles are accumulated with red.global.add.
-// What changes is the tile: a CTA pair owns a 256 x 256 (or 256 x 128) output tile.  Each CTA stages its own 128 columns
-// of X and only HALF of the D tile per 64-row k-block (32 KB instead of the 48 KB of a lone 128 x 256 CTA), the leader issues
-// 256-row tcgen05.mma that read the two D halves from both CTAs' shared memory.  The single-CTA kernel sits at the
-// ~34 B/cycle/SM TMA ingest limit (DESIGN.md 5.2: 96 B/cycle wanted); the pair needs 64 B/cycle for the same MMA rate.
+// All problems reduce over the same rows (K = rows of the chunk); X_p [rows][M_p] and D_p [rows][N_p] are bf16 row-major
+// (both operands MN-major).  Every CTA pair takes (output tile, K split) work items from a flat list; the number of splits
+// per problem is chosen on the host so that the items have equal cost and fill the SMs once.  Partial tiles are accumulated
+// with red.global.add (outputs zeroed by the caller).
+// A CTA pair owns a 256 x 256 (or 256 x 128) output tile.  Each CTA stages its own 128 columns of X and only HALF of the
+// D tile per 64-row k-block (32 KB instead of the 48 KB of a lone 128 x 256 CTA), the leader issues 256-row tcgen05.mma
+// that read the two D halves from both CTAs' shared memory.  A single CTA sits at the ~34 B/cycle/SM TMA ingest limit
+// (DESIGN.md 5.2: 96 B/cycle wanted); the pair needs 64 B/cycle for the same MMA rate.
 //
 // Narrow problems are given with the wide operand as X: the layer-0 products h0^T du / h0^T dv arrive as du^T h0
 // (M = H, N = 64) and are written transposed.  N = 64 problems run as N = 128 (the second CTA's half is out of bounds and
@@ -15,7 +17,8 @@
 
 namespace tcp {
 using namespace tc;
-constexpr int PSTAGES = 6, PBK = 64;
+constexpr int GMAX = 10, PSTAGES = 6, PBK = 64;
+struct GroupMaps { CUtensorMap a[GMAX]; CUtensorMap b[GMAX]; };
 constexpr int PA_STAGE = 128 * PBK * 2, PB_STAGE = 128 * PBK * 2;     // per CTA: 128 X columns, <= 128 D columns
 struct PairProb {
     int m_blocks, n_blocks;           // 256-row output blocks; 256-column (or 128-column) blocks
@@ -181,19 +184,14 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dw_pair_kernel(const __grid_co
 // one problem: out += X^T D with X [rows][M], D [rows][Nd]; transposed: out[n][m] (ld_out = row length of that layout)
 struct PairDesc { const __nv_bfloat16* X; int M; const __nv_bfloat16* D; int Nd; float* out; int M_valid, N_valid, ld_out, transposed; double alg_flops; };
 
-static bool pair_ok(const dppo_handle* h, const PairDesc* d, int n) {
-    if (h->sm_count < 2 || n < 1 || n > GMAX) return false;
-    for (int i = 0; i < n; ++i) if (d[i].M % 64 || d[i].Nd % 64) return false;
-    return true;
-}
-
 static int launch_group_pair(dppo_handle* h, cudaStream_t s, const PairDesc* d, int n, int rows) {
+    if (h->sm_count < 2 || n < 1 || n > GMAX) DPPO_FAIL(-1, "launch_group_pair: bad problem count %d", n);
+    for (int i = 0; i < n; ++i) if (d[i].M % 64 || d[i].Nd % 64) DPPO_FAIL(-7, "launch_group_pair: operand widths must be multiples of 64");
     GroupMaps maps; PairParams gp; memset(&gp, 0, sizeof(gp));
     gp.nprob = n; gp.kblocks = (rows + PBK - 1) / PBK;
     const int npairs = h->sm_count / 2;
     double w[GMAX]; int tiles[GMAX];
-    static double w128 = -1.0;                 // relative k-block time of a 128-wide tile (24 KB staged per CTA vs 32 KB)
-    if (w128 < 0) { const char* e = getenv("DPPO_DW_W128"); w128 = e ? atof(e) : 0.75; if (!(w128 > 0.1 && w128 <= 1.0)) w128 = 0.75; }
+    const double w128 = 0.75;                  // relative k-block time of a 128-wide tile (24 KB staged per CTA vs 32 KB)
     for (int i = 0; i < n; ++i) {
         PairProb& P = gp.p[i];
         DPPO_TRY(make_map(&maps.a[i], d[i].X, rows, d[i].M, d[i].M, PBK, 64));

@@ -483,193 +483,3 @@ static int launch(dppo_handle* h, cudaStream_t s, const Gemm& g) {
 
 }  // namespace tc
 
-// =====================================================================================
-// Grouped weight-gradient GEMM:  out_p[M_p][N_p] += X_p^T D_p  for up to 10 problems in ONE launch.
-// All problems reduce over the same rows (K = rows of the chunk); X_p [rows][M_p] and D_p [rows][N_p] are bf16
-// row-major, i.e. both operands are MN-major.  Every CTA takes (output tile, K split) work items from a flat list;
-// the number of splits per problem is chosen on the host so that the items have equal cost and fill the SMs once.
-// Partial tiles are accumulated with red.global.add.v4.f32 (outputs zeroed by the caller).
-// =====================================================================================
-namespace tc {
-constexpr int GMAX = 10, GBK = 64, GSTAGES = 4;
-struct GroupProb {
-    int m_blocks, n_boxes;            // output tile rows = 128 * m_blocks; B tile = n_boxes x 64 columns (<= 4), one n-block
-    int n_blocks;                     // number of 256-wide (or n_boxes*64-wide) column blocks
-    int splits, kb_per_split;         // K split (in 64-row blocks)
-    int item_begin;                   // prefix sum of work items
-    int M_valid, N_valid, ld_out;
-    float* out;
-};
-struct GroupParams { int nprob, items, kblocks; GroupProb p[GMAX]; };
-struct GroupMaps { CUtensorMap a[GMAX]; CUtensorMap b[GMAX]; };
-
-__global__ void __launch_bounds__(NUM_THREADS, 1) dw_group_kernel(const __grid_constant__ GroupMaps maps, const GroupParams gp) {
-    constexpr int A_STAGE = BM * GBK * 2, B_STAGE = 256 * GBK * 2;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* sA = smem;
-    uint8_t* sB = smem + GSTAGES * A_STAGE;
-    uint64_t* bars = (uint64_t*)(smem + GSTAGES * (A_STAGE + B_STAGE));
-    uint64_t* full = bars; uint64_t* empty = bars + GSTAGES; uint64_t* tfull = bars + 2 * GSTAGES; uint64_t* tempty = tfull + 2;
-    uint32_t* tmem_slot = (uint32_t*)(tempty + 2);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp == 0 && lane == 0) {
-        for (int i = 0; i < GSTAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(&tfull[i], 1); mbar_init(&tempty[i], 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
-
-    // decode a work item -> (problem, m block, n block, split)
-    auto decode = [&](int item, int& pi, int& m_blk, int& n_blk, int& split) {
-        pi = 0;
-        while (pi + 1 < gp.nprob && item >= gp.p[pi + 1].item_begin) ++pi;
-        const GroupProb& P = gp.p[pi];
-        const int local = item - P.item_begin, per = P.m_blocks * P.n_blocks;
-        split = local / per; const int rem = local % per;
-        m_blk = rem / P.n_blocks; n_blk = rem % P.n_blocks;
-    };
-
-    if (warp == 0) {
-        int stage = 0; uint32_t phase = 0;
-        for (int item = blockIdx.x; item < gp.items; item += gridDim.x) {
-            int pi, m_blk, n_blk, split; decode(item, pi, m_blk, n_blk, split);
-            const GroupProb& P = gp.p[pi];
-            const int kb0 = split * P.kb_per_split, kb1 = min(gp.kblocks, kb0 + P.kb_per_split);
-            const uint32_t tx = (uint32_t)(A_STAGE + P.n_boxes * 64 * GBK * 2);
-            for (int kb = kb0; kb < kb1; ++kb) {
-                mbar_wait(&empty[stage], phase ^ 1);
-                if (elect_one_lane()) {
-                    mbar_expect_tx(&full[stage], tx);
-                    uint8_t* a = sA + stage * A_STAGE; uint8_t* b = sB + stage * B_STAGE;
-                    tma_load_2d(a, &maps.a[pi], &full[stage], m_blk * BM, kb * GBK);
-                    tma_load_2d(a + 64 * GBK * 2, &maps.a[pi], &full[stage], m_blk * BM + 64, kb * GBK);
-                    for (int j = 0; j < P.n_boxes; ++j) tma_load_2d(b + j * (64 * GBK * 2), &maps.b[pi], &full[stage], n_blk * 256 + j * 64, kb * GBK);
-                }
-                __syncwarp();
-                if (++stage == GSTAGES) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        int stage = 0; uint32_t phase = 0; int acc = 0; uint32_t acc_phase = 0;
-        for (int item = blockIdx.x; item < gp.items; item += gridDim.x) {
-            int pi, m_blk, n_blk, split; decode(item, pi, m_blk, n_blk, split);
-            const GroupProb& P = gp.p[pi];
-            const int kb0 = split * P.kb_per_split, kb1 = min(gp.kblocks, kb0 + P.kb_per_split);
-            const uint32_t idesc = make_idesc(BM, P.n_boxes * 64, true, true);
-            mbar_wait(&tempty[acc], acc_phase ^ 1);
-            tcgen05_fence_after();
-            const uint32_t tmem_d = tmem_base + (uint32_t)(acc * 256);
-            for (int kb = kb0; kb < kb1; ++kb) {
-                mbar_wait(&full[stage], phase);
-                tcgen05_fence_after();
-                const uint32_t a0 = smem_u32(sA + stage * A_STAGE), b0 = smem_u32(sB + stage * B_STAGE);
-                if (elect_one_lane()) {
-#pragma unroll
-                    for (int k = 0; k < GBK / 16; ++k)
-                        umma_bf16(tmem_d, make_desc(a0 + k * 2048, 64 * GBK * 2, 1024), make_desc(b0 + k * 2048, 64 * GBK * 2, 1024), idesc, (kb > kb0 || k > 0) ? 1u : 0u);
-                    tcgen05_commit(&empty[stage]);
-                }
-                __syncwarp();
-                if (++stage == GSTAGES) { stage = 0; phase ^= 1; }
-            }
-            if (elect_one_lane()) tcgen05_commit(&tfull[acc]);
-            __syncwarp();
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    } else {
-        const int quad = warp & 3;
-        int acc = 0; uint32_t acc_phase = 0;
-        for (int item = blockIdx.x; item < gp.items; item += gridDim.x) {
-            int pi, m_blk, n_blk, split; decode(item, pi, m_blk, n_blk, split);
-            const GroupProb& P = gp.p[pi];
-            mbar_wait(&tfull[acc], acc_phase);
-            tcgen05_fence_after();
-            const int m = m_blk * BM + quad * 32 + lane;
-            const bool row_ok = m < P.M_valid;
-#pragma unroll 1
-            for (int c = 0; c < P.n_boxes * 2; ++c) {
-                uint32_t r[32];
-                tmem_ld32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * 256 + c * 32), r);
-                const int n0 = n_blk * 256 + c * 32;
-                if (row_ok && n0 < P.N_valid) {
-                    float* dst = P.out + (size_t)m * P.ld_out + n0;
-                    if (n0 + 32 <= P.N_valid && (P.ld_out & 3) == 0) {
-#pragma unroll
-                        for (int q = 0; q < 8; ++q)
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + q * 4), "f"(__uint_as_float(r[q * 4])), "f"(__uint_as_float(r[q * 4 + 1])),
-                                         "f"(__uint_as_float(r[q * 4 + 2])), "f"(__uint_as_float(r[q * 4 + 3])) : "memory");
-                    } else {
-                        for (int j = 0; j < 32; ++j) if (n0 + j < P.N_valid) atomicAdd(dst + j, __uint_as_float(r[j]));
-                    }
-                }
-            }
-            tcgen05_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tcgen05_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
-}
-
-// one problem of a grouped launch: out[M_valid][N_valid] (ld_out) += X^T D, X [rows][M] (ld M), D [rows][Nd] (ld Nd)
-struct GroupDesc { const __nv_bfloat16* X; int M; const __nv_bfloat16* D; int Nd; float* out; int M_valid, N_valid, ld_out; double alg_flops; };
-
-static int launch_group(dppo_handle* h, cudaStream_t s, const GroupDesc* d, int n, int rows) {
-    if (n < 1 || n > GMAX) DPPO_FAIL(-1, "launch_group: bad problem count %d", n);
-    GroupMaps maps; GroupParams gp; memset(&gp, 0, sizeof(gp));
-    gp.nprob = n; gp.kblocks = (rows + GBK - 1) / GBK;
-    double cost[GMAX], total = 0; int tiles[GMAX];
-    for (int i = 0; i < n; ++i) {
-        GroupProb& P = gp.p[i];
-        DPPO_TRY(make_map(&maps.a[i], d[i].X, rows, d[i].M, d[i].M, GBK, 64));
-        DPPO_TRY(make_map(&maps.b[i], d[i].D, rows, d[i].Nd, d[i].Nd, GBK, 64));
-        P.m_blocks = (d[i].M + BM - 1) / BM;
-        const int nb64 = (d[i].Nd + 63) / 64;
-        P.n_boxes = nb64 < 4 ? nb64 : 4; P.n_blocks = (nb64 + 3) / 4;
-        P.M_valid = d[i].M_valid; P.N_valid = d[i].N_valid; P.ld_out = d[i].ld_out; P.out = d[i].out;
-        tiles[i] = P.m_blocks * P.n_blocks;
-        cost[i] = tiles[i] * (0.25 + 0.75 * P.n_boxes / 4.0);     // MMA time ~ N, plus the A stream and the epilogue
-        total += cost[i];
-    }
-    for (int i = n; i < GMAX; ++i) { maps.a[i] = maps.a[0]; maps.b[i] = maps.b[0]; }
-    int items = 0; double flops = 0;
-    for (int i = 0; i < n; ++i) {
-        GroupProb& P = gp.p[i];
-        int splits = (int)(h->sm_count * (cost[i] / total) / tiles[i] + 0.5);
-        if (splits < 1) splits = 1;
-        int maxs = gp.kblocks / 4; if (maxs < 1) maxs = 1;
-        if (splits > maxs) splits = maxs;
-        P.kb_per_split = (gp.kblocks + splits - 1) / splits;
-        P.splits = (gp.kblocks + P.kb_per_split - 1) / P.kb_per_split;
-        P.item_begin = items; items += tiles[i] * P.splits;
-        flops += d[i].alg_flops;
-    }
-    gp.items = items;
-    const size_t smem = (size_t)GSTAGES * (BM * GBK * 2 + 256 * GBK * 2) + 1024 + 256;
-    static bool attr_set_dev[64] = {};      // function attributes are per device
-    bool& attr_set = attr_set_dev[h->device & 63];
-    if (!attr_set) { CUDA_TRY(cudaFuncSetAttribute(dw_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); attr_set = true; }
-    const int grid = items < h->sm_count ? items : h->sm_count;
-    prof_begin(h, s);
-    dw_group_kernel<<<grid, NUM_THREADS, smem, s>>>(maps, gp);
-    prof_end(h, s, flops, 1);
-    h->launches++; h->tc_launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) DPPO_FAIL(-3, "grouped dW launch failed: %s", cudaGetErrorString(e));
-    return 0;
-}
-}  // namespace tc

@@ -1,7 +1,7 @@
 // tcgen05 path (DPPO_PREC_BF16) for large row counts: host programs.  Forward / backward chains run on the fused
 // layer-chain kernel (fused_chain.cuh) when the shapes allow it (ReLU at H = 256 / 512, Mish at H = 256, 64-wide h0),
-// else every MLP layer is one tc::gemm_kernel launch; the weight gradients are one grouped tcgen05 launch
-// (tc::dw_group_kernel) or, in the deterministic mode, one split-K GEMM + fixed-order reduction per product.
+// else every MLP layer is one tc::gemm_kernel launch; the weight gradients are one grouped tcgen05 launch on CTA pairs
+// (tcp::dw_pair_kernel) or, in the deterministic mode, one split-K GEMM + fixed-order reduction per product.
 //
 // Data layout in HBM (all bf16 activations are row-major [rows][features]; nothing is transposed):
 //   h0   [N][KP0]   = [ x (A) | obs (Do) | onehot(t) (T) | 1 | 0.. ]          KP0 = roundup(A+Do+T+1, 64)
@@ -617,10 +617,9 @@ static bool fc_critic_ok(const dppo_handle* h) { return fc_net_ok(h, fc_critic_n
 
 static int fc_weight_maps(const dppo_handle* h, const FcNet& n, CUtensorMap* m) {
     const TcNetW& W = h->tc->net[n.net]; const int H = n.H;
-    const int cg = h->chain_cg;
-    DPPO_TRY(fc::weight_map(&m[0], W.w2w0, H + 64, H, H, cg));
-    DPPO_TRY(fc::weight_map(&m[1], W.w1, H, H, H, cg));
-    DPPO_TRY(fc::weight_map(&m[2], W.w3p, H, 64 * cg, 128, cg));      // a CTA pair splits N: the output layer is padded to 128 columns
+    DPPO_TRY(fc::weight_map(&m[0], W.w2w0, H + 64, H, H));
+    DPPO_TRY(fc::weight_map(&m[1], W.w1, H, H, H));
+    DPPO_TRY(fc::weight_map(&m[2], W.w3p, H, 128, 128));      // a CTA pair splits N: the output layer is padded to 128 columns
     return 0;
 }
 // forward program: L0 act(H0 W0 + b0), L1 act(X W1 + b1), L2 X W2 + H0 W0 + b2, L3 X W3 + b3; weight maps at m[wbase..wbase+2]
@@ -631,7 +630,7 @@ static void fc_fwd_layers(const dppo_handle* h, const FcNet& n, int wbase, fc::L
     L[0].a_src = 0; L[0].wmap = wbase; L[0].wrow_h0 = H; L[0].n = H; L[0].bias = n.b0; L[0].act = n.act1;
     L[1].a_src = 1; L[1].wmap = wbase + 1; L[1].n = H; L[1].bias = n.b1; L[1].act = n.act1;
     L[2].a_src = 2; L[2].wmap = wbase; L[2].wrow_h0 = H; L[2].n = H; L[2].bias = n.b2; L[2].h0_last = 1;
-    L[3].a_src = 1; L[3].wmap = wbase + 2; L[3].n = 64 * h->chain_cg; L[3].bias = n.b3;
+    L[3].a_src = 1; L[3].wmap = wbase + 2; L[3].n = 128; L[3].bias = n.b3;
 }
 // algorithmic flops (SURVEY.md 8d: un-padded dims, time-MLP excluded): forward F = 2 (din H + 2 H^2 + H NO) per row
 static double fc_fwd_flops(const FcNet& n, double rows) { const double H = n.H; return 2.0 * rows * (n.din * H + 2.0 * H * H + H * n.NO); }
@@ -691,9 +690,9 @@ static int fc_bwd(dppo_handle* h, cudaStream_t s, const FcNet& n, const bf16* do
     const int H = n.H; const TcNetW& W = h->tc->net[n.net];
     fc::Maps maps; fc::Params p; fc_common(h, p, N, n.NO);
     DPPO_TRY(fc::rowtile_map(&maps.m[0], doutb, N, 64));
-    DPPO_TRY(fc::weight_map(&maps.m[1], W.w3t, 64, H, H, h->chain_cg));
-    DPPO_TRY(fc::weight_map(&maps.m[2], W.w2t, H, H, H, h->chain_cg));
-    DPPO_TRY(fc::weight_map(&maps.m[3], W.w1t, H, H, H, h->chain_cg));
+    DPPO_TRY(fc::weight_map(&maps.m[1], W.w3t, 64, H, H));
+    DPPO_TRY(fc::weight_map(&maps.m[2], W.w2t, H, H, H));
+    DPPO_TRY(fc::weight_map(&maps.m[3], W.w1t, H, H, H));
     DPPO_TRY(fc::rowtile_map(&maps.m[4], dv, N, H));
     DPPO_TRY(fc::rowtile_map(&maps.m[5], dh1, N, H));
     DPPO_TRY(fc::rowtile_map(&maps.m[6], du, N, H));
@@ -856,7 +855,7 @@ static size_t tc_part_floats(const dppo_handle* h, int H) {
 // fused backward chain of one net (dv, dh1, du) + its bias column sums
 static int tc_mlp_backward_dx(dppo_handle* h, cudaStream_t s, const TcMlp& m, const bf16* doutb, int N, float* part, float* gnet, size_t ob1, size_t ob2) {
     const int H = m.H;
-    const int grid = fc::chain_grid(h, N, h->chain_cg);
+    const int grid = fc::chain_grid(h, N);
     float* cpart = m.cpart ? m.cpart : part;                   // [grid][2][H]; `part` is consumed before anything reuses it
     DPPO_TRY(fc_bwd(h, s, m.net == DPPO_NET_CRITIC ? fc_critic_net(h) : fc_actor_net(h, m.net), doutb, N, m.m0, m.m1, m.pre0, m.pre1,
                     m.dv, m.dh1, m.du, cpart));
@@ -865,16 +864,8 @@ static int tc_mlp_backward_dx(dppo_handle* h, cudaStream_t s, const TcMlp& m, co
     }
     return 0;
 }
-// the five weight-gradient products of one net as grouped-GEMM problems (outputs accumulate atomically)
-static void tc_mlp_dw_descs(const TcMlp& m, const bf16* doutb, int N, float* gnet, size_t ow1, size_t ow2, size_t ow3, float* dw0, tc::GroupDesc* d) {
-    const int H = m.H, KP0 = m.KP0; const double r = (double)N;
-    d[0] = tc::GroupDesc{m.a1, H, m.dv, H, gnet + ow2, H, H, H, 2.0 * r * H * H};
-    d[1] = tc::GroupDesc{m.a0, H, m.dh1, H, gnet + ow1, H, H, H, 2.0 * r * H * H};
-    d[2] = tc::GroupDesc{m.h0, KP0, m.du, H, dw0, KP0, H, H, 2.0 * r * m.din * H};
-    d[3] = tc::GroupDesc{m.h0, KP0, m.dv, H, dw0, KP0, H, H, 0.0};                    // residual path: not algorithmic work
-    d[4] = tc::GroupDesc{m.v, H, doutb, 64, gnet + ow3, H, m.NO, m.NO, 2.0 * r * H * m.NO};
-}
-// the same five products for the CTA-pair kernel: the narrow layer-0 products are handed over as du^T h0 / dv^T h0 (transposed output)
+// the five weight-gradient products of one net as grouped-GEMM problems (outputs accumulate atomically); the narrow layer-0
+// products are handed over as du^T h0 / dv^T h0 (transposed output)
 static void tc_mlp_dw_pair_descs(const TcMlp& m, const bf16* doutb, int N, float* gnet, size_t ow1, size_t ow2, size_t ow3, float* dw0, tcp::PairDesc* d) {
     const int H = m.H, KP0 = m.KP0; const double r = (double)N;
     d[0] = tcp::PairDesc{m.a1, H, m.dv, H, gnet + ow2, H, H, H, 0, 2.0 * r * H * H};
@@ -892,14 +883,9 @@ static int tc_mlp_backward(dppo_handle* h, cudaStream_t s, const TcMlp& m, const
         // one launch: dv, dh1 and the non-residual part of du; the residual path joins in dW0 = h0^T du + h0^T dv
         DPPO_TRY(tc_mlp_backward_dx(h, s, m, doutb, N, part, gnet, ob1, ob2));
         if (!h->deterministic) {   // all five weight-gradient products in one grouped launch
-            if (h->dw_pair) {
-                tcp::PairDesc pd[5];
-                tc_mlp_dw_pair_descs(m, doutb, N, gnet, ow1, ow2, ow3, dw0, pd);
-                if (tcp::pair_ok(h, pd, 5)) return tcp::launch_group_pair(h, s, pd, 5, N);
-            }
-            tc::GroupDesc d[5];
-            tc_mlp_dw_descs(m, doutb, N, gnet, ow1, ow2, ow3, dw0, d);
-            return tc::launch_group(h, s, d, 5, N);
+            tcp::PairDesc pd[5];
+            tc_mlp_dw_pair_descs(m, doutb, N, gnet, ow1, ow2, ow3, dw0, pd);
+            return tcp::launch_group_pair(h, s, pd, 5, N);
         }
         DPPO_TRY(tc_dw(h, s, m.v, H, doutb, 64, N, part, gnet + ow3, H, m.NO, m.NO));
         DPPO_TRY(tc_dw(h, s, m.a1, H, m.dv, H, N, part, gnet + ow2, H, H, H));
@@ -1101,7 +1087,7 @@ static int tc_ppo_adv_stats(dppo_handle* h, cudaStream_t s, const float* advanta
     // pack_h0 and the forward chains (the join in front of the loss kernel orders them)
     TcPpoPlan& P = tc_plan(h);
     cudaStream_t st = s;
-    if (P.ma.fused && P.mc.fused && !h->deterministic && h->overlap_chains && !h->prof_on) {
+    if (P.ma.fused && P.mc.fused && !h->deterministic && !h->prof_on) {
         if (!h->aux_stream) {
             CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
             for (int i = 0; i < 2; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
@@ -1157,7 +1143,7 @@ static int tc_ppo_chunk(dppo_handle* h, cudaStream_t s, int chunk, const float* 
     // The actor and the critic chains are independent persistent kernels whose last wave leaves a third of the SMs idle
     // (391 row tiles on 148 SMs): the critic chain goes to a second stream so that its CTAs fill the actor chain's tail.
     // (not while the per-kernel profile is on: its event brackets are meant to time each kernel running alone)
-    const bool overlap = defer && h->overlap_chains && !h->prof_on;
+    const bool overlap = defer && !h->prof_on;
     if (overlap && !h->aux_stream) {
         CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
         for (int i = 0; i < 2; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
@@ -1192,16 +1178,10 @@ static int tc_ppo_chunk(dppo_handle* h, cudaStream_t s, int chunk, const float* 
         const TcMlp da = tc_mlp_at(P.ma, d0), dc = tc_mlp_at(P.mc, d0);
         const bf16* const dd = P.depsb + d0 * 64; const bf16* const dvd = P.dvalb + d0 * 64;
         P.dw_done = P.rows_done;
-        if (h->dw_pair) {
-            tcp::PairDesc pd[10];
-            tc_mlp_dw_pair_descs(da, dd, dn, h->grads, g.ao.w1, g.ao.w2, g.ao.w3, P.dw0a, pd);
-            tc_mlp_dw_pair_descs(dc, dvd, dn, h->grads + nA, g.co.w1, g.co.w2, g.co.w3, P.dw0c, pd + 5);
-            if (tcp::pair_ok(h, pd, 10)) return tcp::launch_group_pair(h, s, pd, 10, dn);
-        }
-        tc::GroupDesc d[10];
-        tc_mlp_dw_descs(da, dd, dn, h->grads, g.ao.w1, g.ao.w2, g.ao.w3, P.dw0a, d);
-        tc_mlp_dw_descs(dc, dvd, dn, h->grads + nA, g.co.w1, g.co.w2, g.co.w3, P.dw0c, d + 5);
-        return tc::launch_group(h, s, d, 10, dn);
+        tcp::PairDesc pd[10];
+        tc_mlp_dw_pair_descs(da, dd, dn, h->grads, g.ao.w1, g.ao.w2, g.ao.w3, P.dw0a, pd);
+        tc_mlp_dw_pair_descs(dc, dvd, dn, h->grads + nA, g.co.w1, g.co.w2, g.co.w3, P.dw0c, pd + 5);
+        return tcp::launch_group_pair(h, s, pd, 10, dn);
     }
     DPPO_TRY(tc_mlp_backward(h, s, ma, depsb, n, P.part, h->grads, g.ao.w1, g.ao.b1, g.ao.w2, g.ao.b2, g.ao.w3, P.dw0a));
     DPPO_TRY(tc_mlp_backward(h, s, mc, dvalb, n, P.part, h->grads + nA, g.co.w1, g.co.b1, g.co.w2, g.co.b2, g.co.w3, P.dw0c));
@@ -1271,18 +1251,9 @@ static int tc_ppo_finish(dppo_handle* h, cudaStream_t s) {
 static int tc_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const float* prev, const float* nxt, const int32_t* inds,
                        const float* returns, const float* oldvalues, const float* advantages, const float* oldlogp,
                        int N, int64_t N_global, float adv_mean, float adv_std) {
-    static int dev_chunk = -2;                       // dev knob DPPO_DEV_CHUNK_ROWS: chunk the device-resident call like the host pipeline does
-    if (dev_chunk == -2) { const char* v = getenv("DPPO_DEV_CHUNK_ROWS"); dev_chunk = v ? atoi(v) : 0; }
-    const Geom& g = h->g;
-    DPPO_TRY(tc_ppo_begin(h, s, N, dev_chunk > 0 ? dev_chunk : 0, N_global));
+    DPPO_TRY(tc_ppo_begin(h, s, N, 0, N_global));
     DPPO_TRY(tc_ppo_adv_stats(h, s, advantages, N, adv_mean, adv_std));
-    const int CR = tc_plan(h).chunk_rows, nch = tc_plan(h).nchunks;
-    for (int c = 0; c < nch; ++c) {
-        const size_t r0 = (size_t)c * CR; if (r0 >= (size_t)N) break;
-        const int n = (int)((size_t)N - r0 < (size_t)CR ? (size_t)N - r0 : (size_t)CR);
-        DPPO_TRY(tc_ppo_chunk(h, s, c, obs + r0 * g.Do, prev + r0 * g.A, nxt + r0 * g.A, inds + r0, returns + r0, oldvalues + r0, advantages + r0,
-                              oldlogp + r0 * g.A, n));
-    }
+    DPPO_TRY(tc_ppo_chunk(h, s, 0, obs, prev, nxt, inds, returns, oldvalues, advantages, oldlogp, N));
     return tc_ppo_finish(h, s);
 }
 

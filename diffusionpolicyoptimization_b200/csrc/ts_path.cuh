@@ -28,9 +28,10 @@
 //       split-K partials of the weight gradients (deterministic fixed-order reduction).  The layers whose output is the next
 //       GEMM's operand run on tsp::pair_gemm_kernel below.
 //     * operands K-major or MN-major as stored (activations [rows][features], weights [in][out]): nothing is transposed
-//   host programs (same data flow as the per-layer bf16 programs of tc_path.cuh, every activation / gradient as two planes):
-//     forward L0..L3 (residual by K-concatenation [a1 | h0] x [W2 ; W0]), backward dv / dh1 / du, the four weight-gradient
-//     products per net, bias gradients by column sums, the time-embedding backward from dW0's one-hot rows.
+//   host programs (the data flow of the per-layer bf16 programs of tc_path.cuh, every activation / gradient as two planes):
+//     forward L0, L1 and the folded output layer [a1 | h0] x [W2 W3 ; W0 W3] (block.l2 and the output layer in one narrow
+//     GEMM), backward dh1 / du, the four weight-gradient products per net (dW3, dW2 and the residual share of dW0 assembled
+//     from a1^T dout / h0^T dout), bias gradients by column sums, the time-embedding backward from dW0's one-hot rows.
 #pragma once
 #include "tc_path.cuh"
 
@@ -424,11 +425,9 @@ static inline void smem_plan(int stage_bytes, int planes_staged, int fixed_slots
 __device__ __forceinline__ void epi_barrier8() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// launches of consecutive plane GEMMs in one stream overlap the next grid's prologue with the previous grid's last wave (DPPO_NO_PDL=1: off)
-static inline bool pdl_enabled() { static int v = -1; if (v < 0) { const char* e = getenv("DPPO_NO_PDL"); v = (e && atoi(e)) ? 0 : 1; } return v != 0; }
+// launches of consecutive plane GEMMs in one stream overlap the next grid's prologue with the previous grid's last wave
 static inline int pdl_attrs(cudaLaunchAttribute* at) {
     at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    if (!pdl_enabled()) return 1;
     at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[1].val.programmaticStreamSerializationAllowed = 1;
     return 2;
 }
@@ -978,8 +977,8 @@ __global__ void __launch_bounds__(256) dw_reduce_kernel(const DwParams gp, const
 // one problem: out = X^T D (+ X2^T D2), X [rows][M], D [rows][Nd] (two planes each); transposed: out[n][m] (ld_out = row length of that layout)
 struct DwDesc { SplitT X; int M; SplitT D; int Nd; SplitT X2, D2; float* out; int M_valid, N_valid, ld_out, transposed; double alg_flops; };
 
-static int launch_dw_group(dppo_handle* h, cudaStream_t s, const DwDesc* d, int n, int rows, float* part, size_t part_floats, int* elem_begin_dev) {
-    if (n < 1 || n > DMAXP) DPPO_FAIL(-1, "launch_dw_group: bad problem count %d", n);
+static int launch_dw_pair(dppo_handle* h, cudaStream_t s, const DwDesc* d, int n, int rows, float* part, size_t part_floats, int* elem_begin_dev) {
+    if (n < 1 || n > DMAXP) DPPO_FAIL(-1, "launch_dw_pair: bad problem count %d", n);
     DwMaps maps; DwParams gp; memset(&gp, 0, sizeof(gp));
     gp.nprob = n; gp.part = part;
     const int kblocks = (rows + 63) / 64;
@@ -987,14 +986,14 @@ static int launch_dw_group(dppo_handle* h, cudaStream_t s, const DwDesc* d, int 
     double w[DMAXP]; int tiles[DMAXP]; int nmap = n;
     for (int i = 0; i < n; ++i) {
         DwProb& P = gp.p[i];
-        if (d[i].M % 64 || d[i].Nd % 64) DPPO_FAIL(-7, "launch_dw_group: operand widths must be multiples of 64");
+        if (d[i].M % 64 || d[i].Nd % 64) DPPO_FAIL(-7, "launch_dw_pair: operand widths must be multiples of 64");
         for (int pl = 0; pl < 2; ++pl) {
             DPPO_TRY(make_map(&maps.a[i][pl], d[i].X.p[pl], rows, d[i].M, d[i].M, 64, 64));
             DPPO_TRY(make_map(&maps.b[i][pl], d[i].D.p[pl], rows, d[i].Nd, d[i].Nd, 64, 64));
         }
         P.kb_seg0 = kblocks; P.kb_total = kblocks; P.map2 = i;
         if (d[i].X2.p[0]) {
-            if (nmap >= DMAPS) DPPO_FAIL(-7, "launch_dw_group: too many second segments");
+            if (nmap >= DMAPS) DPPO_FAIL(-7, "launch_dw_pair: too many second segments");
             for (int pl = 0; pl < 2; ++pl) {
                 DPPO_TRY(make_map(&maps.a[nmap][pl], d[i].X2.p[pl], rows, d[i].M, d[i].M, 64, 64));
                 DPPO_TRY(make_map(&maps.b[nmap][pl], d[i].D2.p[pl], rows, d[i].Nd, d[i].Nd, 64, 64));
@@ -1029,7 +1028,7 @@ static int launch_dw_group(dppo_handle* h, cudaStream_t s, const DwDesc* d, int 
         eb[i + 1] = eb[i] + P.M_valid * P.N_valid;
     }
     gp.items = items;
-    if ((size_t)items * 65536 > part_floats) DPPO_FAIL(-7, "launch_dw_group: partial buffer too small (%d items)", items);
+    if ((size_t)items * 65536 > part_floats) DPPO_FAIL(-7, "launch_dw_pair: partial buffer too small (%d items)", items);
     CUDA_TRY(cudaMemcpyAsync(elem_begin_dev, eb, (n + 1) * sizeof(int), cudaMemcpyHostToDevice, s));
     static bool attr_set_dev[64] = {};      // function attributes are per device
     bool& attr_set = attr_set_dev[h->device & 63];
@@ -1058,14 +1057,12 @@ static int launch_dw_group(dppo_handle* h, cudaStream_t s, const DwDesc* d, int 
 // 2^10 w (forward GEMMs of a net with kinks behind it)
 struct TsW { bf16* p[ts::MAXP]; };
 struct TsNetW {
-    TsW w2w0, w1, w3t, w3p;
-    TsW fw2w0, fw1, fw3t;                 // fp16 planes, scaled by ts::F16_WSCALE
+    TsW w0, w1;                           // [KP0][H] W0 rows in h0 order, [H][H] W1
+    TsW fw0, fw1;                         // fp16 planes, scaled by ts::F16_WSCALE
     TsW ffold;                            // [64][H + KP0] planes of [W2 W3 ; W0 W3]^T (fp16 x 2^10 when the net's forward runs on fp16 planes, else
                                           // bf16): the folded output layer, out = [a1 | h0] [W2 W3 ; W0 W3] + bfold
     float* bfold;                         // [64]  (b2 (+ b_in)) W3 + b3
     TsW w23p;                             // [H][128] bf16 planes of W2 W3 (columns >= NO zero): dh1 = (dout (W2 W3)^T) . act'(h1) without forming dv
-    float* bias2;                         // critic: b2 + b_in (the residual's input-layer bias rides with block.l2's)
-    int H;
 };
 struct TsState { TsNetW net[4]; int KP0; int fold_dirty[4]; char* dw3_buf; size_t dw3_bytes; };
 
@@ -1078,40 +1075,28 @@ __device__ __forceinline__ void ts_put_f16(const TsW& W, size_t i, float v) {
     W.p[0][i] = a; W.p[1][i] = b;
 }
 __device__ __forceinline__ void ts_put2(const TsW& W, const TsW& F, size_t i, float v) { ts_put(W, i, v); ts_put_f16(F, i, v); }
-// same operand layouts as tc_pack_actor_body (w2w0 = [W2 ; W0 rows in h0 order], w3t = W3^T padded to 64 rows, w3p = W3 padded to
-// 128 columns), each as two bf16 planes (+ two fp16 planes for the forward operands); no transposed copies (the backward GEMMs read
-// W1 / W2 K-major as stored)
+// W0 in tc_pack_actor_body's h0 row order and W1, each as two bf16 planes and two fp16 planes; no transposed copy (the backward GEMM
+// reads W1 K-major as stored).  W2 and W3 enter the GEMMs only through the folded output layer (ts_fold_kernel).
 __global__ void ts_pack_actor_kernel(const float* __restrict__ w, ActorOff o, int A, int td, int Do, int T, int H, int KP0,
                                      const float* __restrict__ bt, const TsNetW W) {
     const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = i0; i < (size_t)H * H; i += stride) { ts_put2(W.w2w0, W.fw2w0, i, w[o.w2 + i]); ts_put2(W.w1, W.fw1, i, w[o.w1 + i]); }
+    for (size_t i = i0; i < (size_t)H * H; i += stride) ts_put2(W.w1, W.fw1, i, w[o.w1 + i]);
     for (size_t i = i0; i < (size_t)KP0 * H; i += stride) {
         const int k = (int)(i / H), c = (int)(i % H);
         float v = 0.f;
         if (k < A) v = w[o.win + (size_t)k * H + c];
         else if (k < A + Do) v = w[o.win + (size_t)(k + td) * H + c];
         else if (k < A + Do + T) v = bt[(size_t)(k - A - Do) * H + c];
-        ts_put2(W.w2w0, W.fw2w0, (size_t)H * H + i, v);
-    }
-    for (size_t i = i0; i < (size_t)64 * H; i += stride) {
-        const int a = (int)(i / H), k = (int)(i % H);
-        ts_put2(W.w3t, W.fw3t, i, a < A ? w[o.w3 + (size_t)k * A + a] : 0.f);
-    }
-    for (size_t i = i0; i < (size_t)H * 128; i += stride) {
-        const int k = (int)(i / 128), a = (int)(i % 128);
-        ts_put(W.w3p, i, a < A ? w[o.w3 + (size_t)k * A + a] : 0.f);
+        ts_put2(W.w0, W.fw0, i, v);
     }
 }
 __global__ void ts_pack_critic_kernel(const float* __restrict__ w, CriticOff o, int A, int Do, int Hc, int KP0, const TsNetW W) {
     const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = i0; i < (size_t)Hc * Hc; i += stride) { ts_put2(W.w2w0, W.fw2w0, i, w[o.w2 + i]); ts_put2(W.w1, W.fw1, i, w[o.w1 + i]); }
+    for (size_t i = i0; i < (size_t)Hc * Hc; i += stride) ts_put2(W.w1, W.fw1, i, w[o.w1 + i]);
     for (size_t i = i0; i < (size_t)KP0 * Hc; i += stride) {
         const int k = (int)(i / Hc), c = (int)(i % Hc);
-        ts_put2(W.w2w0, W.fw2w0, (size_t)Hc * Hc + i, (k >= A && k < A + Do) ? w[o.win + (size_t)(k - A) * Hc + c] : 0.f);
+        ts_put2(W.w0, W.fw0, i, (k >= A && k < A + Do) ? w[o.win + (size_t)(k - A) * Hc + c] : 0.f);
     }
-    for (size_t i = i0; i < (size_t)64 * Hc; i += stride) { const int a = (int)(i / Hc), k = (int)(i % Hc); ts_put2(W.w3t, W.fw3t, i, a == 0 ? w[o.w3 + k] : 0.f); }
-    for (size_t i = i0; i < (size_t)Hc * 128; i += stride) { const int k = (int)(i / 128), a = (int)(i % 128); ts_put(W.w3p, i, a == 0 ? w[o.w3 + k] : 0.f); }
-    for (size_t i = i0; i < (size_t)Hc; i += stride) W.bias2[i] = w[o.b2 + i] + w[o.bin + i];
 }
 // h0[r] = [x[r] | obs[r / obs_div] | onehot(t_r) | 1 | 0..] (tc_pack_h0_kernel's layout) as two fp16 planes (hf, when given) and / or two
 // bf16 planes (hb, when given); one thread per 8 columns
@@ -1292,22 +1277,19 @@ static int ts_init(dppo_handle* h) {
     for (int net = 0; net < 4; ++net) {
         TsNetW& w = st->net[net];
         const size_t H = net == DPPO_NET_CRITIC ? g.Hc : g.H;
-        w.H = (int)H;
-        DPPO_TRY(ts_alloc_w(w.w2w0, (H + st->KP0) * H)); DPPO_TRY(ts_alloc_w(w.w1, H * H));
-        DPPO_TRY(ts_alloc_w(w.w3t, 64 * H)); DPPO_TRY(ts_alloc_w(w.w3p, H * 128));
-        DPPO_TRY(ts_alloc_w(w.fw2w0, (H + st->KP0) * H)); DPPO_TRY(ts_alloc_w(w.fw1, H * H)); DPPO_TRY(ts_alloc_w(w.fw3t, 64 * H));
+        DPPO_TRY(ts_alloc_w(w.w0, st->KP0 * H)); DPPO_TRY(ts_alloc_w(w.w1, H * H));
+        DPPO_TRY(ts_alloc_w(w.fw0, st->KP0 * H)); DPPO_TRY(ts_alloc_w(w.fw1, H * H));
         DPPO_TRY(ts_alloc_w(w.ffold, 64 * (H + st->KP0)));
         CUDA_TRY(cudaMalloc(&w.bfold, 64 * sizeof(float)));
         DPPO_TRY(ts_alloc_w(w.w23p, H * 128)); CUDA_TRY(cudaMemset(w.w23p.p[0], 0, 2 * H * 128 * sizeof(bf16)));
         st->fold_dirty[net] = 1;
-        CUDA_TRY(cudaMalloc(&w.bias2, H * sizeof(float)));
     }
     return 0;
 }
 static void ts_destroy(dppo_handle* h) {
     if (!h->ts) return;
     cudaFree(h->ts->dw3_buf);
-    for (int net = 0; net < 4; ++net) { TsNetW& w = h->ts->net[net]; cudaFree(w.w2w0.p[0]); cudaFree(w.w1.p[0]); cudaFree(w.w3t.p[0]); cudaFree(w.w3p.p[0]); cudaFree(w.fw2w0.p[0]); cudaFree(w.fw1.p[0]); cudaFree(w.fw3t.p[0]); cudaFree(w.ffold.p[0]); cudaFree(w.bfold); cudaFree(w.w23p.p[0]); cudaFree(w.bias2); }
+    for (int net = 0; net < 4; ++net) { TsNetW& w = h->ts->net[net]; cudaFree(w.w0.p[0]); cudaFree(w.w1.p[0]); cudaFree(w.fw0.p[0]); cudaFree(w.fw1.p[0]); cudaFree(w.ffold.p[0]); cudaFree(w.bfold); cudaFree(w.w23p.p[0]); }
     delete h->ts; h->ts = nullptr;
 }
 // rebuild the plane copies of one net (after set_weights / an optimizer step; the actor's bt table must be current)
@@ -1322,22 +1304,19 @@ static int ts_refresh_net(dppo_handle* h, int net, cudaStream_t s) {
 }
 
 // ------------------------------------------------------------------ one residual MLP on N rows, every tensor as planes
+// The output layer is folded: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, so block.l2's H x H product is skipped and v never formed (the
+// caller has run ts_ensure_fold).  The weight gradient of the output layer is assembled from a1^T dout and h0^T dout (ts_dw3_assemble_kernel).
 struct TsMlp {
     const TsNetW* W; int H, NO, act1, KP0, net, din;
     int fp;                                // FORWARD GEMMs: 4 = two fp16 planes + two accumulators (22 bits) when the net has kinks behind it,
-                                           // 2 = two bf16 planes, one accumulator (16 bits).  h0 / a0 / a1 / v carry that format.
-    const float *b0, *b1, *b2, *b3;
-    SplitT h0, a0, a1, v, g0, g1, dv, dh1, du;   // g0 / g1: Mish gates mish'(pre-activation) of layer 0 / block.l1 (two planes)
-    SplitT h0b, a0b, a1b, vb;              // fp = 4 with a backward pass: bf16 copies (two planes) for the weight-gradient GEMMs
-    int fold;                              // out = [a1 | h0] [W2 W3 ; W0 W3] + bfold: block.l2's H x H product is skipped and v never formed (the
-                                           // caller has run ts_ensure_fold).  The weight gradient of the output layer is then assembled from
-                                           // a1^T dout and h0^T dout (ts_dw3_assemble_kernel).
+                                           // 2 = two bf16 planes, one accumulator (16 bits).  h0 / a0 / a1 carry that format.
+    const float *b0, *b1;
+    SplitT h0, a0, a1, g0, g1, dh1, du;    // g0 / g1: Mish gates mish'(pre-activation) of layer 0 / block.l1 (two planes)
+    SplitT h0b, a0b, a1b;                  // fp = 4 with a backward pass: bf16 copies (two planes) for the weight-gradient GEMMs
     cudaEvent_t fold_ev;                   // when set: the folded operands are being rebuilt on another stream; wait in front of the folded GEMM
     uint32_t *m0, *m1;                     // ReLU bit masks [N][H/32] of layer 0 / block.l1
     float* out;                            // [N][NO] fp32
 };
-// DPPO_NO_FOLD=1: block.l2 and the output layer as two products everywhere (the unfolded programs; A/B and debugging)
-static inline bool ts_no_fold() { static int v = -1; if (v < 0) { const char* e = getenv("DPPO_NO_FOLD"); v = (e && atoi(e)) ? 1 : 0; } return v != 0; }
 // rebuild the folded output layer of one net if its weights changed (lazily: set_weights / AdamW only mark it stale)
 static int ts_ensure_fold(dppo_handle* h, int net, cudaStream_t s) {
     if (!h->ts->fold_dirty[net]) return 0;
@@ -1367,17 +1346,17 @@ static void ts_actor_mlp(const dppo_handle* h, int net, TsMlp& m) {
     memset(&m, 0, sizeof(m));
     m.W = &h->ts->net[net]; m.H = g.H; m.NO = g.A; m.act1 = h->cfg.actor_act + 1; m.KP0 = h->ts->KP0; m.net = net; m.din = g.Din;
     m.fp = 4;                                                                        // ReLU kinks and the +-1 clip of x0 behind eps
-    m.b0 = nullptr; m.b1 = w + g.ao.b1; m.b2 = w + g.ao.b2; m.b3 = w + g.ao.b3;      // b_in rides in W0's one-hot rows (bt table)
+    m.b0 = nullptr; m.b1 = w + g.ao.b1;                                              // b_in rides in W0's one-hot rows (bt table)
 }
 static void ts_critic_mlp(const dppo_handle* h, TsMlp& m) {
     const Geom& g = h->g; const float* w = h->net_w[DPPO_NET_CRITIC];
     memset(&m, 0, sizeof(m));
     m.W = &h->ts->net[DPPO_NET_CRITIC]; m.H = g.Hc; m.NO = 1; m.act1 = h->cfg.critic_act + 1; m.KP0 = h->ts->KP0; m.net = DPPO_NET_CRITIC; m.din = g.Do;
     m.fp = h->cfg.critic_act == DPPO_ACT_RELU ? 4 : 2;                               // Mish is smooth
-    m.b0 = w + g.co.bin; m.b1 = w + g.co.b1; m.b2 = m.W->bias2; m.b3 = w + g.co.b3;
+    m.b0 = w + g.co.bin; m.b1 = w + g.co.b1;
 }
 static size_t ts_mlp_ws_bytes(int N, int H, int KP0, bool mish, bool bwd) {
-    return 2 * (2 * ws_bytes((size_t)N * KP0, 2) + 3 * ws_bytes((size_t)N * H, 2)) + 2 * ws_bytes((size_t)N * H, 2) * (size_t)((mish ? 2 : 0) + (bwd ? 6 : 0))
+    return 2 * (2 * ws_bytes((size_t)N * KP0, 2) + 2 * ws_bytes((size_t)N * H, 2)) + 2 * ws_bytes((size_t)N * H, 2) * (size_t)((mish ? 2 : 0) + (bwd ? 4 : 0))
          + 2 * ws_bytes((size_t)N * (H / 32), 4);
 }
 static SplitT ts_take(dppo_handle* h, size_t n, int planes) {
@@ -1388,10 +1367,10 @@ static SplitT ts_take(dppo_handle* h, size_t n, int planes) {
 static void ts_mlp_take(dppo_handle* h, int N, TsMlp& m, bool bwd) {
     const size_t n = (size_t)N * m.H;
     m.h0 = ts_take(h, (size_t)N * m.KP0, 2);
-    m.a0 = ts_take(h, n, 2); m.a1 = ts_take(h, n, 2); m.v = ts_take(h, n, 2);
+    m.a0 = ts_take(h, n, 2); m.a1 = ts_take(h, n, 2);
     if (m.act1 == 2) { m.g0 = ts_take(h, n, 2); m.g1 = ts_take(h, n, 2); }
-    if (bwd) { m.dv = ts_take(h, n, 2); m.dh1 = ts_take(h, n, 2); m.du = ts_take(h, n, 2); }
-    if (bwd && m.fp == 4) { m.h0b = ts_take(h, (size_t)N * m.KP0, 2); m.a0b = ts_take(h, n, 2); m.a1b = ts_take(h, n, 2); m.vb = ts_take(h, n, 2); }
+    if (bwd) { m.dh1 = ts_take(h, n, 2); m.du = ts_take(h, n, 2); }
+    if (bwd && m.fp == 4) { m.h0b = ts_take(h, (size_t)N * m.KP0, 2); m.a0b = ts_take(h, n, 2); m.a1b = ts_take(h, n, 2); }
     m.m0 = ws_take<uint32_t>(h, (size_t)N * (m.H / 32)); m.m1 = ws_take<uint32_t>(h, (size_t)N * (m.H / 32));
 }
 static ts::Operand ts_op(const bf16* const* p, size_t off, bool mn_major, int64_t mn, int64_t k, int64_t ld) {
@@ -1423,13 +1402,12 @@ static tsp::Gemm tsp_gemm_of(ts::Operand A, ts::Operand B, int M, int N, int pla
 // phase 0: the whole forward; 1: L0 and L1 only; 2: what follows L1 (lets a caller enqueue other streams' work in between)
 static int ts_mlp_forward(dppo_handle* h, cudaStream_t s, const TsMlp& m, int N, int phase = 0) {
     const int H = m.H, KP0 = m.KP0, P = m.fp; const TsNetW& W = *m.W;
-    const size_t w0 = (size_t)H * H;
     const bool f16 = P == 4;
-    const TsW& Ww2w0 = f16 ? W.fw2w0 : W.w2w0; const TsW& Ww1 = f16 ? W.fw1 : W.w1; const TsW& Ww3t = f16 ? W.fw3t : W.w3t;
+    const TsW& Ww0 = f16 ? W.fw0 : W.w0; const TsW& Ww1 = f16 ? W.fw1 : W.w1;
     tsp::Gemm g;
     if (phase != 2) {
     // L0: a0 = act(h0 W0 (+ b0))
-    g = tsp_gemm_of(tsK(m.h0, N, KP0, KP0), tswMN(Ww2w0, w0, H, KP0, H), N, H, P, m.a0, P, H);
+    g = tsp_gemm_of(tsK(m.h0, N, KP0, KP0), tswMN(Ww0, 0, H, KP0, H), N, H, P, m.a0, P, H);
     g.epi.bias = m.b0; g.epi.act = m.act1;
     if (m.a0b.p[0]) { g.out2[0] = m.a0b.p[0]; g.out2[1] = m.a0b.p[1]; g.epi.out2 = 1; }
     if (m.act1 == 1) { g.epi.mask_out = m.m0; g.epi.ldm = H / 32; } else if (m.act1 == 2) { g.epi.gate_out = 1; g.gate[0] = m.g0.p[0]; g.gate[1] = m.g0.p[1]; }
@@ -1443,28 +1421,13 @@ static int ts_mlp_forward(dppo_handle* h, cudaStream_t s, const TsMlp& m, int N,
     DPPO_TRY(tsp::launch(h, s, g));
     }
     if (phase == 1) return 0;
-    if (m.fold) {
-        // no activation between block.l2 and the output layer: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, one narrow GEMM
-        ts::Gemm o = ts_gemm_of(tsK(m.a1, N, H, H), tswK(W.ffold, 0, 32, H, H + KP0), N, m.NO, 2, f16 ? 1 : 0);
-        o.A2 = tsK(m.h0, N, KP0, KP0); o.B2 = tswK(W.ffold, (size_t)H, 32, KP0, H + KP0);
-        if (f16) { o.f16 = 1; o.epi.scale = 1.0f / ts::F16_WSCALE; }
-        o.epi.bias = W.bfold; o.epi.out_f32 = m.out; o.epi.ld_f32 = m.NO;
-        o.alg_flops = 2.0 * N * ((double)H * H + (double)H * m.NO);        // the algorithmic work it stands for
-        if (m.fold_ev) CUDA_TRY(cudaStreamWaitEvent(s, m.fold_ev, 0));
-        DPPO_TRY(ts_run(h, s, o));
-        return 0;
-    }
-    // L2 + residual: v = [a1 | h0] [W2 ; W0] + b2 (+ b0): the residual u = h0 W0 is re-accumulated instead of stored and re-read
-    g = tsp_gemm_of(tsK(m.a1, N, H, H), tswMN(Ww2w0, 0, H, H, H), N, H, P, m.v, P, H);
-    g.A2 = tsK(m.h0, N, KP0, KP0); g.B2 = tswMN(Ww2w0, w0, H, KP0, H);
-    g.epi.bias = m.b2;
-    if (m.vb.p[0]) { g.out2[0] = m.vb.p[0]; g.out2[1] = m.vb.p[1]; g.epi.out2 = 1; }
-    g.alg_flops = 2.0 * N * (double)H * H;                                       // the re-accumulated residual is not algorithmic work
-    DPPO_TRY(tsp::launch(h, s, g));
-    // L3: out = v W3 + b3 (fp32, narrow: single-CTA kernel)
-    ts::Gemm o = ts_gemm_of(tsK(m.v, N, H, H), tswK(Ww3t, 0, 32, H, H), N, m.NO, 2, f16 ? 1 : 0);
+    // no activation between block.l2 and the output layer: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, one narrow GEMM
+    ts::Gemm o = ts_gemm_of(tsK(m.a1, N, H, H), tswK(W.ffold, 0, 32, H, H + KP0), N, m.NO, 2, f16 ? 1 : 0);
+    o.A2 = tsK(m.h0, N, KP0, KP0); o.B2 = tswK(W.ffold, (size_t)H, 32, KP0, H + KP0);
     if (f16) { o.f16 = 1; o.epi.scale = 1.0f / ts::F16_WSCALE; }
-    o.epi.bias = m.b3; o.epi.out_f32 = m.out; o.epi.ld_f32 = m.NO;
+    o.epi.bias = W.bfold; o.epi.out_f32 = m.out; o.epi.ld_f32 = m.NO;
+    o.alg_flops = 2.0 * N * ((double)H * H + (double)H * m.NO);        // the algorithmic work it stands for
+    if (m.fold_ev) CUDA_TRY(cudaStreamWaitEvent(s, m.fold_ev, 0));
     DPPO_TRY(ts_run(h, s, o));
     return 0;
 }
@@ -1490,25 +1453,15 @@ static int ts_colsum(dppo_handle* h, cudaStream_t s, const SplitT& D, int N, int
     tc_reduce_cols_kernel<<<tc_nblk(ncols, 8), 256, 0, s>>>(part, nb, (size_t)ncols, ncols, out); TC_KCHECK(h);
     return 0;
 }
-// backward chain of the residual MLP from dout [N][64] (two planes, zero padded): dv = dout W3^T, dh1 = (dv W2^T) . act'(h1),
-// du = (dh1 W1^T) . act'(u).  du excludes the residual path: dW0 = h0^T du + h0^T dv.
-// cpart [ceil(N/32)][2][H]: per 32-row block column sums of dv (slot 0 = db2) and dh1 (slot 1 = db1), written by the epilogues
-// m.fold: dv = dout W3^T has rank NO and is never formed: dh1 = (dout (W2 W3)^T) . act'(h1) is ONE K = 64 product, and everything else dv
+// backward chain of the residual MLP from dout [N][64] (two planes, zero padded): dh1 = (dout (W2 W3)^T) . act'(h1),
+// du = (dh1 W1^T) . act'(u).  dv = dout W3^T has rank NO and is never formed: dh1 is ONE K = 64 product, and everything else dv
 // fed - dW2 = a1^T dv = (a1^T dout) W3^T, the residual part of dW0 = (h0^T dout) W3^T, db2 = (1^T dout) W3^T - is assembled from the small
-// products a1^T dout / h0^T dout the folded output layer needs anyway (ts_dw3_assemble_kernel).  cpart slot 0 then stays unwritten.
+// products a1^T dout / h0^T dout the folded output layer needs anyway (ts_dw3_assemble_kernel).
+// cpart [ceil(N/32)][2][H]: per 32-row block column sums of dh1 (slot 1 = db1), written by the epilogue; slot 0 stays unwritten.
 static int ts_mlp_backward_dx(dppo_handle* h, cudaStream_t s, const TsMlp& m, const SplitT& dout, int N, float* cpart) {
     const int H = m.H; const TsNetW& W = *m.W;
-    tsp::Gemm g;
-    if (m.fold) {
-        g = tsp_gemm_of(tsK(dout, N, 64, 64), tswK(W.w23p, 0, H, 64, 128), N, H, 2, m.dh1, 2, H);
-        g.alg_flops = 2.0 * N * ((double)m.NO * H + (double)H * H);              // the two products it stands for
-    } else {
-    g = tsp_gemm_of(tsK(dout, N, 64, 64), tswK(W.w3p, 0, H, 64, 128), N, H, 2, m.dv, 2, H);
-    g.alg_flops = 2.0 * N * (double)m.NO * H;
-    g.epi.colsum_part = cpart; g.epi.colsum_ld = 2 * H;
-    DPPO_TRY(tsp::launch(h, s, g));
-    g = tsp_gemm_of(tsK(m.dv, N, H, H), tswK(W.w2w0, 0, H, H, H), N, H, 2, m.dh1, 2, H);
-    }
+    tsp::Gemm g = tsp_gemm_of(tsK(dout, N, 64, 64), tswK(W.w23p, 0, H, 64, 128), N, H, 2, m.dh1, 2, H);
+    g.alg_flops = 2.0 * N * ((double)m.NO * H + (double)H * H);                  // the two products it stands for
     g.epi.colsum_part = cpart + H; g.epi.colsum_ld = 2 * H;
     if (m.act1 == 1) { g.epi.mask_in = m.m1; g.epi.ldm = H / 32; } else if (m.act1 == 2) { g.epi.gate_in[0] = m.g1.p[0]; g.epi.gate_in[1] = m.g1.p[1]; g.epi.ldg = H; }
     DPPO_TRY(tsp::launch(h, s, g));
@@ -1517,26 +1470,18 @@ static int ts_mlp_backward_dx(dppo_handle* h, cudaStream_t s, const TsMlp& m, co
     DPPO_TRY(tsp::launch(h, s, g));
     return 0;
 }
-// the four weight-gradient products of one net for the grouped pair kernel; the narrow layer-0 product is handed over as
-// du^T h0 + dv^T h0 (wide operand on M, output written transposed into dw0 [KP0][H])
-// (fold: d[3] = a1^T dout -> g1 [H][NO] and d[4] = h0^T dout -> g0 [KP0][NO] instead of v^T dout; returns the number of problems)
-static int ts_mlp_dw_descs(const TsMlp& m, const SplitT& dout, int N, float* gnet, size_t ow1, size_t ow2, size_t ow3, float* dw0, tsp::DwDesc* d,
-                           float* g1 = nullptr, float* g0 = nullptr) {
+// the four weight-gradient products of one net for the grouped pair kernel: dW1 = a0^T dh1, the layer-0 product handed over as du^T h0
+// (wide operand on M, output written transposed into dw0 [KP0][H]), g1 = a1^T dout [H][NO] and g0 = h0^T dout [KP0][NO]; dW2, dW3 and
+// the residual part of dW0 come out of g1 / g0 (see ts_mlp_backward_dx).  Returns the number of problems.
+static int ts_mlp_dw_descs(const TsMlp& m, const SplitT& dout, int N, float* gnet, size_t ow1, float* dw0, tsp::DwDesc* d, float* g1, float* g0) {
     const int H = m.H, KP0 = m.KP0; const double r = (double)N; const SplitT none = split_null();
     // (fp = 4: the bf16 copies of the activations - one tcgen05.mma cannot take an fp16 and a bf16 operand, and the gradients are bf16)
     const bool f = m.fp == 4;
-    const SplitT& a0 = f ? m.a0b : m.a0; const SplitT& a1 = f ? m.a1b : m.a1; const SplitT& v = f ? m.vb : m.v; const SplitT& h0 = f ? m.h0b : m.h0;
-    d[0] = tsp::DwDesc{a1, H, m.dv, H, none, none, gnet + ow2, H, H, H, 0, 2.0 * r * H * H};
-    d[1] = tsp::DwDesc{a0, H, m.dh1, H, none, none, gnet + ow1, H, H, H, 0, 2.0 * r * H * H};
-    d[2] = tsp::DwDesc{m.du, H, h0, KP0, m.dv, h0, dw0, H, KP0, H, 1, 2.0 * r * m.din * H};
-    if (m.fold) {          // no dv: dW2 and the residual part of dW0 come out of g1 / g0 (see ts_mlp_backward_dx)
-        d[0] = tsp::DwDesc{a0, H, m.dh1, H, none, none, gnet + ow1, H, H, H, 0, 2.0 * r * H * H};
-        d[1] = tsp::DwDesc{m.du, H, h0, KP0, none, none, dw0, H, KP0, H, 1, 2.0 * r * m.din * H};
-        d[2] = tsp::DwDesc{a1, H, dout, 64, none, none, g1, H, m.NO, m.NO, 0, 2.0 * r * (H * m.NO + (double)H * H)};
-        d[3] = tsp::DwDesc{h0, KP0, dout, 64, none, none, g0, KP0, m.NO, m.NO, 0, 0.0};
-        return 4;
-    }
-    d[3] = tsp::DwDesc{v, H, dout, 64, none, none, gnet + ow3, H, m.NO, m.NO, 0, 2.0 * r * H * m.NO};
+    const SplitT& a0 = f ? m.a0b : m.a0; const SplitT& a1 = f ? m.a1b : m.a1; const SplitT& h0 = f ? m.h0b : m.h0;
+    d[0] = tsp::DwDesc{a0, H, m.dh1, H, none, none, gnet + ow1, H, H, H, 0, 2.0 * r * H * H};
+    d[1] = tsp::DwDesc{m.du, H, h0, KP0, none, none, dw0, H, KP0, H, 1, 2.0 * r * m.din * H};
+    d[2] = tsp::DwDesc{a1, H, dout, 64, none, none, g1, H, m.NO, m.NO, 0, 2.0 * r * (H * m.NO + (double)H * H)};
+    d[3] = tsp::DwDesc{h0, KP0, dout, 64, none, none, g0, KP0, m.NO, m.NO, 0, 0.0};
     return 4;
 }
 // dW3[j][a] = sum_r v[r][j] dout[r][a] with v = a1 W2 + (b2 + b0) + h0 W0 never formed:
@@ -1758,9 +1703,9 @@ static int ts_actor_forward(dppo_handle* h, cudaStream_t s, int net, const float
     TsMlp m; ts_actor_mlp(h, net, m);
     ts_mlp_take(h, N, m, false);
     m.out = eps;
-    // every program of this mode folds (or none: DPPO_NO_FOLD), so that the log-prob forward and the update's forward are the same
-    // arithmetic and the PPO ratio of unchanged weights is exactly 1 (the full-size parity tests assert it)
-    if (!ts_no_fold()) { DPPO_TRY(ts_ensure_fold(h, net, s)); m.fold = 1; }
+    // every program of this mode folds, so that the log-prob forward and the update's forward are the same arithmetic and the PPO
+    // ratio of unchanged weights is exactly 1 (the full-size parity tests assert it)
+    DPPO_TRY(ts_ensure_fold(h, net, s));
     ts_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(x, obs, trow, tconst, N, g.A, g.Do, g.T, KP0, obs_div, m.h0, split_null(), chainK);
     TC_KCHECK(h);
     const int r = ts_mlp_forward(h, s, m, N);
@@ -1773,7 +1718,7 @@ static int ts_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, flo
     TsMlp m; ts_critic_mlp(h, m);
     ts_mlp_take(h, N, m, false);
     m.out = v;
-    if (!ts_no_fold()) { DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, s)); m.fold = 1; }
+    DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, s));
     ts_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(nullptr, obs, nullptr, -1, N, g.A, g.Do, g.T, KP0, 1,
                                                                           m.fp == 4 ? m.h0 : split_null(), m.fp == 4 ? split_null() : m.h0, 0);
     TC_KCHECK(h);
@@ -1820,14 +1765,12 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     float* cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H); float* cpc = ws_take<float>(h, (size_t)nrb * 2 * g.Hc);
     float* gfold = ws_take<float>(h, (size_t)(g.H + g.Hc + 2 * KP0) * 32 + g.H + g.Hc);       // a1^T dout / h0^T dout of both nets (folded output layer) + scratch
     float* ga1 = gfold; float* ga0 = ga1 + (size_t)g.H * g.A; float* gc1 = ga0 + (size_t)KP0 * g.A; float* gc0 = gc1 + g.Hc;
-    const bool fold = !ts_no_fold();
-    ma.fold = mc.fold = fold ? 1 : 0;
     ma.out = eps; mc.out = val;
     // The critic's GEMMs are independent of the actor's until the loss (and again until the weight gradients) and their tiles are
     // short (K = 256: epilogue-latency-bound), while every persistent GEMM leaves SMs idle in its last wave: the critic (and the
     // advantage statistics, which only the loss kernel reads) run on a second stream and fill the actor kernels' tails.
     // (not while the per-kernel profile is on: its event brackets are meant to time each kernel running alone)
-    const bool side = h->overlap_chains && !h->prof_on;
+    const bool side = !h->prof_on;
     cudaStream_t sc = s;
     if (side) {
         if (!h->aux_stream) {
@@ -1856,10 +1799,8 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
         CUDA_TRY(cudaStreamWaitEvent(sc, h->aux_ev[0], 0));
     }
     // the folded output layers of the current weights (stale after every AdamW step): on the second stream, under the actor's L0 / L1
-    if (fold) {
-        DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR_FT, sc)); DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, sc));
-        if (side) { CUDA_TRY(cudaEventRecord(h->aux_ev[2], sc)); ma.fold_ev = h->aux_ev[2]; }      // the actor's stream waits in front of its folded GEMM only
-    }
+    DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR_FT, sc)); DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, sc));
+    if (side) { CUDA_TRY(cudaEventRecord(h->aux_ev[2], sc)); ma.fold_ev = h->aux_ev[2]; }      // the actor's stream waits in front of its folded GEMM only
     if (adv_std < 0.f) {
         if (idx) adv_stats_kernel<<<1, 1024, 0, sc>>>(idx->adv, N, h->scalars, idx->flat, idx->K, idx->P);
         else adv_stats_kernel<<<1, 1024, 0, sc>>>(advantages, N, h->scalars);
@@ -1895,35 +1836,27 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     DPPO_TRY(ts_mlp_backward_dx(h, sc, mc, dvalb, N, cpc));
     DPPO_TRY(join());
     tsp::DwDesc dd[10];
-    const int nda = ts_mlp_dw_descs(ma, depsb, N, gr, g.ao.w1, g.ao.w2, g.ao.w3, dw0a, dd, ga1, ga0);
-    const int ndc = ts_mlp_dw_descs(mc, dvalb, N, gr + nA, g.co.w1, g.co.w2, g.co.w3, dw0c, dd + nda, gc1, gc0);
-    DPPO_TRY(tsp::launch_dw_group(h, s, dd, nda + ndc, N, part, pf, ebeg));
+    const int nda = ts_mlp_dw_descs(ma, depsb, N, gr, g.ao.w1, dw0a, dd, ga1, ga0);
+    const int ndc = ts_mlp_dw_descs(mc, dvalb, N, gr + nA, g.co.w1, dw0c, dd + nda, gc1, gc0);
+    DPPO_TRY(tsp::launch_dw_pair(h, s, dd, nda + ndc, N, part, pf, ebeg));
     // everything dv would have fed (dW3, dW2, db2, the residual share of dw0) from the two small products; before the tail, which reads dw0
     // (the dw0 / db2 rows first, on this stream; dW3 and dW2 - which only AdamW reads - beside the tail kernel on the second stream)
-    if (fold) {
-        DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 0));
-        DPPO_TRY(fork());
-        DPPO_TRY(ts_dw3_assemble(h, sc, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 1));
-    }
-    float* b2scr = fold ? gfold + (size_t)(g.H + g.Hc + 2 * KP0) * 32 : nullptr;      // the unwritten slot-0 column sums land here, not in db2
-    static int split_tail = -1;     // dev knob DPPO_TS_SPLIT_TAIL=1: the tail's roles as separate launches (to time them one by one)
-    if (split_tail < 0) { const char* e = getenv("DPPO_TS_SPLIT_TAIL"); split_tail = (e && atoi(e)) ? 1 : 0; }
-    if (loss8 && !split_tail) {
-        DPPO_TRY(tc_launch_tail(h, s, bsum, nlb, hp.inv_nglobal, frac_local, colb3, cpa, nrb, cpc, nrb, dw0a, dw0c, b2scr, b2scr ? b2scr + g.H : nullptr));
-        if (fold) DPPO_TRY(join());
+    DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 0));
+    DPPO_TRY(fork());
+    DPPO_TRY(ts_dw3_assemble(h, sc, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 1));
+    float* b2scr = gfold + (size_t)(g.H + g.Hc + 2 * KP0) * 32;      // the unwritten slot-0 column sums land here, not in db2
+    if (loss8) {
+        DPPO_TRY(tc_launch_tail(h, s, bsum, nlb, hp.inv_nglobal, frac_local, colb3, cpa, nrb, cpc, nrb, dw0a, dw0c, b2scr, b2scr + g.H));
+        DPPO_TRY(join());
         return 0;
     }
-    if (fold) DPPO_TRY(join());
+    DPPO_TRY(join());
     // (unaligned / wide action rows) the same pieces as separate launches
     ppo_metrics_kernel<<<1, 256, 0, s>>>(bsum, nlb, hp.inv_nglobal, frac_local, gr + nA + nC); TC_KCHECK(h);
-    if (loss8) {
-        tc_reduce_cols_kernel<<<tc_nblk(g.A + 1, 8), 256, 0, s>>>(colb3, nlb, (size_t)(g.A + 1), g.A + 1, gr + g.ao.b3, g.A, gr + nA + g.co.b3); TC_KCHECK(h);
-    } else {
-        DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
-        DPPO_TRY(colsum(h, s, dval, 1, N, 1, nullptr, 1, part, gr + nA + g.co.b3));
-    }
-    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, b2scr ? b2scr : gr + g.ao.b2, g.H, gr + g.ao.b1); TC_KCHECK(h);
-    tc_reduce_cols_kernel<<<tc_nblk(2 * g.Hc, 8), 256, 0, s>>>(cpc, nrb, (size_t)2 * g.Hc, 2 * g.Hc, b2scr ? b2scr + g.H : gr + nA + g.co.b2, g.Hc, gr + nA + g.co.b1); TC_KCHECK(h);
+    DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
+    DPPO_TRY(colsum(h, s, dval, 1, N, 1, nullptr, 1, part, gr + nA + g.co.b3));
+    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, b2scr, g.H, gr + g.ao.b1); TC_KCHECK(h);
+    tc_reduce_cols_kernel<<<tc_nblk(2 * g.Hc, 8), 256, 0, s>>>(cpc, nrb, (size_t)2 * g.Hc, 2 * g.Hc, b2scr + g.H, g.Hc, gr + nA + g.co.b1); TC_KCHECK(h);
     const float* w = h->net_w[DPPO_NET_ACTOR_FT]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR_FT];
     const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
     time_backward_kernel<<<1 + (g.H + 127) / 128, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, dw0a + (size_t)(g.A + g.Do) * g.H, d.sinemb, d.thpre, d.temb, gr); TC_KCHECK(h);
@@ -1949,7 +1882,7 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     TsMlp ma; ts_actor_mlp(h, DPPO_NET_ACTOR, ma);
     ts_mlp_take(h, N, ma, true);
     float* ga1 = ws_take<float>(h, (size_t)(g.H + KP0) * 32 + g.H); float* ga0 = ga1 + (size_t)g.H * g.A;     // + scratch for the unwritten slot-0 sums
-    if (!ts_no_fold()) { DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR, s)); ma.fold = 1; }
+    DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR, s));
     float* eps = ws_take<float>(h, ne); float* deps = ws_take<float>(h, ne); float* noise = ws_take<float>(h, ne); float* xn = ws_take<float>(h, ne);
     int* trow = ws_take<int>(h, N);
     SplitT depsb = ts_take(h, (size_t)N * 64, 2);
@@ -1968,10 +1901,10 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     ts_pad64_kernel<<<tc_nblk((size_t)N * 8, 256), 256, 0, s>>>(deps, N, g.A, depsb.p[0], depsb.p[1]); TC_KCHECK(h);
     DPPO_TRY(ts_mlp_backward_dx(h, s, ma, depsb, N, cpa));
     tsp::DwDesc dd[5];
-    const int nd = ts_mlp_dw_descs(ma, depsb, N, gr, g.ao.w1, g.ao.w2, g.ao.w3, dw0, dd, ga1, ga0);
-    DPPO_TRY(tsp::launch_dw_group(h, s, dd, nd, N, part, pf, ebeg));
-    if (ma.fold) DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR, ga1, ga0, gr, dw0, nullptr, nullptr, nullptr, nullptr));
-    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ma.fold ? ga1 + (size_t)(g.H + KP0) * 32 : gr + g.ao.b2, g.H, gr + g.ao.b1); TC_KCHECK(h);
+    const int nd = ts_mlp_dw_descs(ma, depsb, N, gr, g.ao.w1, dw0, dd, ga1, ga0);
+    DPPO_TRY(tsp::launch_dw_pair(h, s, dd, nd, N, part, pf, ebeg));
+    DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR, ga1, ga0, gr, dw0, nullptr, nullptr, nullptr, nullptr));
+    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ga1 + (size_t)(g.H + KP0) * 32, g.H, gr + g.ao.b1); TC_KCHECK(h);
     DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
     const float* w = h->net_w[DPPO_NET_ACTOR]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR];
     const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
