@@ -156,7 +156,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dw_pair_kernel(const __grid_co
                     for (int j = 0; j < 32; ++j) if (n0 + j < P.N_valid) atomicAdd(P.out + (size_t)(n0 + j) * P.ld_out + m, __uint_as_float(r[j]));
                 } else {
                     float* dst = P.out + (size_t)m * P.ld_out + n0;
-                    if (n0 + 32 <= P.N_valid && (P.ld_out & 3) == 0) {
+                    if (n0 + 32 <= P.N_valid && (P.ld_out & 3) == 0 && ((uintptr_t)dst & 15) == 0) {   // (a net's slice of the flat gradient need not start 16-byte aligned)
 #pragma unroll
                         for (int q = 0; q < 8; ++q)
                             asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + q * 4), "f"(__uint_as_float(r[q * 4])), "f"(__uint_as_float(r[q * 4 + 1])),

@@ -328,7 +328,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                     }
                     if (e.out_f32 && e.f32_atomic) {
                         float* dst = e.out_f32 + (size_t)m * e.ld_f32 + n0;
-                        if (full32 && (e.ld_f32 & 3) == 0) {
+                        if (full32 && (e.ld_f32 & 3) == 0 && ((uintptr_t)dst & 15) == 0) {   // (a net's slice of the flat gradient need not start 16-byte aligned)
 #pragma unroll
                             for (int q = 0; q < 8; ++q)
                                 asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + q * 4), "f"(v[q * 4]), "f"(v[q * 4 + 1]), "f"(v[q * 4 + 2]), "f"(v[q * 4 + 3]) : "memory");
@@ -337,7 +337,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                         }
                     } else if (e.out_f32) {
                         float* dst = e.out_f32 + (size_t)split * e.split_stride + (size_t)m * e.ld_f32 + n0;
-                        if (full32 && (e.ld_f32 & 3) == 0) {
+                        if (full32 && (e.ld_f32 & 3) == 0 && ((uintptr_t)dst & 15) == 0) {
 #pragma unroll
                             for (int q = 0; q < 8; ++q)
                                 *reinterpret_cast<float4*>(dst + q * 4) = make_float4(v[q * 4], v[q * 4 + 1], v[q * 4 + 2], v[q * 4 + 3]);
