@@ -123,11 +123,28 @@ struct Geom {
 };
 
 // derived, recomputed after every weight change of that net
+// programmatic dependent launch for the short kernels at the end of an update: launch_pdl lets the kernel start while the previous
+// kernel of the stream drains (hiding the launch gap); such a kernel calls pdl_grid_begin() before it touches global memory, which
+// waits until the previous grids have completed and their writes are visible, then lets its own dependent launch early
+__device__ __forceinline__ void pdl_grid_begin() {
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s; cfg.attrs = at; cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
 struct ActorDerived {
     float* sinemb;  // [T][td]
     float* thpre;   // [T][2td]
     float* temb;    // [T][td]
     float* bt;      // [T][H]   = b_in + temb(t) @ W_in[A:A+td]
+    float* dte;     // [T][td] + a counter: scratch of the time-MLP backward (time_backward_body)
     float* w0p;     // [KP][H]  = rows of W_in for [x | obs], zero padded
     // no activation sits between block.l2 and the output layer: eps = (a1 W2 + b2 + u) W3 + b3 = a1 (W2 W3) + u W3 + (b2 W3 + b3).
     // Forward-only programs (the samplers, the log-prob forward) use the folded operands and skip the H x H product.

@@ -281,6 +281,7 @@ static int dppo_create_impl(const dppo_cfg* cfg, int device, dppo_handle** out, 
         CUDA_TRY(cudaMalloc(&d.thpre, (size_t)g.T * 2 * g.td * sizeof(float)));
         CUDA_TRY(cudaMalloc(&d.temb, (size_t)g.T * g.td * sizeof(float)));
         CUDA_TRY(cudaMalloc(&d.bt, (size_t)g.T * g.H * sizeof(float)));
+        CUDA_TRY(cudaMalloc(&d.dte, ((size_t)g.T * g.td + 4) * sizeof(float))); CUDA_TRY(cudaMemset(d.dte, 0, ((size_t)g.T * g.td + 4) * sizeof(float)));
         CUDA_TRY(cudaMalloc(&d.w23, (size_t)g.H * g.A * sizeof(float))); CUDA_TRY(cudaMalloc(&d.b23, (size_t)g.A * sizeof(float)));
         CUDA_TRY(cudaMalloc(&d.w0p, (size_t)g.KP * g.H * sizeof(float)));
     }
@@ -326,7 +327,7 @@ extern "C" void dppo_destroy(dppo_handle* h) {
     cudaFree(h->env_norm);
     cudaFree(h->params); cudaFree(h->sched); cudaFree(h->grads_buf[0]); cudaFree(h->grads_buf[1]); /* gsum lives inside grads_buf[1] */ cudaFree(h->flags); cudaFree(h->scalars);
     for (int i = 0; i < 2; ++i) { cudaFree(h->opt[i].m); cudaFree(h->opt[i].v); }
-    for (int net = 0; net < 4; ++net) { ActorDerived& d = h->ad[net]; cudaFree(d.sinemb); cudaFree(d.thpre); cudaFree(d.temb); cudaFree(d.bt); cudaFree(d.w0p); cudaFree(d.w23); cudaFree(d.b23); }
+    for (int net = 0; net < 4; ++net) { ActorDerived& d = h->ad[net]; cudaFree(d.sinemb); cudaFree(d.thpre); cudaFree(d.temb); cudaFree(d.bt); cudaFree(d.dte); cudaFree(d.w0p); cudaFree(d.w23); cudaFree(d.b23); }
     if (h->ws.base) cudaFree(h->ws.base);
     if (h->copy_stream) { cudaStreamDestroy(h->copy_stream); for (int i = 0; i < 9; ++i) cudaEventDestroy(h->copy_ev[i]); }
     if (h->aux_stream) { cudaStreamDestroy(h->aux_stream); for (int i = 0; i < 3; ++i) if (h->aux_ev[i]) cudaEventDestroy(h->aux_ev[i]); }
@@ -507,11 +508,10 @@ static void bwd_take(dppo_handle* h, int N, int KP, int H, int nseg, BwdBufs& b,
 }
 static int actor_bwd_fp32(dppo_handle* h, cudaStream_t s, int net, const FwdBufs& f, const float* deps, int N, const int* trow,
                           BwdBufs& b, float* Gseg, float* dw0p, float* gnet) {
-    const Geom& g = h->g; const float* w = h->net_w[net]; const ActorDerived& d = h->ad[net];
+    const Geom& g = h->g; const float* w = h->net_w[net];
     DPPO_TRY(mlp_bwd_fp32(h, s, w, g.ao.w1, g.ao.b1, g.ao.w2, g.ao.b2, g.ao.w3, g.ao.b3, h->cfg.actor_act + 1, f, deps, N,
                           g.KP, g.H, g.A, trow, g.T, b, gnet, dw0p, Gseg));
-    size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
-    time_backward_kernel<<<1, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, Gseg, d.sinemb, d.thpre, d.temb, gnet); KLAUNCH(h); KCHECK();
+    CUDA_TRY(launch_time_backward(h, s, net, Gseg, gnet)); KLAUNCH(h);
     unpack_dw0_kernel<<<nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0p, g.A, g.td, g.Do, g.H, gnet + g.ao.win); KLAUNCH(h); KCHECK();
     return 0;
 }
@@ -965,12 +965,17 @@ extern "C" int dppo_comm_status(dppo_handle* h) {
 }
 
 // ------------------------------------------------------------------ AdamW
-static int adam_apply(dppo_handle* h, cudaStream_t s, int opt, float* w, const float* g, size_t n, float lr, float wd) {
+// advances optimizer `opt` by one step and returns that step's bias-corrected step size
+static float adam_next_alpha(dppo_handle* h, int opt, float lr) {
     OptState& o = h->opt[opt];
     o.step += 1;
+    const float b1p = powf(h->cfg.adam_beta1, (float)o.step), b2p = powf(h->cfg.adam_beta2, (float)o.step);
+    return lr * sqrtf(1.f - b2p) / (1.f - b1p);
+}
+static int adam_apply(dppo_handle* h, cudaStream_t s, int opt, float* w, const float* g, size_t n, float lr, float wd) {
+    OptState& o = h->opt[opt];
     const float b1 = h->cfg.adam_beta1, b2 = h->cfg.adam_beta2;
-    float b1p = powf(b1, (float)o.step), b2p = powf(b2, (float)o.step);
-    float alpha = lr * sqrtf(1.f - b2p) / (1.f - b1p);
+    const float alpha = adam_next_alpha(h, opt, lr);
     adamw_kernel<<<nblk(n, 256), 256, 0, s>>>(w, g, o.m, o.v, n, lr, alpha, b1, b2, h->cfg.adam_eps, wd, h->skip_update, nullptr); KLAUNCH(h); KCHECK();
     return 0;
 }
@@ -978,9 +983,13 @@ static int adam_apply(dppo_handle* h, cudaStream_t s, int opt, float* w, const f
 // ------------------------------------------------------------------ PPO step
 static int prep_net(dppo_handle* h, int net, cudaStream_t s);
 // all-reduce (if a communicator is attached) + AdamW + derived-table refresh + metric / gradient read-out
+// The split-precision mode applies AdamW and rebuilds every derived table in ONE launch (ts_apply_update) after a local or NCCL
+// reduction; with gradient clipping or the peer-memory exchange (whose kernel fuses the reduction with AdamW) it keeps the separate
+// AdamW launch and prep_net, like the other modes.
 static int ppo_apply_tail(dppo_handle* h, cudaStream_t s, float lr, int apply, float* metrics8, float* grads_out) {
     const size_t nA = h->g.ao.n, nC = h->g.co.n; float* gr = h->grads;
     if (apply) {
+        bool tables_done = false;
         // actor_ft and critic are contiguous in `params` and share one optimizer (train_ppo_diffusion_agent.py:354-356)
         if (h->grad_clip_norm > 0.f) {
             // clipping needs the norms of the REDUCED gradient before the update: reduce, (hand out the unclipped gradient), clip, update
@@ -998,9 +1007,15 @@ static int ppo_apply_tail(dppo_handle* h, cudaStream_t s, float lr, int apply, f
             gr = h->gsum;
         } else {
             DPPO_TRY(allreduce_sum(h, gr, nA + nC + 8, s));
-            DPPO_TRY(adam_apply(h, s, DPPO_OPT_FINETUNE, h->net_w[DPPO_NET_ACTOR_FT], gr, nA + nC, lr, h->cfg.weight_decay));
+            if (ts_update_ok(h)) {
+                DPPO_TRY(ts_apply_update(h, s, gr, lr, adam_next_alpha(h, DPPO_OPT_FINETUNE, lr), h->cfg.weight_decay, nullptr));
+                tables_done = true;
+            } else {
+                DPPO_TRY(adam_apply(h, s, DPPO_OPT_FINETUNE, h->net_w[DPPO_NET_ACTOR_FT], gr, nA + nC, lr, h->cfg.weight_decay));
+            }
         }
-        if (h->cfg.precision == DPPO_PREC_BF16 && tc_shapes_ok(h) && 2 * h->g.td <= 256) {
+        if (tables_done) {
+        } else if (h->cfg.precision == DPPO_PREC_BF16 && tc_shapes_ok(h) && 2 * h->g.td <= 256) {
             DPPO_TRY(tc_prep_pack_ft_critic(h, s));
         } else {
             DPPO_TRY(prep_net(h, DPPO_NET_ACTOR_FT, s));

@@ -231,7 +231,11 @@ __global__ void reduce_partials_kernel(const float* __restrict__ part, int S, si
 //   modules.py:10-15, mlp_diffusion.py:40-45,83-86.  grid = T blocks of H threads (H <= 1024).
 // =====================================================================================
 // bt16 (optional): the same table rounded to bf16, written straight into the time rows of the packed layer-0 operand
-__device__ __forceinline__ void actor_prep_body(const int t, float* sm, const float* __restrict__ w, ActorOff o, int A, int td, int H,
+// w(i): parameter i of the actor's flat vector (WRead: as stored; the fused update of the split-precision mode passes the
+// AdamW-updated values)
+struct WRead { const float* __restrict__ p; __device__ __forceinline__ float operator()(size_t i) const { return p[i]; } };
+template <class WF>
+__device__ __forceinline__ void actor_prep_body(const int t, float* sm, const WF w, ActorOff o, int A, int td, int H,
                                   float* __restrict__ sinemb, float* __restrict__ thpre,
                                   float* __restrict__ temb, float* __restrict__ bt, __nv_bfloat16* __restrict__ bt16) {
     float* se = sm;            // [td]
@@ -248,21 +252,21 @@ __device__ __forceinline__ void actor_prep_body(const int t, float* sm, const fl
     }
     __syncthreads();
     if (tid < 2 * td) {
-        float s = w[o.tb1 + tid];
-        for (int j = 0; j < td; ++j) s = fmaf(se[j], w[o.tw1 + (size_t)j * 2 * td + tid], s);
+        float s = w(o.tb1 + tid);
+        for (int j = 0; j < td; ++j) s = fmaf(se[j], w(o.tw1 + (size_t)j * 2 * td + tid), s);
         thpre[t * 2 * td + tid] = s;
         hp[tid] = mish_f(s);
     }
     __syncthreads();
     if (tid < td) {
-        float s = w[o.tb2 + tid];
-        for (int j = 0; j < 2 * td; ++j) s = fmaf(hp[j], w[o.tw2 + (size_t)j * td + tid], s);
+        float s = w(o.tb2 + tid);
+        for (int j = 0; j < 2 * td; ++j) s = fmaf(hp[j], w(o.tw2 + (size_t)j * td + tid), s);
         te[tid] = s; temb[t * td + tid] = s;
     }
     __syncthreads();
     for (int c = tid; c < H; c += blockDim.x) {
-        float s = w[o.bin + c];
-        for (int j = 0; j < td; ++j) s = fmaf(te[j], w[o.win + (size_t)(A + j) * H + c], s);
+        float s = w(o.bin + c);
+        for (int j = 0; j < td; ++j) s = fmaf(te[j], w(o.win + (size_t)(A + j) * H + c), s);
         bt[(size_t)t * H + c] = s;
         if (bt16) bt16[(size_t)t * H + c] = __float2bfloat16(s);
     }
@@ -271,7 +275,7 @@ __global__ void actor_prep_kernel(const float* __restrict__ w, ActorOff o, int A
                                   float* __restrict__ sinemb, float* __restrict__ thpre,
                                   float* __restrict__ temb, float* __restrict__ bt) {
     extern __shared__ float sm[];
-    actor_prep_body(blockIdx.x, sm, w, o, A, td, H, sinemb, thpre, temb, bt, nullptr);
+    actor_prep_body(blockIdx.x, sm, WRead{w}, o, A, td, H, sinemb, thpre, temb, bt, nullptr);
 }
 // w23[k][a] = sum_j W2[k][j] W3[j][a] (k < H), b23[a] = b3[a] + sum_j b2[j] W3[j][a] (the thread row k == H): products of the folded output
 // layer (MLP / ResidualMLP of model/common/mlp.py: the last Dense follows the residual add without an activation)
@@ -653,29 +657,30 @@ __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ D
     for (int i = threadIdx.x; i < nseg * ncols; i += blockDim.x) part[(size_t)blockIdx.x * nseg * ncols + i] = sm[i];
 }
 
-// time-MLP + layer-0 bias backward from G[T][H] = per-t column sums of du.  One block, 512 threads.
-// `bid` of `nblk` blocks (a stand-alone launch or a block range of the merged tail kernel).  `staged`: sm also has room for
-// G [T][H] and the td time rows of W_in [td][H]; block 0 then reads them once, coalesced, instead of walking L2 per t.
-__device__ __forceinline__ void time_backward_body(const int bid, const int nblk, float* sm, const bool staged,
+// time-MLP + layer-0 bias backward from G[T][H] = per-t column sums of du, on time_backward_grid() blocks of 512 threads
+// (`bid` of a stand-alone launch or of a block range of the merged tail kernel):
+//  * blocks [0, T): dte[t][j] = sum_c W_in[A+j][c] G[t][c] for t = bid, one warp per j (lane-strided columns, butterfly), into
+//    dte_g [T][td]; the LAST of these blocks to finish (counter dte_g[T*td], left at zero) runs the time MLP's backward from the
+//    T rows: dh, dW2 / dW1 of the time MLP and their biases, every operand in shared memory (the T-long loops of a single block
+//    walking L2 were the whole cost of the first version: ~58 k cycles);
+//  * blocks [T, ..): db_in and the td time rows of dW_in for 32 columns each, 16 threads per column over j.
+// Every output keeps the summation order of the single-block version (t ascending; c ascending per lane, then the butterfly).
+__device__ __forceinline__ void time_backward_body(const int bid, float* sm,
                                      const float* __restrict__ w, ActorOff o, int A, int td, int H, int T,
                                      const float* __restrict__ G, const float* __restrict__ sinemb,
                                      const float* __restrict__ thpre, const float* __restrict__ temb,
-                                     float* __restrict__ g) {
-    float* dte = sm;                 // [T][td]
-    float* dh = dte + T * td;        // [T][2td]
+                                     float* __restrict__ dte_g, float* __restrict__ g) {
     const int tid = threadIdx.x, nt = blockDim.x;
-    // gridDim.x == 1: one block does everything.  Otherwise block 0 does the time-MLP part and blocks 1.. split the
-    // per-column part (db_in and dW_in[A+j]) 128 columns each, 4 threads per column over j.
-    if (nblk == 1 || bid > 0) {
-        const int c0 = nblk == 1 ? 0 : (bid - 1) * 128, c1 = nblk == 1 ? H : min(H, c0 + 128);
-        const int lanes = nblk == 1 ? 1 : 4;            // threads per column
+    if (bid >= T) {
+        const int lanes = 16;                           // threads per column
+        const int c0 = (bid - T) * (nt / lanes), c1 = min(H, c0 + nt / lanes);
         for (int i = tid; i < (c1 - c0) * lanes; i += nt) {
             const int c = c0 + i / lanes, part = i % lanes;
             // the T values of column c are loaded up front (independent loads: one L2 latency instead of T)
             float bsum = 0.f;
-            float acc[16];
+            float acc[2];
 #pragma unroll
-            for (int q = 0; q < 16; ++q) acc[q] = 0.f;
+            for (int q = 0; q < 2; ++q) acc[q] = 0.f;
             for (int t0 = 0; t0 < T; t0 += 32) {
                 float gc[32];
 #pragma unroll
@@ -683,7 +688,7 @@ __device__ __forceinline__ void time_backward_body(const int bid, const int nblk
 #pragma unroll
                 for (int q = 0; q < 32; ++q) bsum += gc[q];
 #pragma unroll
-                for (int jj = 0; jj < 16; ++jj) {
+                for (int jj = 0; jj < 2; ++jj) {
                     const int j = part + jj * lanes;
                     if (j < td) {
 #pragma unroll
@@ -692,51 +697,54 @@ __device__ __forceinline__ void time_backward_body(const int bid, const int nblk
                 }
             }
             if (part == 0) g[o.bin + c] = bsum;
-            for (int jj = 0; jj < 16; ++jj) {
+            for (int jj = 0; jj < 2; ++jj) {
                 const int j = part + jj * lanes;
                 if (j < td) g[o.win + (size_t)(A + j) * H + c] = acc[jj];
             }
-            // time_dim > 16 * lanes columns per thread do not fit the register tile: plain loop for the rest
-            for (int j = part + 16 * lanes; j < td; j += lanes) {
+            // time_dim > 2 * lanes: plain loop for the rest
+            for (int j = part + 2 * lanes; j < td; j += lanes) {
                 float a = 0.f;
                 for (int t = 0; t < T; ++t) a = fmaf(temb[t * td + j], G[(size_t)t * H + c], a);
                 g[o.win + (size_t)(A + j) * H + c] = a;
             }
         }
-        if (nblk > 1) return;
+        return;
     }
-    // d temb[t][j] = sum_c W_in[A+j][c] * G[t][c]: one warp per j keeps its W_in row in registers (H <= 1024) and walks t;
-    // the H/32 loads of a step are independent, so the load latency is paid ~T times, not T*H/32 times
-    if (staged) {
-        float* sG = dh + T * 2 * td;   // [T][H]
-        float* sW = sG + T * H;        // [td][H]: rows A .. A+td of W_in are contiguous
-        for (int i = tid; i < T * H; i += nt) sG[i] = G[i];
-        for (int i = tid; i < td * H; i += nt) sW[i] = w[o.win + (size_t)A * H + i];
-        __syncthreads();
-        const int lane = tid & 31;
-        for (int p = tid >> 5; p < T * td; p += nt >> 5) {       // same summation order as the register-tiled loop below
-            const int t = p / td, j = p % td;
-            float s = 0.f;
-            for (int c = lane; c < H; c += 32) s = fmaf(sW[j * H + c], sG[t * H + c], s);
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-            if (lane == 0) dte[t * td + j] = s;
-        }
-    } else
-    for (int j = tid >> 5; j < td; j += nt >> 5) {
-        const int lane = tid & 31;
-        float wr[32];
-#pragma unroll
-        for (int q = 0; q < 32; ++q) { const int c = lane + q * 32; wr[q] = c < H ? w[o.win + (size_t)(A + j) * H + c] : 0.f; }
-        for (int t = 0; t < T; ++t) {
+    // d temb[t][j]: a warp walks its W_in row and the G row (H <= 1024)
+    {
+        const int t = bid, lane = tid & 31;
+        for (int j = tid >> 5; j < td; j += nt >> 5) {
             float s = 0.f;
 #pragma unroll
-            for (int q = 0; q < 32; ++q) { const int c = lane + q * 32; if (c < H) s = fmaf(wr[q], G[(size_t)t * H + c], s); }
+            for (int q0 = 0; q0 < 32; q0 += 16) {       // 16 columns of both rows in flight at once
+                float wr[16], gv[16];
+#pragma unroll
+                for (int q = 0; q < 16; ++q) {
+                    const int c = lane + (q0 + q) * 32;
+                    wr[q] = c < H ? w[o.win + (size_t)(A + j) * H + c] : 0.f;
+                    gv[q] = c < H ? G[(size_t)t * H + c] : 0.f;
+                }
+#pragma unroll
+                for (int q = 0; q < 16; ++q) { const int c = lane + (q0 + q) * 32; if (c < H) s = fmaf(wr[q], gv[q], s); }
+            }
 #pragma unroll
             for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-            if (lane == 0) dte[t * td + j] = s;
+            if (lane == 0) dte_g[t * td + j] = s;
         }
     }
+    __shared__ int last_flag;
+    int* done = reinterpret_cast<int*>(dte_g + T * td);
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) last_flag = (atomicAdd(done, 1) == T - 1) ? 1 : 0;
+    __syncthreads();
+    if (!last_flag) return;
+    __threadfence();
+    float* dte = sm;                 // [T][td]
+    float* dh = dte + T * td;        // [T][2td]
+    float* mt = dh + T * 2 * td;     // [T][2td] mish(thpre)
+    for (int i = tid; i < T * td; i += nt) dte[i] = __ldcg(dte_g + i);
+    for (int i = tid; i < T * 2 * td; i += nt) mt[i] = mish_f(thpre[i]);
     __syncthreads();
     for (int i = tid; i < T * 2 * td; i += nt) {    // d hidden pre-activation
         int t = i / (2 * td), k = i % (2 * td);
@@ -748,7 +756,7 @@ __device__ __forceinline__ void time_backward_body(const int bid, const int nblk
     for (int i = tid; i < 2 * td * td; i += nt) {   // dW2[k][j], dW1[s][k]
         int k = i / td, j = i % td;
         float s = 0.f;
-        for (int t = 0; t < T; ++t) s = fmaf(mish_f(thpre[t * 2 * td + k]), dte[t * td + j], s);
+        for (int t = 0; t < T; ++t) s = fmaf(mt[t * 2 * td + k], dte[t * td + j], s);
         g[o.tw2 + i] = s;
         int ss = i / (2 * td), kk = i % (2 * td);
         float a = 0.f;
@@ -757,13 +765,29 @@ __device__ __forceinline__ void time_backward_body(const int bid, const int nblk
     }
     for (int j = tid; j < td; j += nt) { float s = 0.f; for (int t = 0; t < T; ++t) s += dte[t * td + j]; g[o.tb2 + j] = s; }
     for (int k = tid; k < 2 * td; k += nt) { float s = 0.f; for (int t = 0; t < T; ++t) s += dh[t * 2 * td + k]; g[o.tb1 + k] = s; }
+    if (tid == 0) *done = 0;                         // ready for the next launch
 }
 __global__ void __launch_bounds__(512) time_backward_kernel(const float* __restrict__ w, ActorOff o, int A, int td, int H, int T,
                                      const float* __restrict__ G, const float* __restrict__ sinemb,
                                      const float* __restrict__ thpre, const float* __restrict__ temb,
-                                     float* __restrict__ g) {
+                                     float* __restrict__ dte_g, float* __restrict__ g) {
     extern __shared__ float sm[];
-    time_backward_body(blockIdx.x, gridDim.x, sm, false, w, o, A, td, H, T, G, sinemb, thpre, temb, g);
+    time_backward_body(blockIdx.x, sm, w, o, A, td, H, T, G, sinemb, thpre, temb, dte_g, g);
+}
+static inline int time_backward_grid(const Geom& g) { return g.T + (g.H + 31) / 32; }
+static inline size_t time_backward_smem(const Geom& g) { return (size_t)5 * g.T * g.td * sizeof(float); }
+// the time-MLP / layer-0 bias backward of actor `net` from G [T][H] into its gradient slice gnet
+static cudaError_t launch_time_backward(const dppo_handle* h, cudaStream_t s, int net, const float* G, float* gnet) {
+    static bool attr_set_dev[64] = {};
+    const Geom& g = h->g; const ActorDerived& d = h->ad[net];
+    const size_t sm = time_backward_smem(g);
+    if (sm > 48 * 1024 && !attr_set_dev[h->device & 63]) {
+        const cudaError_t e = cudaFuncSetAttribute(time_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        if (e != cudaSuccess) return e;
+        attr_set_dev[h->device & 63] = true;
+    }
+    time_backward_kernel<<<time_backward_grid(g), 512, sm, s>>>(h->net_w[net], g.ao, g.A, g.td, g.H, g.T, G, d.sinemb, d.thpre, d.temb, d.dte, gnet);
+    return cudaGetLastError();
 }
 // scatter dW0p[KP][H] rows back into dW_in: k < A -> row k; A <= k < A+Do -> row k+skip
 __device__ __forceinline__ void unpack_dw0_body(const int bid, const float* __restrict__ dw0p, int A, int skip, int Do, int H, float* __restrict__ gwin) {
@@ -779,6 +803,13 @@ __global__ void unpack_dw0_kernel(const float* __restrict__ dw0p, int A, int ski
 // =====================================================================================
 // Keras-3 AdamW (decoupled decay first, then Adam with folded bias correction)
 // =====================================================================================
+// one element: every kernel that applies the update calls this, so that the arithmetic (and its contraction) cannot differ
+__device__ __forceinline__ void adamw_elem(float& p, float& mi, float& vi, float gi, float lr, float alpha, float b1, float b2, float eps, float wd) {
+    if (wd != 0.f) p = p - p * (wd * lr);
+    mi = mi + (gi - mi) * (1.f - b1);
+    vi = vi + (gi * gi - vi) * (1.f - b2);
+    p = p - mi * alpha / (sqrtf(vi) + eps);
+}
 // skip[0] | skip[1] != 0 (optional device flags: bad minibatch indices, a peer barrier that timed out): leave everything untouched
 __global__ void adamw_kernel(float* __restrict__ w, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                              size_t n, float lr, float alpha, float b1, float b2, float eps, float wd,
@@ -786,11 +817,8 @@ __global__ void adamw_kernel(float* __restrict__ w, const float* __restrict__ g,
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     if ((skip0 && *skip0) || (skip1 && *skip1)) return;
-    float p = w[i], gi = g[i], mi = m[i], vi = v[i];
-    if (wd != 0.f) p = p - p * (wd * lr);
-    mi = mi + (gi - mi) * (1.f - b1);
-    vi = vi + (gi * gi - vi) * (1.f - b2);
-    p = p - mi * alpha / (sqrtf(vi) + eps);
+    float p = w[i], mi = m[i], vi = v[i];
+    adamw_elem(p, mi, vi, g[i], lr, alpha, b1, b2, eps, wd);
     w[i] = p; m[i] = mi; v[i] = vi;
 }
 // tf.clip_by_norm on every variable of the flat gradient (train_ppo_diffusion_agent.py:352): one block per variable,

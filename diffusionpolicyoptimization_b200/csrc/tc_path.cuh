@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(256) tc_prep_pack_kernel(const TcPrepPackArgs 
     extern __shared__ float prep_sm[];
     const int b = blockIdx.x;
     if (b < a.T)
-        actor_prep_body(b, prep_sm, a.wa, a.ao, a.A, a.td, a.H, a.sinemb, a.thpre, a.temb, a.bt, a.a_w2w0 + (size_t)a.H * a.H + (size_t)(a.A + a.Do) * a.H);
+        actor_prep_body(b, prep_sm, WRead{a.wa}, a.ao, a.A, a.td, a.H, a.sinemb, a.thpre, a.temb, a.bt, a.a_w2w0 + (size_t)a.H * a.H + (size_t)(a.A + a.Do) * a.H);
     else if (b < a.T + a.na)
         tc_pack_actor_body((size_t)(b - a.T) * blockDim.x + threadIdx.x, (size_t)a.na * blockDim.x, a.wa, a.ao, a.A, a.td, a.Do, a.T, a.H, a.KP0, nullptr,
                            a.a_w2w0, a.a_w1, a.a_w3t, a.a_w3p, a.a_w1t, a.a_w2t);
@@ -254,11 +254,12 @@ struct TcTailArgs {
     const float* cpa; int rows_a; int HA; float* b2a; float* b1a;
     const float* cpc; int rows_c; int HC; float* b2c; float* b1c;
     // time backward
-    const float* w; ActorOff ao; int A, td, T, Do; int tb_staged; const float* Gt; const float* sinemb; const float* thpre; const float* temb; float* gr;
+    const float* w; ActorOff ao; int A, td, T, Do; const float* Gt; const float* sinemb; const float* thpre; const float* temb; float* dte; float* gr;
     // unpack
     const float* dw0a; float* gwin_a; const float* dw0c_obs; float* gwin_c; const float* dw0c_bias; float* gbin_c;
 };
 __global__ void __launch_bounds__(512) tc_ppo_tail_kernel(const TcTailArgs a) {
+    pdl_grid_begin();
     extern __shared__ float tail_sm[];
     const int b = blockIdx.x;
     if (b < a.first[1]) ppo_metrics_body(a.bsum, a.blocks_done, a.inv_nglobal, a.frac_local, a.metrics);
@@ -273,8 +274,7 @@ __global__ void __launch_bounds__(512) tc_ppo_tail_kernel(const TcTailArgs a) {
         if (a.wide) tc_reduce_cols_wide_body(b - a.first[3], a.cpc, a.rows_c, (size_t)2 * a.HC, 2 * a.HC, a.b2c, a.HC, a.b1c);
         else tc_reduce_cols_body(b - a.first[3], a.cpc, a.rows_c, (size_t)2 * a.HC, 2 * a.HC, a.b2c, a.HC, a.b1c);
     }
-    else if (b < a.first[5]) time_backward_body(b - a.first[4], a.first[5] - a.first[4], tail_sm, a.tb_staged != 0, a.w, a.ao, a.A, a.td, a.HA, a.T,
-                                                a.Gt, a.sinemb, a.thpre, a.temb, a.gr);
+    else if (b < a.first[5]) time_backward_body(b - a.first[4], tail_sm, a.w, a.ao, a.A, a.td, a.HA, a.T, a.Gt, a.sinemb, a.thpre, a.temb, a.dte, a.gr);
     else if (b < a.first[6]) unpack_dw0_body(b - a.first[5], a.dw0a, a.A, a.td, a.Do, a.HA, a.gwin_a);
     else if (b < a.first[7]) unpack_dw0_body(b - a.first[6], a.dw0c_obs, 0, 0, a.Do, a.HC, a.gwin_c);
     else { const int i = (b - a.first[7]) * blockDim.x + threadIdx.x; if (i < a.HC) a.gbin_c[i] = a.dw0c_bias[i]; }
@@ -985,12 +985,11 @@ static int colsum(dppo_handle* h, cudaStream_t s, const float* D, int ld, int N,
 // actor backward from deps [N][A] fp32 (+ its padded bf16 copy): fills gnet[0 : nA]
 static int tc_actor_grads(dppo_handle* h, cudaStream_t s, int net, const TcMlp& m, const float* deps, const bf16* depsb, int N,
                           float* part, float* dw0, float* gnet) {
-    const Geom& g = h->g; const float* w = h->net_w[net]; const ActorDerived& d = h->ad[net];
+    const Geom& g = h->g;
     DPPO_TRY(tc_mlp_backward(h, s, m, depsb, N, part, gnet, g.ao.w1, g.ao.b1, g.ao.w2, g.ao.b2, g.ao.w3, dw0));
     if (deps) DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gnet + g.ao.b3));   // else: the loss kernel already reduced it
     // dw0 rows [A+Do, A+Do+T) are the per-t column sums of du: the gradient of the bt table
-    const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
-    time_backward_kernel<<<1, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, dw0 + (size_t)(g.A + g.Do) * g.H, d.sinemb, d.thpre, d.temb, gnet);
+    CUDA_TRY(launch_time_backward(h, s, net, dw0 + (size_t)(g.A + g.Do) * g.H, gnet));
     TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0, g.A, g.td, g.Do, g.H, gnet + g.ao.win);
     TC_KCHECK(h);
@@ -1199,9 +1198,8 @@ static int tc_launch_tail(dppo_handle* h, cudaStream_t s, const double* bsum, in
     const size_t nA = g.ao.n, nC = g.co.n;
     float* gr = h->grads;
     const float* w = h->net_w[DPPO_NET_ACTOR_FT]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR_FT];
-    const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
-    const size_t sm_staged = sm + (size_t)(g.T + g.td) * g.H * sizeof(float);
-    const bool staged = sm_staged <= 160 * 1024;
+    const size_t sm = time_backward_smem(g);
+    if (sm > 160 * 1024) DPPO_FAIL(-7, "tc_launch_tail: time_dim x denoising_steps too large");
     static bool attr_set_dev[64] = {};      // function attributes are per device
     bool& attr_set = attr_set_dev[h->device & 63];
     if (!attr_set) { CUDA_TRY(cudaFuncSetAttribute(tc_ppo_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024)); attr_set = true; }
@@ -1211,7 +1209,7 @@ static int tc_launch_tail(dppo_handle* h, cudaStream_t s, const double* bsum, in
     const int cpb = wide ? 32 : wpb;
     const bool wide3 = blocks_done >= 256;
     a.wide = wide ? 1 : 0; a.wide3 = wide3 ? 1 : 0;
-    const int nb[8] = {1, tc_nblk(g.A + 1, wide3 ? 32 : wpb), tc_nblk(2 * g.H, cpb), tc_nblk(2 * g.Hc, cpb), 1 + (g.H + 127) / 128,
+    const int nb[8] = {1, tc_nblk(g.A + 1, wide3 ? 32 : wpb), tc_nblk(2 * g.H, cpb), tc_nblk(2 * g.Hc, cpb), time_backward_grid(g),
                        tc_nblk((size_t)(g.A + g.Do) * g.H, nthr), tc_nblk((size_t)g.Do * g.Hc, nthr), tc_nblk(g.Hc, nthr)};
     a.first[0] = 0;
     for (int r = 0; r < 8; ++r) a.first[r + 1] = a.first[r] + nb[r];
@@ -1219,11 +1217,11 @@ static int tc_launch_tail(dppo_handle* h, cudaStream_t s, const double* bsum, in
     a.colb3 = colb3; a.ncol3 = g.A + 1; a.b3a = gr + g.ao.b3; a.split3 = g.A; a.b3c = gr + nA + g.co.b3;
     a.cpa = cpa; a.rows_a = rows_a; a.HA = g.H; a.b2a = b2a_out ? b2a_out : gr + g.ao.b2; a.b1a = gr + g.ao.b1;
     a.cpc = cpc; a.rows_c = rows_c; a.HC = g.Hc; a.b2c = b2c_out ? b2c_out : gr + nA + g.co.b2; a.b1c = gr + nA + g.co.b1;
-    a.w = w; a.ao = g.ao; a.A = g.A; a.td = g.td; a.T = g.T; a.Do = g.Do; a.tb_staged = staged ? 1 : 0;
-    a.Gt = dw0a + (size_t)(g.A + g.Do) * g.H; a.sinemb = d.sinemb; a.thpre = d.thpre; a.temb = d.temb; a.gr = gr;
+    a.w = w; a.ao = g.ao; a.A = g.A; a.td = g.td; a.T = g.T; a.Do = g.Do;
+    a.Gt = dw0a + (size_t)(g.A + g.Do) * g.H; a.sinemb = d.sinemb; a.thpre = d.thpre; a.temb = d.temb; a.dte = d.dte; a.gr = gr;
     a.dw0a = dw0a; a.gwin_a = gr + g.ao.win; a.dw0c_obs = dw0c + (size_t)g.A * g.Hc; a.gwin_c = gr + nA + g.co.win;
     a.dw0c_bias = dw0c + (size_t)(g.A + g.Do + g.T) * g.Hc; a.gbin_c = gr + nA + g.co.bin;
-    tc_ppo_tail_kernel<<<a.first[8], nthr, staged ? sm_staged : sm, s>>>(a); TC_KCHECK(h);
+    CUDA_TRY(launch_pdl(tc_ppo_tail_kernel, dim3(a.first[8]), dim3(nthr), sm, s, a)); TC_KCHECK(h);
     return 0;
 }
 static int tc_ppo_finish(dppo_handle* h, cudaStream_t s) {
@@ -1232,15 +1230,13 @@ static int tc_ppo_finish(dppo_handle* h, cudaStream_t s) {
     TcPpoPlan& P = tc_plan(h);
     float* gr = h->grads;
     const bool defer = P.ma.fused && P.mc.fused && !h->deterministic;
-    const float* w = h->net_w[DPPO_NET_ACTOR_FT]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR_FT];
-    const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
     if (defer) return tc_launch_tail(h, s, P.bsum, P.blocks_done, P.hp.inv_nglobal, (float)((double)P.N / (double)P.N_global), P.colb3,
                                      P.cpa, P.nchunks * h->sm_count, P.cpc, P.nchunks * h->sm_count, P.dw0a, P.dw0c);
     ppo_metrics_kernel<<<1, 256, 0, s>>>(P.bsum, P.blocks_done, P.hp.inv_nglobal, (float)((double)P.N / (double)P.N_global), gr + nA + nC); TC_KCHECK(h);
     // output-layer bias gradients = column sums of the seeds (per-block partials from the loss kernel)
     tc_reduce_cols_kernel<<<tc_nblk(g.A + 1, 8), 256, 0, s>>>(P.colb3, P.blocks_done, (size_t)(g.A + 1), g.A + 1, gr + g.ao.b3, g.A, gr + nA + g.co.b3); TC_KCHECK(h);
     // actor: dw0 rows [A+Do, A+Do+T) are the per-t column sums of du = the gradient of the bt table
-    time_backward_kernel<<<1 + (g.H + 127) / 128, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, P.dw0a + (size_t)(g.A + g.Do) * g.H, d.sinemb, d.thpre, d.temb, gr);
+    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR_FT, P.dw0a + (size_t)(g.A + g.Do) * g.H, gr));
     TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(P.dw0a, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
     // critic: obs rows of dw0 -> dW_in; the ones column of h0 collected the input-layer bias gradient

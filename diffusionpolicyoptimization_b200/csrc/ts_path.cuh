@@ -1194,18 +1194,22 @@ struct TsFoldArgs {
     const float* bt;                          // rows of h0 columns [A + Do, A + Do + T): bt + (k0 - A - Do) * H, or null
     int A, Do, T, H, NO, KP0, f16;
 };
-// one warp per output row k (k == H + KP0: the bias row): the lanes split j (16 products each, fp32), W3 sits transposed and padded in
-// shared memory (conflict-free both ways), the lane partials meet in a butterfly.  (A first version accumulated in double: 30 us - the
-// CUDA-core fp64 rate of this part - for sums that are rounded to 22-bit planes anyway.)
+// one warp per output row k (k == H + KP0: the bias row) and 8-column group a0 = 8 blockIdx.y of the output: the lanes split j (16
+// products each, fp32), the group's 8 columns of W3 sit transposed and padded in shared memory (conflict-free both ways), the lane
+// partials meet in a butterfly.  (A first version accumulated in double: 30 us - the CUDA-core fp64 rate of this part - for sums that
+// are rounded to 22-bit planes anyway.  One block per 8 rows for all 64 columns: 20 us on 73 blocks; split by column group the launch
+// has 8x the blocks and each stages an eighth of W3.)
 __global__ void __launch_bounds__(256) ts_fold_kernel(const TsFoldArgs f, const TsW F, float* __restrict__ bfold, const TsW B23) {
-    extern __shared__ float w3t[];               // [NO][H + 1]
-    const int H = f.H, NO = f.NO, ld = f.H + f.KP0, HP = f.H + 1;
-    for (int i0 = threadIdx.x; i0 < H * NO; i0 += blockDim.x * 8) {        // eight loads in flight per thread (one per iteration: 29 us of latency)
+    pdl_grid_begin();
+    extern __shared__ float w3t[];               // [8][H + 1]: columns a0 .. a0 + 7 of W3
+    const int H = f.H, NO = f.NO, ld = f.H + f.KP0, HP = f.H + 1, a0 = 8 * blockIdx.y;
+    const int nq = min(8, NO - a0);              // columns of this group inside the layer (<= 0: the zero padding)
+    for (int i0 = threadIdx.x; i0 < H * 8; i0 += blockDim.x * 8) {         // eight loads in flight per thread
         float t8[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; t8[u] = i < H * NO ? __ldg(f.w3 + i) : 0.f; }
+        for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; t8[u] = (i < H * 8 && i % 8 < nq) ? __ldg(f.w3 + (size_t)(i / 8) * NO + a0 + i % 8) : 0.f; }
 #pragma unroll
-        for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; if (i < H * NO) w3t[(size_t)(i % NO) * HP + i / NO] = t8[u]; }
+        for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; if (i < H * 8) w3t[(size_t)(i % 8) * HP + i / 8] = t8[u]; }
     }
     __syncthreads();
     const int lane = threadIdx.x & 31, k = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -1218,14 +1222,15 @@ __global__ void __launch_bounds__(256) ts_fold_kernel(const TsFoldArgs f, const 
         else if (k0 < f.A + f.Do) row = f.win + (size_t)(k0 - f.A + f.obs_skip) * H;
         else if (k0 < f.A + f.Do + f.T) { if (f.bt) row = f.bt + (size_t)(k0 - f.A - f.Do) * H; }
     } else { row = f.b2; bias_row = true; }
+    if (a0 >= NO) row = nullptr;                 // zero columns: nothing to load
     float rv[32];                                // the lane's row elements, all loads in flight at once
 #pragma unroll
     for (int q = 0; q < 32; ++q) {
         const int j = lane + 32 * q;
         rv[q] = (row && j < H) ? row[j] : 0.f;
-        if (bias_row && f.b0 && j < H) rv[q] += f.b0[j];
+        if (row && bias_row && f.b0 && j < H) rv[q] += f.b0[j];
     }
-    for (int a0 = 0; a0 < 64; a0 += 8) {
+    {
         float acc[8];
 #pragma unroll
         for (int q = 0; q < 8; ++q) acc[q] = 0.f;
@@ -1235,7 +1240,7 @@ __global__ void __launch_bounds__(256) ts_fold_kernel(const TsFoldArgs f, const 
                 const int j = lane + 32 * qq;
                 if (j < H) {
 #pragma unroll
-                    for (int q = 0; q < 8; ++q) if (a0 + q < NO) acc[q] = fmaf(rv[qq], w3t[(size_t)(a0 + q) * HP + j], acc[q]);
+                    for (int q = 0; q < 8; ++q) if (a0 + q < NO) acc[q] = fmaf(rv[qq], w3t[(size_t)q * HP + j], acc[q]);
                 }
             }
 #pragma unroll
@@ -1303,6 +1308,133 @@ static int ts_refresh_net(dppo_handle* h, int net, cudaStream_t s) {
     return 0;
 }
 
+static int ts_ensure_fold(dppo_handle* h, int net, cudaStream_t s);
+// ------------------------------------------------------------------ AdamW and every weight-derived table in one launch
+// The optimizer step of [actor_ft | critic] followed by what prep_net rebuilds for both nets (the actor's time tables, the plane
+// copies of W1 and of the layer-0 rows), bit-identical to that sequence:
+//  * element blocks (after the time blocks): one parameter per thread (adamw_elem); an element of W1 or of a W_in x / obs row also writes its planes.  The
+//    zero rows of the layer-0 planes (the critic's x / time rows, the pad rows) never change and are left as prep_net wrote them.
+//  * T time blocks (blocks 0 .. T-1): block t evaluates the update of the time MLP, the W_in time rows and b_in itself (from the old w, g,
+//    m, v, into shared memory), runs actor_prep_body on those values and writes row A + Do + t of the layer-0 planes (= bt[t]).
+//    The last time block to finish (counter) writes those small parameters back; until then every time block still reads the old
+//    ones, so the element blocks skip their ranges.
+struct TsUpdateArgs {
+    float* w; const float* g; float* m; float* v; size_t n, nA;            // [actor_ft | critic] and its optimizer moments
+    float lr, alpha, b1, b2, eps, wd; const int *skip0, *skip1;
+    ActorOff ao; CriticOff co; int A, td, Do, T, H, Hc, elem_blocks;
+    TsNetW wa, wc;                                                           // plane copies of actor_ft / critic
+    float *sinemb, *thpre, *temb, *bt; int* done;                            // actor_ft's time tables
+};
+__device__ __forceinline__ bool ts_update_time_param(const TsUpdateArgs& a, size_t i) {      // written by the last time block
+    const size_t wt0 = a.ao.win + (size_t)a.A * a.H, wt1 = wt0 + (size_t)a.td * a.H;
+    return i < a.ao.win || (i >= wt0 && i < wt1) || (i >= a.ao.bin && i < a.ao.bin + a.H);
+}
+__device__ __forceinline__ float ts_update_new(const TsUpdateArgs& a, size_t i, float* mo = nullptr, float* vo = nullptr) {
+    float p = a.w[i], mi = a.m[i], vi = a.v[i];
+    adamw_elem(p, mi, vi, a.g[i], a.lr, a.alpha, a.b1, a.b2, a.eps, a.wd);
+    if (mo) { *mo = mi; *vo = vi; }
+    return p;
+}
+// the parameters the time blocks own, numbered q: [time MLP (q < ao.win, ao.tw1 == 0) | W_in time rows | b_in]
+__device__ __forceinline__ size_t ts_update_time_count(const TsUpdateArgs& a) { return a.ao.win + (size_t)(a.td + 1) * a.H; }
+__device__ __forceinline__ size_t ts_update_time_index(const TsUpdateArgs& a, size_t q) {
+    const size_t nmlp = a.ao.win, ntd = (size_t)a.td * a.H;
+    return q < nmlp ? q : (q < nmlp + ntd ? a.ao.win + (size_t)a.A * a.H + (q - nmlp) : a.ao.bin + (q - nmlp - ntd));
+}
+// the update of every time parameter, eight of them in flight per thread: into sm[q] (WRITE_BACK false) or into w, m, v
+template <bool WRITE_BACK>
+__device__ __forceinline__ void ts_update_time_params(const TsUpdateArgs& a, float* sm) {
+    const size_t nq = ts_update_time_count(a);
+    for (size_t q0 = threadIdx.x; q0 < nq; q0 += 8 * (size_t)blockDim.x) {
+        float p[8], mi[8], vi[8], gi[8]; size_t idx[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            const size_t q = q0 + (size_t)u * blockDim.x;
+            idx[u] = q < nq ? ts_update_time_index(a, q) : 0;
+            p[u] = a.w[idx[u]]; mi[u] = a.m[idx[u]]; vi[u] = a.v[idx[u]]; gi[u] = a.g[idx[u]];
+        }
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            const size_t q = q0 + (size_t)u * blockDim.x;
+            if (q >= nq) break;
+            adamw_elem(p[u], mi[u], vi[u], gi[u], a.lr, a.alpha, a.b1, a.b2, a.eps, a.wd);
+            if (WRITE_BACK) { a.w[idx[u]] = p[u]; a.m[idx[u]] = mi[u]; a.v[idx[u]] = vi[u]; }
+            else sm[q] = p[u];
+        }
+    }
+}
+struct WUpdated {        // actor_prep_body's view of the updated actor: the time parameters staged in shared memory (the only ones it reads)
+    const TsUpdateArgs* a; const float* tp;
+    __device__ __forceinline__ float operator()(size_t i) const {
+        const size_t nmlp = a->ao.win, wt0 = a->ao.win + (size_t)a->A * a->H, ntd = (size_t)a->td * a->H;
+        return i < nmlp ? tp[i] : (i < a->ao.bin ? tp[nmlp + (i - wt0)] : tp[nmlp + ntd + (i - a->ao.bin)]);
+    }
+};
+__global__ void __launch_bounds__(512) ts_update_kernel(const TsUpdateArgs a) {
+    pdl_grid_begin();
+    if ((a.skip0 && *a.skip0) || (a.skip1 && *a.skip1)) return;          // bad minibatch / failed exchange: nothing changes
+    const int tid = threadIdx.x;
+    if ((int)blockIdx.x >= a.T) {                 // the time blocks come first: their chain is the longest
+        const size_t i = (size_t)(blockIdx.x - a.T) * blockDim.x + tid;
+        if (i >= a.n || (i < a.nA && ts_update_time_param(a, i))) return;
+        float mi, vi;
+        const float p = ts_update_new(a, i, &mi, &vi);
+        a.w[i] = p; a.m[i] = mi; a.v[i] = vi;
+        if (i < a.nA) {
+            const size_t H = a.H;
+            if (i >= a.ao.w1 && i < a.ao.w1 + H * H) ts_put2(a.wa.w1, a.wa.fw1, i - a.ao.w1, p);
+            else if (i >= a.ao.win && i < a.ao.win + (size_t)(a.A + a.td + a.Do) * H) {
+                const size_t r = (i - a.ao.win) / H, c = (i - a.ao.win) % H;      // W_in rows [x | time | obs]; h0 order [x | obs | ..]
+                ts_put2(a.wa.w0, a.wa.fw0, (r < (size_t)a.A ? r : r - a.td) * H + c, p);
+            }
+        } else {
+            const size_t j = i - a.nA, Hc = a.Hc;
+            if (j >= a.co.w1 && j < a.co.w1 + Hc * Hc) ts_put2(a.wc.w1, a.wc.fw1, j - a.co.w1, p);
+            else if (j >= a.co.win && j < a.co.win + (size_t)a.Do * Hc) ts_put2(a.wc.w0, a.wc.fw0, (size_t)a.A * Hc + (j - a.co.win), p);
+        }
+        return;
+    }
+    const int t = blockIdx.x;
+    extern __shared__ float upd_sm[];            // [ts_update_time_count] updated time parameters | actor_prep_body's [4 td]
+    ts_update_time_params<false>(a, upd_sm);
+    __syncthreads();
+    actor_prep_body(t, upd_sm + ts_update_time_count(a), WUpdated{&a, upd_sm}, a.ao, a.A, a.td, a.H, a.sinemb, a.thpre, a.temb, a.bt, nullptr);
+    for (int c = tid; c < a.H; c += blockDim.x)  // this thread wrote bt[t][c]
+        ts_put2(a.wa.w0, a.wa.fw0, (size_t)(a.A + a.Do + t) * a.H + c, a.bt[(size_t)t * a.H + c]);
+    __shared__ int last_flag;
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) last_flag = (atomicAdd(a.done, 1) == a.T - 1) ? 1 : 0;
+    __syncthreads();
+    if (!last_flag) return;
+    ts_update_time_params<true>(a, nullptr);
+    if (tid == 0) *a.done = 0;                   // ready for the next launch
+}
+static size_t ts_update_smem(const Geom& g) { return (g.ao.win + (size_t)(g.td + 1) * g.H + 4 * (size_t)g.td) * sizeof(float); }
+static bool ts_update_ok(const dppo_handle* h) {
+    return h->cfg.precision == DPPO_PREC_BF16X3 && ts_shapes_ok(h) && 2 * h->g.td <= 512 && h->g.ao.tw1 == 0 && ts_update_smem(h->g) <= 48 * 1024;
+}
+// AdamW (alpha: the bias-corrected step size of this step) on [actor_ft | critic] with gradient g, then the derived tables of both
+// nets: replaces adamw_kernel + prep_net(ACTOR_FT) + prep_net(CRITIC) of the split-precision mode
+static int ts_apply_update(dppo_handle* h, cudaStream_t s, const float* g, float lr, float alpha, float wd, const int* skip1) {
+    const Geom& gm = h->g; OptState& o = h->opt[DPPO_OPT_FINETUNE]; ActorDerived& d = h->ad[DPPO_NET_ACTOR_FT];
+    TsUpdateArgs a;
+    a.w = h->net_w[DPPO_NET_ACTOR_FT]; a.g = g; a.m = o.m; a.v = o.v; a.nA = gm.ao.n; a.n = gm.ao.n + gm.co.n;
+    a.lr = lr; a.alpha = alpha; a.b1 = h->cfg.adam_beta1; a.b2 = h->cfg.adam_beta2; a.eps = h->cfg.adam_eps; a.wd = wd;
+    a.skip0 = h->skip_update; a.skip1 = skip1;
+    a.ao = gm.ao; a.co = gm.co; a.A = gm.A; a.td = gm.td; a.Do = gm.Do; a.T = gm.T; a.H = gm.H; a.Hc = gm.Hc;
+    a.elem_blocks = tc_nblk(a.n, 512);
+    a.wa = h->ts->net[DPPO_NET_ACTOR_FT]; a.wc = h->ts->net[DPPO_NET_CRITIC];
+    a.sinemb = d.sinemb; a.thpre = d.thpre; a.temb = d.temb; a.bt = d.bt;
+    a.done = reinterpret_cast<int*>(d.dte + (size_t)gm.T * gm.td) + 1;
+    CUDA_TRY(launch_pdl(ts_update_kernel, dim3(a.elem_blocks + gm.T), dim3(512), ts_update_smem(gm), s, a)); TC_KCHECK(h);
+    for (int net : {DPPO_NET_ACTOR_FT, DPPO_NET_CRITIC}) { h->w0p_dirty[net] = 1; h->w23_dirty[net] = 1; h->ts->fold_dirty[net] = 1; }
+    // the folded output layers of the new weights, here rather than lazily at the next update's start: there they ran on the second
+    // stream but got SMs only when the actor's persistent L1 drained, and the actor's folded GEMM waited for them
+    DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR_FT, s)); DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, s));
+    return 0;
+}
+
 // ------------------------------------------------------------------ one residual MLP on N rows, every tensor as planes
 // The output layer is folded: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, so block.l2's H x H product is skipped and v never formed (the
 // caller has run ts_ensure_fold).  The weight gradient of the output layer is assembled from a1^T dout and h0^T dout (ts_dw3_assemble_kernel).
@@ -1334,9 +1466,9 @@ static int ts_ensure_fold(dppo_handle* h, int net, cudaStream_t s) {
     }
     static bool attr_set_dev[64] = {};
     if (!attr_set_dev[h->device & 63]) { CUDA_TRY(cudaFuncSetAttribute(ts_fold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024)); attr_set_dev[h->device & 63] = true; }
-    const size_t sm = (size_t)(f.H + 1) * f.NO * sizeof(float);
-    if (sm > 96 * 1024 || f.H > 1024) DPPO_FAIL(-7, "ts_ensure_fold: output layer too wide for the fold kernel");
-    ts_fold_kernel<<<tc_nblk((size_t)(f.H + f.KP0 + 1), 8), 256, sm, s>>>(f, W.ffold, W.bfold, W.w23p);
+    const size_t sm = (size_t)(f.H + 1) * 8 * sizeof(float);
+    if (sm > 96 * 1024 || f.H > 1024 || f.NO > 64) DPPO_FAIL(-7, "ts_ensure_fold: output layer too wide for the fold kernel");
+    CUDA_TRY(launch_pdl(ts_fold_kernel, dim3(tc_nblk((size_t)(f.H + f.KP0 + 1), 8), 8), dim3(256), sm, s, f, W.ffold, W.bfold, W.w23p));
     TC_KCHECK(h);
     h->ts->fold_dirty[net] = 0;
     return 0;
@@ -1611,6 +1743,7 @@ __device__ __forceinline__ void ts_rank_rows_body(const TsDw3Args& f, int bid, f
 // dW2 rows (q < H), which nothing but AdamW reads - next to the tail kernel on the second stream
 __global__ void __launch_bounds__(512) ts_dw3_assemble_kernel(const TsDw3Args fa, int blocks_a, const TsDw3Args fc, int blocks_c,
                                                               float* __restrict__ part, int* __restrict__ done, int rank_a, int rank_c, int phase) {
+    pdl_grid_begin();
     extern __shared__ float dw3_sm[];
     int b = blockIdx.x;
     if (phase == 1) {
@@ -1683,7 +1816,7 @@ static int ts_dw3_assemble(dppo_handle* h, cudaStream_t s, int actor_net, const 
     }
     int* done = reinterpret_cast<int*>(st->dw3_buf);
     float* partb = reinterpret_cast<float*>(st->dw3_buf + 1024);
-    ts_dw3_assemble_kernel<<<(phase == 1 ? nba + nbc : 0) + nra + nrc, 512, sm, s>>>(fa, nba, fc, nbc, partb, done, nra, nrc, phase);
+    CUDA_TRY(launch_pdl(ts_dw3_assemble_kernel, dim3((phase == 1 ? nba + nbc : 0) + nra + nrc), dim3(512), sm, s, fa, nba, fc, nbc, partb, done, nra, nrc, phase));
     TC_KCHECK(h);
     return 0;
 }
@@ -1857,9 +1990,7 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     DPPO_TRY(colsum(h, s, dval, 1, N, 1, nullptr, 1, part, gr + nA + g.co.b3));
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, b2scr, g.H, gr + g.ao.b1); TC_KCHECK(h);
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.Hc, 8), 256, 0, s>>>(cpc, nrb, (size_t)2 * g.Hc, 2 * g.Hc, b2scr + g.H, g.Hc, gr + nA + g.co.b1); TC_KCHECK(h);
-    const float* w = h->net_w[DPPO_NET_ACTOR_FT]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR_FT];
-    const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
-    time_backward_kernel<<<1 + (g.H + 127) / 128, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, dw0a + (size_t)(g.A + g.Do) * g.H, d.sinemb, d.thpre, d.temb, gr); TC_KCHECK(h);
+    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR_FT, dw0a + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0a, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)g.Do * g.Hc, 256), 256, 0, s>>>(dw0c + (size_t)g.A * g.Hc, 0, 0, g.Do, g.Hc, gr + nA + g.co.win); TC_KCHECK(h);
     CUDA_TRY(cudaMemcpyAsync(gr + nA + g.co.bin, dw0c + (size_t)(g.A + g.Do + g.T) * g.Hc, g.Hc * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -1906,9 +2037,7 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR, ga1, ga0, gr, dw0, nullptr, nullptr, nullptr, nullptr));
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ga1 + (size_t)(g.H + KP0) * 32, g.H, gr + g.ao.b1); TC_KCHECK(h);
     DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
-    const float* w = h->net_w[DPPO_NET_ACTOR]; const ActorDerived& d = h->ad[DPPO_NET_ACTOR];
-    const size_t sm = (size_t)(g.T * g.td * 3) * sizeof(float);
-    time_backward_kernel<<<1 + (g.H + 127) / 128, 512, sm, s>>>(w, g.ao, g.A, g.td, g.H, g.T, dw0 + (size_t)(g.A + g.Do) * g.H, d.sinemb, d.thpre, d.temb, gr); TC_KCHECK(h);
+    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR, dw0 + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
     return 0;
 }
