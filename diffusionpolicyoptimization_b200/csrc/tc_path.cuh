@@ -389,7 +389,9 @@ __global__ void __launch_bounds__(128) tc_ppo_loss_kernel(
 // The same loss with EIGHT lanes per row (A % 4 == 0, A <= 32): lane `sub` of a row owns elements [4 sub, 4 sub + 4) and reads them
 // as one float4 per input array (coalesced; the thread-per-row kernel above walks 96-byte strides and leaves the SMs at ~10 warps).
 // 32 rows per 256-thread block.  Row scalars are computed redundantly by the row's lanes after a 3-step shuffle reduction.
+// LPR = 32 (split-precision mode, A % 4 == 0, 32 < A <= 128): a warp per row, 8 rows per block, seed rows 128 wide (the actor's NOP).
 constexpr int LOSS8_ROWS = 32;
+template <int LPR = 8>
 __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
     const float* __restrict__ prev, const float* __restrict__ nxt, const float* __restrict__ eps,
     const int* __restrict__ inds, const float* __restrict__ returns, const float* __restrict__ oldvalues,
@@ -397,8 +399,10 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
     const float* __restrict__ advstats, const float* __restrict__ sch, PpoHyper hp, int N,
     bf16* __restrict__ depsb, bf16* __restrict__ dvalb, double* __restrict__ block_sums, float* __restrict__ col_part /*[blocks][A+1]*/,
     const TcIdxView iv, bf16* __restrict__ depsb_lo = nullptr, bf16* __restrict__ dvalb_lo = nullptr /* second planes (DPPO_PREC_BF16X3) */) {
-    const int tid = threadIdx.x, sub = tid & 7, lane = tid & 31, wrp = tid >> 5;
-    const int r = blockIdx.x * LOSS8_ROWS + (tid >> 3);
+    static_assert(LPR == 8 || LPR == 32, "eight lanes (A <= 32) or a warp (A <= 128) per row");
+    constexpr int ROWS = 256 / LPR, DLD = LPR == 8 ? 64 : 128;     // rows per block; seed row width
+    const int tid = threadIdx.x, sub = tid & (LPR - 1), lane = tid & 31, wrp = tid >> 5;
+    const int r = blockIdx.x * ROWS + tid / LPR;
     const int A = hp.A, a0 = sub * 4;
     const bool row_ok = r < N;
     // where this row's inputs live: the materialised minibatch arrays, or (index-driven) the resident rollout buffers
@@ -444,7 +448,7 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
         }
     }
 #pragma unroll
-    for (int off = 1; off < 8; off <<= 1) { newp += __shfl_xor_sync(0xffffffffu, newp, off); oldp += __shfl_xor_sync(0xffffffffu, oldp, off); }
+    for (int off = 1; off < LPR; off <<= 1) { newp += __shfl_xor_sync(0xffffffffu, newp, off); oldp += __shfl_xor_sync(0xffffffffu, oldp, off); }
     if (row_ok) {
         const float newm = newp / (float)nuse, oldm = oldp / (float)nuse;
         float adv = advantages[srow];
@@ -461,16 +465,16 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
 #pragma unroll
         for (int e = 0; e < 4; ++e) gq[e] = ((live >> e) & 1u) ? gscale * z[e] : 0.f;
         // padded bf16 seed row [deps (A) | 0..]: this lane's 4 columns and 4 of the zero columns
-        uint2* drow = reinterpret_cast<uint2*>(depsb + (size_t)r * 64);
+        uint2* drow = reinterpret_cast<uint2*>(depsb + (size_t)r * DLD);
         drow[sub] = make_uint2(fc::pack_bf16(gq[0], gq[1]), fc::pack_bf16(gq[2], gq[3]));
-        drow[8 + sub] = make_uint2(0u, 0u);
+        if (LPR == 8) drow[8 + sub] = make_uint2(0u, 0u);
         if (depsb_lo) {   // second plane: what the first one rounded away
             float lo[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) lo[e] = gq[e] - __bfloat162float(__float2bfloat16(gq[e]));
-            uint2* lrow = reinterpret_cast<uint2*>(depsb_lo + (size_t)r * 64);
+            uint2* lrow = reinterpret_cast<uint2*>(depsb_lo + (size_t)r * DLD);
             lrow[sub] = make_uint2(fc::pack_bf16(lo[0], lo[1]), fc::pack_bf16(lo[2], lo[3]));
-            lrow[8 + sub] = make_uint2(0u, 0u);
+            if (LPR == 8) lrow[8 + sub] = make_uint2(0u, 0u);
         }
         if (sub == 0) {
             const float v = newvalues[r], ret = returns[srow];
@@ -490,29 +494,29 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
         }
         // padded bf16 seed row [dvalue | 0..]: 16 bytes per lane
         uint4* vrow = reinterpret_cast<uint4*>(dvalb + (size_t)r * 64);
-        vrow[sub] = sub == 0 ? make_uint4(fc::pack_bf16(dv_out, 0.f), 0u, 0u, 0u) : make_uint4(0u, 0u, 0u, 0u);
-        if (dvalb_lo) {
+        if (sub < 8) vrow[sub] = sub == 0 ? make_uint4(fc::pack_bf16(dv_out, 0.f), 0u, 0u, 0u) : make_uint4(0u, 0u, 0u, 0u);
+        if (dvalb_lo && sub < 8) {
             uint4* lrow = reinterpret_cast<uint4*>(dvalb_lo + (size_t)r * 64);       // dv_out lives in the row's lane 0
             lrow[sub] = sub == 0 ? make_uint4(fc::pack_bf16(dv_out - __bfloat162float(__float2bfloat16(dv_out)), 0.f), 0u, 0u, 0u) : make_uint4(0u, 0u, 0u, 0u);
         }
     }
     // ---- block reductions: rows of a warp (lanes differing in bits 3,4), then the 8 warps through shared memory
     __shared__ double red[5][8];
-    __shared__ float cred[8][33];
+    __shared__ float cred[8][4 * LPR + 1];
 #pragma unroll
-    for (int off = 8; off < 32; off <<= 1) {
+    for (int off = LPR; off < 32; off <<= 1) {
 #pragma unroll
         for (int k = 0; k < 5; ++k) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
 #pragma unroll
         for (int e = 0; e < 4; ++e) gq[e] += __shfl_xor_sync(0xffffffffu, gq[e], off);
         dv_out += __shfl_xor_sync(0xffffffffu, dv_out, off);
     }
-    if (lane == 0) { for (int k = 0; k < 5; ++k) red[k][wrp] = acc[k]; cred[wrp][32] = dv_out; }
-    if (lane < 8) { for (int e = 0; e < 4; ++e) cred[wrp][lane * 4 + e] = gq[e]; }
+    if (lane == 0) { for (int k = 0; k < 5; ++k) red[k][wrp] = acc[k]; cred[wrp][4 * LPR] = dv_out; }
+    if (lane < LPR) { for (int e = 0; e < 4; ++e) cred[wrp][lane * 4 + e] = gq[e]; }
     __syncthreads();
     if (tid < 5) { double t = 0; for (int w = 0; w < 8; ++w) t += red[tid][w]; block_sums[(size_t)blockIdx.x * 5 + tid] = t; }
     if (tid <= A) {
-        const int a = tid < A ? tid : 32;
+        const int a = tid < A ? tid : 4 * LPR;
         float t = 0.f;
         for (int w = 0; w < 8; ++w) t += cred[w][a];
         col_part[(size_t)blockIdx.x * (A + 1) + tid] = t;

@@ -345,6 +345,8 @@ static int launch(dppo_handle* h, cudaStream_t s, const Gemm& g) {
     const bool a = g.A.mn_major, b = g.B.mn_major;
     if (g.f16) {
         if (g.planes == 2 && g.dual && !a && !b && g.N <= 32) return launch_t<32, false, false, 2, true, true>(h, s, g);
+        // the folded output layer of an action chunk wider than 32: one 128-wide column block, so the [a1 | h0] rows are read once
+        if (g.planes == 2 && g.dual && !a && !b && g.N <= 128) return launch_t<128, false, false, 2, true, true>(h, s, g);
         if (g.planes == 2 && g.dual && !a && b) return launch_t<128, false, true, 2, true, true>(h, s, g);
         DPPO_FAIL(-7, "split gemm: this fp16-plane operand layout is not instantiated");
     }
@@ -1059,12 +1061,15 @@ struct TsW { bf16* p[ts::MAXP]; };
 struct TsNetW {
     TsW w0, w1;                           // [KP0][H] W0 rows in h0 order, [H][H] W1
     TsW fw0, fw1;                         // fp16 planes, scaled by ts::F16_WSCALE
-    TsW ffold;                            // [64][H + KP0] planes of [W2 W3 ; W0 W3]^T (fp16 x 2^10 when the net's forward runs on fp16 planes, else
+    TsW ffold;                            // [NOP][H + KP0] planes of [W2 W3 ; W0 W3]^T (fp16 x 2^10 when the net's forward runs on fp16 planes, else
                                           // bf16): the folded output layer, out = [a1 | h0] [W2 W3 ; W0 W3] + bfold
-    float* bfold;                         // [64]  (b2 (+ b_in)) W3 + b3
+    float* bfold;                         // [NOP]  (b2 (+ b_in)) W3 + b3
     TsW w23p;                             // [H][128] bf16 planes of W2 W3 (columns >= NO zero): dh1 = (dout (W2 W3)^T) . act'(h1) without forming dv
 };
 struct TsState { TsNetW net[4]; int KP0; int fold_dirty[4]; char* dw3_buf; size_t dw3_bytes; };
+// NOP: the padded width of a net's output (gradient seeds dout [N][NOP], rows of ffold / bfold, K of dh1 = dout (W2 W3)^T).  64 up to 32
+// outputs; an actor with a wider action chunk (up to 128) takes 128.  The critic (one output) keeps 64.
+static inline int ts_nop(int NO) { return NO <= 32 ? 64 : 128; }
 
 __device__ __forceinline__ void ts_put(const TsW& W, size_t i, float v) {
     bf16 a, b; ts::split_bf16(v, a, b);
@@ -1136,16 +1141,17 @@ __global__ void ts_pack_h0_kernel(const float* __restrict__ x, const float* __re
         if (hb.p[0]) *reinterpret_cast<uint4*>(hb.p[pl] + (size_t)r * KP0 + k0) = *reinterpret_cast<const uint4*>(o3[2 + pl]);
     }
 }
-// dst[r][0:64] = [src[r][0:ncols] | 0..] as two planes
-__global__ void ts_pad64_kernel(const float* __restrict__ src, int N, int ncols, bf16* __restrict__ hi, bf16* __restrict__ lo) {
+// dst[r][0:ld] = [src[r][0:ncols] | 0..] as two planes (ld a multiple of 8: the padded width NOP); one thread per 8 columns
+__global__ void ts_pad64_kernel(const float* __restrict__ src, int N, int ncols, int ld, bf16* __restrict__ hi, bf16* __restrict__ lo) {
+    const int g8 = ld / 8;
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (size_t)N * 8) return;
-    const int r = (int)(i >> 3), k0 = (int)(i & 7) * 8;
+    if (i >= (size_t)N * g8) return;
+    const int r = (int)(i / g8), k0 = (int)(i % g8) * 8;
     __align__(16) bf16 oh[8]; __align__(16) bf16 ol[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) ts::split_bf16(k0 + j < ncols ? src[(size_t)r * ncols + k0 + j] : 0.f, oh[j], ol[j]);
-    *reinterpret_cast<uint4*>(hi + (size_t)r * 64 + k0) = *reinterpret_cast<const uint4*>(oh);
-    *reinterpret_cast<uint4*>(lo + (size_t)r * 64 + k0) = *reinterpret_cast<const uint4*>(ol);
+    *reinterpret_cast<uint4*>(hi + (size_t)r * ld + k0) = *reinterpret_cast<const uint4*>(oh);
+    *reinterpret_cast<uint4*>(lo + (size_t)r * ld + k0) = *reinterpret_cast<const uint4*>(ol);
 }
 // column sums of a two-plane matrix [N][ncols] (ncols even, ncols/2 <= 256): part[blk][ncols]
 __global__ void __launch_bounds__(256) ts_colsum_kernel(const bf16* __restrict__ Dh, const bf16* __restrict__ Dl, int N, int ncols, int rows_per_block,
@@ -1185,7 +1191,7 @@ static int ensure_w23(dppo_handle* h, int net, cudaStream_t s) {
 // Folded output layer of one net.  No activation sits between block.l2 and the last Dense (model/common/mlp.py), so
 //   out = (a1 W2 + b2 + u) W3 + b3 = [a1 | h0] [W2 W3 ; W0 W3] + ((b2 + b0) W3 + b3),      u = h0 W0 + b0
 // with W0 = the h0-order rows of layer 0 ([x | obs | bt[t] | 0..]; the actor's b0 rides in the bt rows, the critic's is `b0`).
-// ffold[a][k] (a < 64, k < H + KP0) = that matrix transposed, as fp16 planes of 2^10 x (f16) or bf16 planes; bfold[a] the bias.
+// ffold[a][k] (a < NOP, k < H + KP0) = that matrix transposed, as fp16 planes of 2^10 x (f16) or bf16 planes; bfold[a] the bias.
 // One thread per (k, a) and one for each bias entry; double accumulation, rounded once.
 struct TsFoldArgs {
     const float *w2, *w3, *b2, *b3, *b0;      // [H][H], [H][NO], [H], [NO], [H] or null
@@ -1198,7 +1204,7 @@ struct TsFoldArgs {
 // products each, fp32), the group's 8 columns of W3 sit transposed and padded in shared memory (conflict-free both ways), the lane
 // partials meet in a butterfly.  (A first version accumulated in double: 30 us - the CUDA-core fp64 rate of this part - for sums that
 // are rounded to 22-bit planes anyway.  One block per 8 rows for all 64 columns: 20 us on 73 blocks; split by column group the launch
-// has 8x the blocks and each stages an eighth of W3.)
+// has 8x the blocks and each stages an eighth of W3.)  gridDim.y = NOP / 8 groups; the groups at and past NO write the zero padding.
 __global__ void __launch_bounds__(256) ts_fold_kernel(const TsFoldArgs f, const TsW F, float* __restrict__ bfold, const TsW B23) {
     pdl_grid_begin();
     extern __shared__ float w3t[];               // [8][H + 1]: columns a0 .. a0 + 7 of W3
@@ -1278,14 +1284,15 @@ static int ts_init(dppo_handle* h) {
     memset(st, 0, sizeof(*st));
     h->ts = st;
     st->KP0 = round_up(g.A + g.Do + g.T + 1, 64);
-    if ((g.H % 64) || (g.Hc % 64) || g.A > 32) return 0;     // shapes this path does not cover: stays on FFMA
+    if ((g.H % 64) || (g.Hc % 64) || g.A > 128) return 0;    // shapes this path does not cover: stays on FFMA
     for (int net = 0; net < 4; ++net) {
         TsNetW& w = st->net[net];
         const size_t H = net == DPPO_NET_CRITIC ? g.Hc : g.H;
+        const size_t NOP = ts_nop(net == DPPO_NET_CRITIC ? 1 : g.A);
         DPPO_TRY(ts_alloc_w(w.w0, st->KP0 * H)); DPPO_TRY(ts_alloc_w(w.w1, H * H));
         DPPO_TRY(ts_alloc_w(w.fw0, st->KP0 * H)); DPPO_TRY(ts_alloc_w(w.fw1, H * H));
-        DPPO_TRY(ts_alloc_w(w.ffold, 64 * (H + st->KP0)));
-        CUDA_TRY(cudaMalloc(&w.bfold, 64 * sizeof(float)));
+        DPPO_TRY(ts_alloc_w(w.ffold, NOP * (H + st->KP0)));
+        CUDA_TRY(cudaMalloc(&w.bfold, NOP * sizeof(float)));
         DPPO_TRY(ts_alloc_w(w.w23p, H * 128)); CUDA_TRY(cudaMemset(w.w23p.p[0], 0, 2 * H * 128 * sizeof(bf16)));
         st->fold_dirty[net] = 1;
     }
@@ -1439,7 +1446,7 @@ static int ts_apply_update(dppo_handle* h, cudaStream_t s, const float* g, float
 // The output layer is folded: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, so block.l2's H x H product is skipped and v never formed (the
 // caller has run ts_ensure_fold).  The weight gradient of the output layer is assembled from a1^T dout and h0^T dout (ts_dw3_assemble_kernel).
 struct TsMlp {
-    const TsNetW* W; int H, NO, act1, KP0, net, din;
+    const TsNetW* W; int H, NO, NOP, act1, KP0, net, din;
     int fp;                                // FORWARD GEMMs: 4 = two fp16 planes + two accumulators (22 bits) when the net has kinks behind it,
                                            // 2 = two bf16 planes, one accumulator (16 bits).  h0 / a0 / a1 carry that format.
     const float *b0, *b1;
@@ -1467,8 +1474,8 @@ static int ts_ensure_fold(dppo_handle* h, int net, cudaStream_t s) {
     static bool attr_set_dev[64] = {};
     if (!attr_set_dev[h->device & 63]) { CUDA_TRY(cudaFuncSetAttribute(ts_fold_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024)); attr_set_dev[h->device & 63] = true; }
     const size_t sm = (size_t)(f.H + 1) * 8 * sizeof(float);
-    if (sm > 96 * 1024 || f.H > 1024 || f.NO > 64) DPPO_FAIL(-7, "ts_ensure_fold: output layer too wide for the fold kernel");
-    CUDA_TRY(launch_pdl(ts_fold_kernel, dim3(tc_nblk((size_t)(f.H + f.KP0 + 1), 8), 8), dim3(256), sm, s, f, W.ffold, W.bfold, W.w23p));
+    if (sm > 96 * 1024 || f.H > 1024 || f.NO > 128) DPPO_FAIL(-7, "ts_ensure_fold: output layer too wide for the fold kernel");
+    CUDA_TRY(launch_pdl(ts_fold_kernel, dim3(tc_nblk((size_t)(f.H + f.KP0 + 1), 8), ts_nop(f.NO) / 8), dim3(256), sm, s, f, W.ffold, W.bfold, W.w23p));
     TC_KCHECK(h);
     h->ts->fold_dirty[net] = 0;
     return 0;
@@ -1476,14 +1483,14 @@ static int ts_ensure_fold(dppo_handle* h, int net, cudaStream_t s) {
 static void ts_actor_mlp(const dppo_handle* h, int net, TsMlp& m) {
     const Geom& g = h->g; const float* w = h->net_w[net];
     memset(&m, 0, sizeof(m));
-    m.W = &h->ts->net[net]; m.H = g.H; m.NO = g.A; m.act1 = h->cfg.actor_act + 1; m.KP0 = h->ts->KP0; m.net = net; m.din = g.Din;
+    m.W = &h->ts->net[net]; m.H = g.H; m.NO = g.A; m.NOP = ts_nop(g.A); m.act1 = h->cfg.actor_act + 1; m.KP0 = h->ts->KP0; m.net = net; m.din = g.Din;
     m.fp = 4;                                                                        // ReLU kinks and the +-1 clip of x0 behind eps
     m.b0 = nullptr; m.b1 = w + g.ao.b1;                                              // b_in rides in W0's one-hot rows (bt table)
 }
 static void ts_critic_mlp(const dppo_handle* h, TsMlp& m) {
     const Geom& g = h->g; const float* w = h->net_w[DPPO_NET_CRITIC];
     memset(&m, 0, sizeof(m));
-    m.W = &h->ts->net[DPPO_NET_CRITIC]; m.H = g.Hc; m.NO = 1; m.act1 = h->cfg.critic_act + 1; m.KP0 = h->ts->KP0; m.net = DPPO_NET_CRITIC; m.din = g.Do;
+    m.W = &h->ts->net[DPPO_NET_CRITIC]; m.H = g.Hc; m.NO = 1; m.NOP = ts_nop(1); m.act1 = h->cfg.critic_act + 1; m.KP0 = h->ts->KP0; m.net = DPPO_NET_CRITIC; m.din = g.Do;
     m.fp = h->cfg.critic_act == DPPO_ACT_RELU ? 4 : 2;                               // Mish is smooth
     m.b0 = w + g.co.bin; m.b1 = w + g.co.b1;
 }
@@ -1554,8 +1561,9 @@ static int ts_mlp_forward(dppo_handle* h, cudaStream_t s, const TsMlp& m, int N,
     }
     if (phase == 1) return 0;
     // no activation between block.l2 and the output layer: out = [a1 | h0] [W2 W3 ; W0 W3] + bfold, one narrow GEMM
-    ts::Gemm o = ts_gemm_of(tsK(m.a1, N, H, H), tswK(W.ffold, 0, 32, H, H + KP0), N, m.NO, 2, f16 ? 1 : 0);
-    o.A2 = tsK(m.h0, N, KP0, KP0); o.B2 = tswK(W.ffold, (size_t)H, 32, KP0, H + KP0);
+    const int nb = m.NO <= 32 ? 32 : m.NOP;                              // ffold rows the GEMM reads (the B box)
+    ts::Gemm o = ts_gemm_of(tsK(m.a1, N, H, H), tswK(W.ffold, 0, nb, H, H + KP0), N, m.NO, 2, f16 ? 1 : 0);
+    o.A2 = tsK(m.h0, N, KP0, KP0); o.B2 = tswK(W.ffold, (size_t)H, nb, KP0, H + KP0);
     if (f16) { o.f16 = 1; o.epi.scale = 1.0f / ts::F16_WSCALE; }
     o.epi.bias = W.bfold; o.epi.out_f32 = m.out; o.epi.ld_f32 = m.NO;
     o.alg_flops = 2.0 * N * ((double)H * H + (double)H * m.NO);        // the algorithmic work it stands for
@@ -1585,14 +1593,14 @@ static int ts_colsum(dppo_handle* h, cudaStream_t s, const SplitT& D, int N, int
     tc_reduce_cols_kernel<<<tc_nblk(ncols, 8), 256, 0, s>>>(part, nb, (size_t)ncols, ncols, out); TC_KCHECK(h);
     return 0;
 }
-// backward chain of the residual MLP from dout [N][64] (two planes, zero padded): dh1 = (dout (W2 W3)^T) . act'(h1),
-// du = (dh1 W1^T) . act'(u).  dv = dout W3^T has rank NO and is never formed: dh1 is ONE K = 64 product, and everything else dv
+// backward chain of the residual MLP from dout [N][NOP] (two planes, zero padded): dh1 = (dout (W2 W3)^T) . act'(h1),
+// du = (dh1 W1^T) . act'(u).  dv = dout W3^T has rank NO and is never formed: dh1 is ONE K = NOP product, and everything else dv
 // fed - dW2 = a1^T dv = (a1^T dout) W3^T, the residual part of dW0 = (h0^T dout) W3^T, db2 = (1^T dout) W3^T - is assembled from the small
 // products a1^T dout / h0^T dout the folded output layer needs anyway (ts_dw3_assemble_kernel).
 // cpart [ceil(N/32)][2][H]: per 32-row block column sums of dh1 (slot 1 = db1), written by the epilogue; slot 0 stays unwritten.
 static int ts_mlp_backward_dx(dppo_handle* h, cudaStream_t s, const TsMlp& m, const SplitT& dout, int N, float* cpart) {
     const int H = m.H; const TsNetW& W = *m.W;
-    tsp::Gemm g = tsp_gemm_of(tsK(dout, N, 64, 64), tswK(W.w23p, 0, H, 64, 128), N, H, 2, m.dh1, 2, H);
+    tsp::Gemm g = tsp_gemm_of(tsK(dout, N, m.NOP, m.NOP), tswK(W.w23p, 0, H, m.NOP, 128), N, H, 2, m.dh1, 2, H);
     g.alg_flops = 2.0 * N * ((double)m.NO * H + (double)H * H);                  // the two products it stands for
     g.epi.colsum_part = cpart + H; g.epi.colsum_ld = 2 * H;
     if (m.act1 == 1) { g.epi.mask_in = m.m1; g.epi.ldm = H / 32; } else if (m.act1 == 2) { g.epi.gate_in[0] = m.g1.p[0]; g.epi.gate_in[1] = m.g1.p[1]; g.epi.ldg = H; }
@@ -1612,8 +1620,8 @@ static int ts_mlp_dw_descs(const TsMlp& m, const SplitT& dout, int N, float* gne
     const SplitT& a0 = f ? m.a0b : m.a0; const SplitT& a1 = f ? m.a1b : m.a1; const SplitT& h0 = f ? m.h0b : m.h0;
     d[0] = tsp::DwDesc{a0, H, m.dh1, H, none, none, gnet + ow1, H, H, H, 0, 2.0 * r * H * H};
     d[1] = tsp::DwDesc{m.du, H, h0, KP0, none, none, dw0, H, KP0, H, 1, 2.0 * r * m.din * H};
-    d[2] = tsp::DwDesc{a1, H, dout, 64, none, none, g1, H, m.NO, m.NO, 0, 2.0 * r * (H * m.NO + (double)H * H)};
-    d[3] = tsp::DwDesc{h0, KP0, dout, 64, none, none, g0, KP0, m.NO, m.NO, 0, 0.0};
+    d[2] = tsp::DwDesc{a1, H, dout, m.NOP, none, none, g1, H, m.NO, m.NO, 0, 2.0 * r * (H * m.NO + (double)H * H)};
+    d[3] = tsp::DwDesc{h0, KP0, dout, m.NOP, none, none, g0, KP0, m.NO, m.NO, 0, 0.0};
     return 4;
 }
 // dW3[j][a] = sum_r v[r][j] dout[r][a] with v = a1 W2 + (b2 + b0) + h0 W0 never formed:
@@ -1630,13 +1638,17 @@ struct TsDw3Args {
 // coalesced 128-byte row segment, all of a warp's loads in flight at once; g1 / g0 rows in shared memory), writes the partial
 // [32][NO] tile, and the LAST block of a column chunk to finish (a counter per chunk) adds the KS partials in slice order - the result
 // does not depend on which block that is.  (A first version walked all k in one block per chunk: 41 us of serialised load latency.)
-constexpr int DW3_KS = 8;
+// WIDE (NO > 32): the warp partials pass through shared memory DW3_WC columns at a time ([16][32][DW3_WC] instead of [16][32][NO]);
+// every output keeps the same sums in the same order.
+constexpr int DW3_KS = 8, DW3_WC = 16;
+template <bool WIDE>
 __device__ __forceinline__ void ts_dw3_assemble_body(const TsDw3Args& f, int bid, float* sm, float* __restrict__ part, int* __restrict__ done) {
     const int H = f.H, NO = f.NO, KT = f.A + f.Do + f.T, K = H + KT;       // k < H: W2 rows; then the h0-order rows of layer 0
     const int jc = bid / DW3_KS, ks = bid % DW3_KS;
     const int kper = (K + DW3_KS - 1) / DW3_KS, kbeg = ks * kper, kend = min(K, kbeg + kper);
+    const int NC = WIDE ? DW3_WC : NO;                // columns per pass
     float* gs = sm;                                   // [kper][NO]
-    float* red = gs + (size_t)kper * NO;              // [16][32][NO]
+    float* red = gs + (size_t)kper * NO;              // [16][32][NC]
     __shared__ int last_flag;
     for (int i = threadIdx.x; i < (kend - kbeg) * NO; i += blockDim.x) {
         const int k = kbeg + i / NO, a = i % NO;
@@ -1658,21 +1670,25 @@ __device__ __forceinline__ void ts_dw3_assemble_body(const TsDw3Args& f, int bid
         const float* row = (k < kend && j < H) ? row_of(k) : nullptr;
         wv[u] = row ? row[j] : 0.f;
     }
-    for (int a = 0; a < NO; ++a) {
-        float acc = 0.f;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-            const int kl = warp + u * nw;
-            if (kbeg + kl < kend) acc = fmaf(wv[u], gs[(size_t)kl * NO + a], acc);
-        }
-        red[((size_t)warp * 32 + lane) * NO + a] = acc;
-    }
-    __syncthreads();
     float* mine = part + ((size_t)jc * DW3_KS + ks) * 32 * NO;
-    for (int i = threadIdx.x; i < 32 * NO; i += blockDim.x) {
-        float s = 0.f;
-        for (int w = 0; w < nw; ++w) s += red[(size_t)w * 32 * NO + i];
-        mine[i] = s;
+    for (int c0 = 0; c0 < NO; c0 += NC) {
+        const int nc = min(NC, NO - c0);
+        for (int a = 0; a < nc; ++a) {
+            float acc = 0.f;
+#pragma unroll
+            for (int u = 0; u < 8; ++u) {
+                const int kl = warp + u * nw;
+                if (kbeg + kl < kend) acc = fmaf(wv[u], gs[(size_t)kl * NO + c0 + a], acc);
+            }
+            red[((size_t)warp * 32 + lane) * nc + a] = acc;
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < 32 * nc; i += blockDim.x) {
+            float s = 0.f;
+            for (int w = 0; w < nw; ++w) s += red[(size_t)w * 32 * nc + i];
+            mine[(size_t)(i / nc) * NO + c0 + i % nc] = s;
+        }
+        if (WIDE) __syncthreads();                    // red is overwritten by the next pass
     }
     __threadfence();
     __syncthreads();
@@ -1739,22 +1755,83 @@ __device__ __forceinline__ void ts_rank_rows_body(const TsDw3Args& f, int bid, f
         }
     }
 }
+// The same rows for 32 < NO <= 128: W3 passes through shared memory 32 columns at a time ([H][33]); a thread's eight sums run on across the
+// passes, so each is the same a = 0 .. NO - 1 chain as above.
+__device__ __forceinline__ void ts_rank_rows_wide_body(const TsDw3Args& f, int bid, float* sm, int row_begin, int row_end) {
+    const int H = f.H, NO = f.NO, nrows = min(H + f.KP0 + 1, row_end), q0 = row_begin + bid * DW3_RB;
+    const int ones = f.A + f.Do + f.T;
+    for (int i = threadIdx.x; i < DW3_RB * NO; i += blockDim.x) {
+        const int q = q0 + i / NO, a = i % NO;
+        float v = 0.f;
+        if (q < H) v = f.g1[(size_t)q * NO + a];
+        else if (q < H + f.KP0) v = f.g0[(size_t)(q - H) * NO + a];
+        else if (q == H + f.KP0) v = f.g0[(size_t)ones * NO + a];
+        sm[i] = v;
+    }
+    float* w3s = sm + DW3_RB * NO;                   // [H][33]: columns [c0, c0 + 32) of W3
+    for (int j0 = 0; j0 < H; j0 += blockDim.x) {     // the same trip count in every thread: the passes below synchronise the block
+        const int j = j0 + (int)threadIdx.x;
+        float old[DW3_RB], acc[DW3_RB];
+#pragma unroll
+        for (int r = 0; r < DW3_RB; ++r) {
+            const int q = q0 + r;
+            old[r] = (j < H && q >= H && q < H + f.KP0 && q < nrows) ? f.dw0[(size_t)(q - H) * H + j] : 0.f;
+            acc[r] = 0.f;
+        }
+        for (int c0 = 0; c0 < NO; c0 += 32) {
+            const int nc = min(32, NO - c0), n3 = H * nc;
+            __syncthreads();                          // the previous pass has read w3s (and, first time, sm is complete)
+            for (int i0 = threadIdx.x; i0 < n3; i0 += blockDim.x * 8) {
+                float t8[8];
+#pragma unroll
+                for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; t8[u] = i < n3 ? __ldg(f.w3 + (size_t)(i / nc) * NO + c0 + i % nc) : 0.f; }
+#pragma unroll
+                for (int u = 0; u < 8; ++u) { const int i = i0 + u * blockDim.x; if (i < n3) w3s[(i / nc) * 33 + i % nc] = t8[u]; }
+            }
+            __syncthreads();
+            if (j < H) {
+                float w3r[32];
+#pragma unroll
+                for (int a = 0; a < 32; ++a) w3r[a] = a < nc ? w3s[j * 33 + a] : 0.f;
+#pragma unroll
+                for (int r = 0; r < DW3_RB; ++r) {
+#pragma unroll
+                    for (int a = 0; a < 32; ++a) if (a < nc) acc[r] = fmaf(sm[r * NO + c0 + a], w3r[a], acc[r]);
+                }
+            }
+        }
+        if (j >= H) continue;
+#pragma unroll
+        for (int r = 0; r < DW3_RB; ++r) {
+            const int q = q0 + r;
+            if (q >= nrows) break;
+            if (q < H) f.dw2[(size_t)q * H + j] = acc[r];
+            else if (q < H + f.KP0) f.dw0[(size_t)(q - H) * H + j] = old[r] + acc[r];
+            else f.db2[j] = acc[r];
+        }
+    }
+}
 // phase 0: the rows that feed dw0 and db2 (q >= H; the tail kernel reads dw0, so these run first, on the main stream); phase 1: dW3 and the
-// dW2 rows (q < H), which nothing but AdamW reads - next to the tail kernel on the second stream
+// dW2 rows (q < H), which nothing but AdamW reads - next to the tail kernel on the second stream.  WIDE: the actor has 32 < NO <= 128 outputs
+// (the critic's one output always takes the narrow bodies).
+template <bool WIDE>
 __global__ void __launch_bounds__(512) ts_dw3_assemble_kernel(const TsDw3Args fa, int blocks_a, const TsDw3Args fc, int blocks_c,
                                                               float* __restrict__ part, int* __restrict__ done, int rank_a, int rank_c, int phase) {
     pdl_grid_begin();
     extern __shared__ float dw3_sm[];
     int b = blockIdx.x;
     if (phase == 1) {
-        if (b < blocks_a) { ts_dw3_assemble_body(fa, b, dw3_sm, part, done); return; }
+        if (b < blocks_a) { ts_dw3_assemble_body<WIDE>(fa, b, dw3_sm, part, done); return; }
         b -= blocks_a;
-        if (b < blocks_c) { ts_dw3_assemble_body(fc, b, dw3_sm, part + (size_t)blocks_a * 32 * fa.NO, done + blocks_a / DW3_KS); return; }
+        if (b < blocks_c) { ts_dw3_assemble_body<false>(fc, b, dw3_sm, part + (size_t)blocks_a * 32 * fa.NO, done + blocks_a / DW3_KS); return; }
         b -= blocks_c;
     }
     const int ra0 = phase == 0 ? fa.H : 0, ra1 = phase == 0 ? fa.H + fa.KP0 + 1 : fa.H;
     const int rc0 = phase == 0 ? fc.H : 0, rc1 = phase == 0 ? fc.H + fc.KP0 + 1 : fc.H;
-    if (b < rank_a) { ts_rank_rows_body(fa, b, dw3_sm, ra0, ra1); return; }
+    if (b < rank_a) {
+        if (WIDE) ts_rank_rows_wide_body(fa, b, dw3_sm, ra0, ra1); else ts_rank_rows_body(fa, b, dw3_sm, ra0, ra1);
+        return;
+    }
     b -= rank_a;
     if (b < rank_c) ts_rank_rows_body(fc, b, dw3_sm, rc0, rc1);
 }
@@ -1793,16 +1870,19 @@ static int ts_dw3_assemble(dppo_handle* h, cudaStream_t s, int actor_net, const 
         nrc = phase == 0 ? tc_nblk((size_t)KP0r, DW3_RB) : tc_nblk((size_t)g.Hc, DW3_RB);
     }
     const int nba = tc_nblk((size_t)g.H, 32) * tsDW3KS();
-    auto smf = [&](const TsDw3Args& f) {
-        const int K = f.H + f.A + f.Do + f.T;
-        const size_t a = (size_t)(((K + DW3_KS - 1) / DW3_KS) * f.NO + 16 * 32 * f.NO), b = (size_t)(DW3_RB * f.NO + f.H * (f.NO + 1));
+    const bool wide = fa.NO > 32;
+    auto smf = [&](const TsDw3Args& f, bool w) {
+        const int K = f.H + f.A + f.Do + f.T, nc = w ? DW3_WC : f.NO, n3 = w ? 32 : f.NO;
+        const size_t a = (size_t)(((K + DW3_KS - 1) / DW3_KS) * f.NO + 16 * 32 * nc), b = (size_t)(DW3_RB * f.NO + f.H * (n3 + 1));
         return (a > b ? a : b) * sizeof(float);
     };
     auto kper = [&](const TsDw3Args& f) { return (f.H + f.A + f.Do + f.T + DW3_KS - 1) / DW3_KS; };
-    const size_t sm = smf(fa) > smf(fc) ? smf(fa) : smf(fc);
-    static bool attr_set_dev[64] = {};
-    if (!attr_set_dev[h->device & 63]) { CUDA_TRY(cudaFuncSetAttribute(ts_dw3_assemble_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024)); attr_set_dev[h->device & 63] = true; }
-    if (sm > 100 * 1024 || g.A > 32 || kper(fa) > 128 || kper(fc) > 128) DPPO_FAIL(-7, "ts_dw3_assemble: shape not covered");
+    // (without the critic fc is a copy of fa: size it as the actor)
+    const size_t sm = smf(fa, wide) > smf(fc, fc.NO > 32) ? smf(fa, wide) : smf(fc, fc.NO > 32);
+    auto kern = wide ? ts_dw3_assemble_kernel<true> : ts_dw3_assemble_kernel<false>;
+    static bool attr_set_dev[2][64] = {};
+    if (!attr_set_dev[wide][h->device & 63]) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024)); attr_set_dev[wide][h->device & 63] = true; }
+    if (sm > 100 * 1024 || g.A > 128 || kper(fa) > 128 || kper(fc) > 128) DPPO_FAIL(-7, "ts_dw3_assemble: shape not covered");
     TsState* st = h->ts;
     // buffer: [256 chunk counters (always at the front: launches with and without the critic share them, every launch leaves them zero)
     //          | partial tiles]
@@ -1816,7 +1896,7 @@ static int ts_dw3_assemble(dppo_handle* h, cudaStream_t s, int actor_net, const 
     }
     int* done = reinterpret_cast<int*>(st->dw3_buf);
     float* partb = reinterpret_cast<float*>(st->dw3_buf + 1024);
-    CUDA_TRY(launch_pdl(ts_dw3_assemble_kernel, dim3((phase == 1 ? nba + nbc : 0) + nra + nrc), dim3(512), sm, s, fa, nba, fc, nbc, partb, done, nra, nrc, phase));
+    CUDA_TRY(launch_pdl(kern, dim3((phase == 1 ? nba + nbc : 0) + nra + nrc), dim3(512), sm, s, fa, nba, fc, nbc, partb, done, nra, nrc, phase));
     TC_KCHECK(h);
     return 0;
 }
@@ -1864,7 +1944,7 @@ static int ts_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, flo
 // h0 pack | folded output layers + adv-stats (second stream) | 3 + 3 forward | loss | 3 + 3 backward | grouped dW + reduce | tail || dW3 assembly.
 // shapes / alignment the index-driven variant needs (float4 row reads of the resident rollout buffers)
 static bool ts_ppo_indexed_ok(const dppo_handle* h, const TcIdxView& v) {
-    return (h->g.A % 4 == 0) && h->g.A <= 32 && ((((uintptr_t)v.chains | (uintptr_t)v.olp) & 15) == 0);
+    return (h->g.A % 4 == 0) && h->g.A <= 128 && ((((uintptr_t)v.chains | (uintptr_t)v.olp) & 15) == 0);
 }
 // idx (optional): the minibatch is given as flat (rollout row, denoising index) indices into the resident rollout buffers; the h0 pack,
 // the advantage statistics and the loss kernel address those buffers directly (no gathered copy), the row pointers are unused
@@ -1875,28 +1955,33 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     const size_t nA = g.ao.n, nC = g.co.n;
     float* gr = h->grads;
     const bool amish = h->cfg.actor_act == DPPO_ACT_MISH, cmish = h->cfg.critic_act == DPPO_ACT_MISH;
-    const bool loss8 = idx ? true : (g.A % 4 == 0) && g.A <= 32 && ((((uintptr_t)prev | (uintptr_t)nxt | (uintptr_t)oldlogp) & 15) == 0);   // float4 row reads
-    const int nlb = loss8 ? tc_nblk(N, LOSS8_ROWS) : tc_nblk(N, 128);
+    // float4 row reads (the indexed program is only taken when ts_ppo_indexed_ok holds)
+    const bool loss8 = (g.A % 4 == 0) && g.A <= 128 && (idx || ((((uintptr_t)prev | (uintptr_t)nxt | (uintptr_t)oldlogp) & 15) == 0));
+    const int NOP = ts_nop(g.A);                                  // the actor's seed width: 64 (A <= 32) or 128
+    const bool wide = NOP > 64;                                   // the loss kernel takes a warp per row (tc_ppo_loss8_kernel<32>)
+    const int NOg = g.A > 32 ? g.A : 32;                          // columns of the a1^T dout / h0^T dout scratch
+    if (idx && !loss8) DPPO_FAIL(-7, "ts_ppo_step: the indexed update needs A %% 4 == 0 and A <= 128");
+    const int nlb = loss8 ? tc_nblk(N, wide ? 256 / 32 : LOSS8_ROWS) : tc_nblk(N, 128);
     const int nrb = (N + 31) / 32;
     const size_t pf = ts_part_floats(h, g.H);
     const size_t need = ts_mlp_ws_bytes(N, g.H, KP0, amish, true) + ts_mlp_ws_bytes(N, g.Hc, KP0, cmish, true)
-                      + 2 * ws_bytes((size_t)N * g.A, 4) + 2 * ws_bytes(N, 4) + 4 * ws_bytes((size_t)N * 64, 2)
+                      + 2 * ws_bytes((size_t)N * g.A, 4) + 2 * ws_bytes(N, 4) + 2 * ws_bytes((size_t)N * NOP, 2) + 2 * ws_bytes((size_t)N * 64, 2)
                       + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes((size_t)KP0 * g.Hc, 4) + ws_bytes((size_t)nlb * 5, 8) + ws_bytes(16, 4)
                       + ws_bytes((size_t)nlb * (g.A + 1), 4) + ws_bytes((size_t)nrb * 2 * g.H, 4) + ws_bytes((size_t)nrb * 2 * g.Hc, 4)
-                      + ws_bytes((size_t)(g.H + g.Hc + 2 * KP0) * 32 + g.H + g.Hc, 4);
+                      + ws_bytes((size_t)(g.H + g.Hc + 2 * KP0) * NOg + g.H + g.Hc, 4);
     DPPO_TRY(ws_reserve(h, need, s));
     TsMlp ma, mc; ts_actor_mlp(h, DPPO_NET_ACTOR_FT, ma); ts_critic_mlp(h, mc);
     ts_mlp_take(h, N, ma, true); ts_mlp_take(h, N, mc, true);
     float* eps = ws_take<float>(h, (size_t)N * g.A); float* deps = ws_take<float>(h, (size_t)N * g.A);
     float* val = ws_take<float>(h, N); float* dval = ws_take<float>(h, N);
-    SplitT depsb = ts_take(h, (size_t)N * 64, 2), dvalb = ts_take(h, (size_t)N * 64, 2);
+    SplitT depsb = ts_take(h, (size_t)N * NOP, 2), dvalb = ts_take(h, (size_t)N * 64, 2);
     float* part = ws_take<float>(h, pf);
     float* dw0a = ws_take<float>(h, (size_t)KP0 * g.H); float* dw0c = ws_take<float>(h, (size_t)KP0 * g.Hc);
     double* bsum = ws_take<double>(h, (size_t)nlb * 5);
     int* ebeg = ws_take<int>(h, 16);
     float* colb3 = ws_take<float>(h, (size_t)nlb * (g.A + 1));
     float* cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H); float* cpc = ws_take<float>(h, (size_t)nrb * 2 * g.Hc);
-    float* gfold = ws_take<float>(h, (size_t)(g.H + g.Hc + 2 * KP0) * 32 + g.H + g.Hc);       // a1^T dout / h0^T dout of both nets (folded output layer) + scratch
+    float* gfold = ws_take<float>(h, (size_t)(g.H + g.Hc + 2 * KP0) * NOg + g.H + g.Hc);      // a1^T dout / h0^T dout of both nets (folded output layer) + scratch
     float* ga1 = gfold; float* ga0 = ga1 + (size_t)g.H * g.A; float* gc1 = ga0 + (size_t)KP0 * g.A; float* gc0 = gc1 + g.Hc;
     ma.out = eps; mc.out = val;
     // The critic's GEMMs are independent of the actor's until the loss (and again until the weight gradients) and their tiles are
@@ -1954,14 +2039,15 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
         // loss, metric partial sums, the two-plane padded gradient seeds and the output-bias column partials in one pass
         TcIdxView iv; memset(&iv, 0, sizeof(iv));
         if (idx) iv = *idx;
-        tc_ppo_loss8_kernel<<<nlb, 256, 0, s>>>(prev, nxt, eps, inds, returns, oldvalues, advantages, oldlogp, val, h->scalars, h->sched, hp, N,
-                                               depsb.p[0], dvalb.p[0], bsum, colb3, iv, depsb.p[1], dvalb.p[1]);
+        auto loss = wide ? tc_ppo_loss8_kernel<32> : tc_ppo_loss8_kernel<8>;
+        loss<<<nlb, 256, 0, s>>>(prev, nxt, eps, inds, returns, oldvalues, advantages, oldlogp, val, h->scalars, h->sched, hp, N,
+                                 depsb.p[0], dvalb.p[0], bsum, colb3, iv, depsb.p[1], dvalb.p[1]);
         TC_KCHECK(h);
     } else {
         ppo_loss_kernel<<<nlb, 128, 0, s>>>(prev, nxt, eps, inds, returns, oldvalues, advantages, oldlogp, val, h->scalars, h->sched, hp, N, deps, dval, bsum);
         TC_KCHECK(h);
-        ts_pad64_kernel<<<tc_nblk((size_t)N * 8, 256), 256, 0, s>>>(deps, N, g.A, depsb.p[0], depsb.p[1]); TC_KCHECK(h);
-        ts_pad64_kernel<<<tc_nblk((size_t)N * 8, 256), 256, 0, s>>>(dval, N, 1, dvalb.p[0], dvalb.p[1]); TC_KCHECK(h);
+        ts_pad64_kernel<<<tc_nblk((size_t)N * (NOP / 8), 256), 256, 0, s>>>(deps, N, g.A, NOP, depsb.p[0], depsb.p[1]); TC_KCHECK(h);
+        ts_pad64_kernel<<<tc_nblk((size_t)N * 8, 256), 256, 0, s>>>(dval, N, 1, 64, dvalb.p[0], dvalb.p[1]); TC_KCHECK(h);
     }
     // both backward chains, then ONE grouped launch with the eight weight-gradient products of actor and critic
     DPPO_TRY(fork());
@@ -1977,7 +2063,7 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 0));
     DPPO_TRY(fork());
     DPPO_TRY(ts_dw3_assemble(h, sc, DPPO_NET_ACTOR_FT, ga1, ga0, gr, dw0a, gc1, gc0, gr + nA, dw0c, 1));
-    float* b2scr = gfold + (size_t)(g.H + g.Hc + 2 * KP0) * 32;      // the unwritten slot-0 column sums land here, not in db2
+    float* b2scr = gfold + (size_t)(g.H + g.Hc + 2 * KP0) * NOg;     // the unwritten slot-0 column sums land here, not in db2
     if (loss8) {
         DPPO_TRY(tc_launch_tail(h, s, bsum, nlb, hp.inv_nglobal, frac_local, colb3, cpa, nrb, cpc, nrb, dw0a, dw0c, b2scr, b2scr + g.H));
         DPPO_TRY(join());
@@ -2005,18 +2091,19 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     const size_t ne = (size_t)N * g.A;
     const int nlb = tc_nblk(ne, 256);
     const int nrb = (N + 31) / 32;
+    const int NOP = ts_nop(g.A), NOg = g.A > 32 ? g.A : 32;
     const size_t pf = ts_part_floats(h, g.H);
     const size_t need = ts_mlp_ws_bytes(N, g.H, KP0, h->cfg.actor_act == DPPO_ACT_MISH, true) + 4 * ws_bytes(ne, 4) + ws_bytes(N, 4)
-                      + 2 * ws_bytes((size_t)N * 64, 2) + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes(nlb, 8) + ws_bytes(16, 4)
-                      + ws_bytes((size_t)nrb * 2 * g.H, 4) + ws_bytes((size_t)(g.H + KP0) * 32 + g.H, 4);
+                      + 2 * ws_bytes((size_t)N * NOP, 2) + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes(nlb, 8) + ws_bytes(16, 4)
+                      + ws_bytes((size_t)nrb * 2 * g.H, 4) + ws_bytes((size_t)(g.H + KP0) * NOg + g.H, 4);
     DPPO_TRY(ws_reserve(h, need, s));
     TsMlp ma; ts_actor_mlp(h, DPPO_NET_ACTOR, ma);
     ts_mlp_take(h, N, ma, true);
-    float* ga1 = ws_take<float>(h, (size_t)(g.H + KP0) * 32 + g.H); float* ga0 = ga1 + (size_t)g.H * g.A;     // + scratch for the unwritten slot-0 sums
+    float* ga1 = ws_take<float>(h, (size_t)(g.H + KP0) * NOg + g.H); float* ga0 = ga1 + (size_t)g.H * g.A;    // + scratch for the unwritten slot-0 sums
     DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR, s));
     float* eps = ws_take<float>(h, ne); float* deps = ws_take<float>(h, ne); float* noise = ws_take<float>(h, ne); float* xn = ws_take<float>(h, ne);
     int* trow = ws_take<int>(h, N);
-    SplitT depsb = ts_take(h, (size_t)N * 64, 2);
+    SplitT depsb = ts_take(h, (size_t)N * NOP, 2);
     float* part = ws_take<float>(h, pf);
     float* dw0 = ws_take<float>(h, (size_t)KP0 * g.H);
     double* bsum = ws_take<double>(h, nlb);
@@ -2029,13 +2116,13 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     const float scale = 1.0f / ((float)N_global * (float)g.A);
     mse_loss_kernel<<<nlb, 256, 0, s>>>(eps, noise, ne, scale, deps, bsum); TC_KCHECK(h);
     sum_blocks_kernel<<<1, 256, 0, s>>>(bsum, nlb, scale, gr + nA); TC_KCHECK(h);
-    ts_pad64_kernel<<<tc_nblk((size_t)N * 8, 256), 256, 0, s>>>(deps, N, g.A, depsb.p[0], depsb.p[1]); TC_KCHECK(h);
+    ts_pad64_kernel<<<tc_nblk((size_t)N * (NOP / 8), 256), 256, 0, s>>>(deps, N, g.A, NOP, depsb.p[0], depsb.p[1]); TC_KCHECK(h);
     DPPO_TRY(ts_mlp_backward_dx(h, s, ma, depsb, N, cpa));
     tsp::DwDesc dd[5];
     const int nd = ts_mlp_dw_descs(ma, depsb, N, gr, g.ao.w1, dw0, dd, ga1, ga0);
     DPPO_TRY(tsp::launch_dw_pair(h, s, dd, nd, N, part, pf, ebeg));
     DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR, ga1, ga0, gr, dw0, nullptr, nullptr, nullptr, nullptr));
-    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ga1 + (size_t)(g.H + KP0) * 32, g.H, gr + g.ao.b1); TC_KCHECK(h);
+    tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ga1 + (size_t)(g.H + KP0) * NOg, g.H, gr + g.ao.b1); TC_KCHECK(h);
     DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
     CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR, dw0 + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
     unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);

@@ -45,7 +45,9 @@ enum {
                            fp32 epilogues; looser bound stated in DESIGN.md                         */
     DPPO_PREC_BF16X3 = 2 /* tcgen05, every operand as bf16 hi + lo planes and every product as
                            hi*hi + lo*hi + hi*lo into one fp32 TMEM accumulator: meets the fp32
-                           parity tolerance (1e-4 rel / 1e-3 abs) on the tensor pipe               */
+                           parity tolerance (1e-4 rel / 1e-3 abs) on the tensor pipe.  Covers action
+                           chunks A = horizon_steps * action_dim <= 128; a wider chunk runs every
+                           call on the FFMA path of DPPO_PREC_FP32                                  */
 };
 /* optimizer slots */
 enum { DPPO_OPT_PRETRAIN = 0 /* actor */, DPPO_OPT_FINETUNE = 1 /* actor_ft ++ critic */ };
