@@ -1062,16 +1062,10 @@ extern "C" int dppo_ppo_step(dppo_handle* h, const float* obs, const float* prev
         double* bsum = ws_take<double>(h, (size_t)nlb * 5);
 
         make_trow_kernel<<<nblk(N, 256), 256, 0, s>>>(inds, N, g.K, 0, trow); KLAUNCH(h); KCHECK();
-        if (adv_std < 0.f) { adv_stats_kernel<<<1, 1024, 0, s>>>(advantages, N, h->scalars); KLAUNCH(h); KCHECK(); }
-        else { set_scalars_kernel<<<1, 1, 0, s>>>(h->scalars, adv_mean, adv_std); KLAUNCH(h); KCHECK(); }
+        DPPO_TRY(launch_adv_stats(h, s, advantages, nullptr, N, adv_mean, adv_std));
         DPPO_TRY(actor_fwd_fp32(h, s, DPPO_NET_ACTOR_FT, prev, obs, 1, N, trow, 0, fa));
         DPPO_TRY(critic_fwd_fp32(h, s, obs, N, fc));
-        PpoHyper hp;
-        hp.A = g.A; hp.Da = h->cfg.action_dim; hp.K = g.K; hp.T = g.T; hp.reward_horizon = h->cfg.reward_horizon; hp.norm_adv = h->cfg.norm_adv;
-        hp.dcv = h->cfg.denoised_clip_value; hp.min_lp_std = h->cfg.min_logprob_denoising_std;
-        hp.lp_lo = h->cfg.logprob_clip_lo; hp.lp_hi = h->cfg.logprob_clip_hi; hp.gamma_d = h->cfg.gamma_denoising;
-        hp.clip_coef = h->cfg.clip_ploss_coef; hp.clip_base = h->cfg.clip_ploss_coef_base; hp.clip_rate = h->cfg.clip_ploss_coef_rate;
-        hp.clip_v = h->cfg.clip_vloss_coef; hp.vf_coef = h->cfg.vf_coef; hp.inv_nglobal = 1.0f / (float)N_global;
+        const PpoHyper hp = ppo_hyper(h, N_global);
         ppo_loss_kernel<<<nlb, 128, 0, s>>>(prev, nxt, fa.out, inds, returns, oldvalues, advantages, oldlogp, fc.out,
                                            h->scalars, h->sched, hp, N, deps, dval, bsum); KLAUNCH(h); KCHECK();
         ppo_metrics_kernel<<<1, 256, 0, s>>>(bsum, nlb, hp.inv_nglobal, (float)((double)N / (double)N_global), gr + nA + nC); KLAUNCH(h); KCHECK();

@@ -431,6 +431,57 @@ struct PpoHyper {
     float dcv, min_lp_std, lp_lo, lp_hi, gamma_d, clip_coef, clip_base, clip_rate, clip_v, vf_coef;
     float inv_nglobal;
 };
+static PpoHyper ppo_hyper(const dppo_handle* h, int64_t N_global) {
+    const dppo_cfg& c = h->cfg;
+    PpoHyper hp;
+    hp.A = h->g.A; hp.Da = c.action_dim; hp.K = h->g.K; hp.T = h->g.T; hp.reward_horizon = c.reward_horizon; hp.norm_adv = c.norm_adv;
+    hp.dcv = c.denoised_clip_value; hp.min_lp_std = c.min_logprob_denoising_std;
+    hp.lp_lo = c.logprob_clip_lo; hp.lp_hi = c.logprob_clip_hi; hp.gamma_d = c.gamma_denoising;
+    hp.clip_coef = c.clip_ploss_coef; hp.clip_base = c.clip_ploss_coef_base; hp.clip_rate = c.clip_ploss_coef_rate;
+    hp.clip_v = c.clip_vloss_coef; hp.vf_coef = c.vf_coef; hp.inv_nglobal = 1.0f / (float)N_global;
+    return hp;
+}
+// The per-row loss math of every loss kernel (the kernels differ in row layout, loads, seed formula and reductions only).
+// Policy part from the row's means of the clamped new / old log-probs, the raw advantage and the denoising index:
+// dnew = d loss / d newm for this row, already scaled by 1 / N_global.
+struct PpoRowPolicy { float pg, clipc, ratio, logratio, dnew; };
+__device__ __forceinline__ PpoRowPolicy ppo_row_policy(float newm, float oldm, float adv, const float* __restrict__ advstats, int ind,
+                                                       const PpoHyper& hp) {
+    PpoRowPolicy o;
+    if (hp.norm_adv) adv = (adv - advstats[0]) / (advstats[1] + 1e-8f);
+    adv *= powf(hp.gamma_d, (float)(hp.K - ind - 1));
+    o.logratio = newm - oldm; o.ratio = expf(o.logratio);
+    // exponential clip schedule over the denoising index; K = 1 takes clip coefficient 0 (the reference divides 0 by 0)
+    const float tt = hp.K > 1 ? (float)ind / (float)(hp.K - 1) : (float)ind;
+    o.clipc = hp.K > 1 ? hp.clip_base + (hp.clip_coef - hp.clip_base) * (expf(hp.clip_rate * tt) - 1.f) / (expf(hp.clip_rate) - 1.f) : tt;
+    const float rc = fminf(fmaxf(o.ratio, 1.f - o.clipc), 1.f + o.clipc);
+    const float pg1 = -adv * o.ratio, pg2 = -adv * rc;
+    o.pg = fmaxf(pg1, pg2);
+    // d pg / d ratio: tf.maximum sends the gradient to pg1 on ties; clip_by_value passes inside the range
+    const float dpg = (pg1 >= pg2) ? -adv : ((o.ratio >= 1.f - o.clipc && o.ratio <= 1.f + o.clipc) ? -adv : 0.f);
+    o.dnew = dpg * o.ratio * hp.inv_nglobal;
+    return o;
+}
+// value loss of the row (clipped when clip_v >= 0; *oldvalue is read only then) and its seed vf_coef * dv / N_global
+struct PpoRowValue { float vl, seed; };
+__device__ __forceinline__ PpoRowValue ppo_row_value(float v, float ret, const float* __restrict__ oldvalue, const PpoHyper& hp) {
+    float vl, dv;
+    if (hp.clip_v >= 0.f) {
+        const float ov = *oldvalue;
+        const float un = (v - ret) * (v - ret);
+        const float dcl = v - ov;
+        const float vc = ov + fminf(fmaxf(dcl, -hp.clip_v), hp.clip_v);
+        const float cl = (vc - ret) * (vc - ret);
+        if (un >= cl) { vl = 0.5f * un; dv = (v - ret); }
+        else { vl = 0.5f * cl; dv = (dcl >= -hp.clip_v && dcl <= hp.clip_v) ? (vc - ret) : 0.f; }
+    } else { vl = 0.5f * (v - ret) * (v - ret); dv = (v - ret); }
+    return {vl, hp.vf_coef * dv * hp.inv_nglobal};
+}
+// the row's terms of the five metric sums
+__device__ __forceinline__ void ppo_row_metrics(double acc[5], const PpoRowPolicy& p, float vl) {
+    acc[0] = p.pg; acc[1] = vl; acc[2] = (fabsf(p.ratio - 1.f) > p.clipc) ? 1.0 : 0.0;
+    acc[3] = (p.ratio - 1.f) - p.logratio; acc[4] = p.ratio;
+}
 // flat != nullptr: row i of the minibatch is rollout row flat[i] / K (index-driven minibatch); out-of-range indices read row 0
 __global__ void adv_stats_kernel(const float* __restrict__ adv, int N, float* __restrict__ out /*mean,std*/,
                                  const int* __restrict__ flat = nullptr, int K = 1, long long P = 0) {
@@ -473,18 +524,7 @@ __global__ void __launch_bounds__(128) ppo_loss_kernel(
             oldm += fminf(fmaxf(oldlogp[i], hp.lp_lo), hp.lp_hi);
         }
         newm /= (float)nuse; oldm /= (float)nuse;
-        float adv = advantages[r];
-        if (hp.norm_adv) adv = (adv - advstats[0]) / (advstats[1] + 1e-8f);
-        adv *= powf(hp.gamma_d, (float)(hp.K - ind - 1));
-        float logratio = newm - oldm, ratio = expf(logratio);
-        float tt = hp.K > 1 ? (float)ind / (float)(hp.K - 1) : (float)ind;
-        float clipc = hp.K > 1 ? hp.clip_base + (hp.clip_coef - hp.clip_base) * (expf(hp.clip_rate * tt) - 1.f) / (expf(hp.clip_rate) - 1.f) : tt;
-        float rc = fminf(fmaxf(ratio, 1.f - clipc), 1.f + clipc);
-        float pg1 = -adv * ratio, pg2 = -adv * rc;
-        float pg = fmaxf(pg1, pg2);
-        // d pg / d ratio: tf.maximum sends the gradient to pg1 on ties; clip_by_value passes inside the range
-        float dpg = (pg1 >= pg2) ? -adv : ((ratio >= 1.f - clipc && ratio <= 1.f + clipc) ? -adv : 0.f);
-        float dnew = dpg * ratio * hp.inv_nglobal;
+        const PpoRowPolicy p = ppo_row_policy(newm, oldm, advantages[r], advstats, ind, hp);
         for (int a = 0; a < A; ++a) {
             size_t i = (size_t)r * A + a;
             float g = 0.f;
@@ -492,24 +532,13 @@ __global__ void __launch_bounds__(128) ppo_loss_kernel(
                 float z, sd; bool in;
                 float lp = logprob_elem(prev[i], eps[i], nxt[i], t, sch, hp.T, hp.dcv, hp.min_lp_std, &z, &sd, &in);
                 if (lp >= hp.lp_lo && lp <= hp.lp_hi && in)
-                    g = dnew / (float)nuse * (z / sd) * sch[SCH_COEF1 * hp.T + t] * (-sch[SCH_SQRT_RECIPM1 * hp.T + t]);
+                    g = p.dnew / (float)nuse * (z / sd) * sch[SCH_COEF1 * hp.T + t] * (-sch[SCH_SQRT_RECIPM1 * hp.T + t]);
             }
             deps[i] = g;
         }
-        // value loss
-        float v = newvalues[r], ret = returns[r], vl, dv;
-        if (hp.clip_v >= 0.f) {
-            float ov = oldvalues[r];
-            float un = (v - ret) * (v - ret);
-            float dcl = v - ov;
-            float vc = ov + fminf(fmaxf(dcl, -hp.clip_v), hp.clip_v);
-            float cl = (vc - ret) * (vc - ret);
-            if (un >= cl) { vl = 0.5f * un; dv = (v - ret); }
-            else { vl = 0.5f * cl; dv = (dcl >= -hp.clip_v && dcl <= hp.clip_v) ? (vc - ret) : 0.f; }
-        } else { vl = 0.5f * (v - ret) * (v - ret); dv = (v - ret); }
-        dvalue[r] = hp.vf_coef * dv * hp.inv_nglobal;
-        acc[0] = pg; acc[1] = vl; acc[2] = (fabsf(ratio - 1.f) > clipc) ? 1.0 : 0.0;
-        acc[3] = (ratio - 1.f) - logratio; acc[4] = ratio;
+        const PpoRowValue vr = ppo_row_value(newvalues[r], returns[r], oldvalues + r, hp);
+        dvalue[r] = vr.seed;
+        ppo_row_metrics(acc, p, vr.vl);
     }
     __shared__ double red[5][128];
     for (int k = 0; k < 5; ++k) red[k][threadIdx.x] = acc[k];

@@ -318,34 +318,13 @@ __global__ void __launch_bounds__(128) tc_ppo_loss_kernel(
             }
         }
         newm /= (float)nuse; oldm /= (float)nuse;
-        float adv = advantages[r];
-        if (hp.norm_adv) adv = (adv - advstats[0]) / (advstats[1] + 1e-8f);
-        adv *= powf(hp.gamma_d, (float)(hp.K - ind - 1));
-        const float logratio = newm - oldm, ratio = expf(logratio);
-        const float tt = hp.K > 1 ? (float)ind / (float)(hp.K - 1) : (float)ind;
-        const float clipc = hp.K > 1 ? hp.clip_base + (hp.clip_coef - hp.clip_base) * (expf(hp.clip_rate * tt) - 1.f) / (expf(hp.clip_rate) - 1.f) : tt;
-        const float rc = fminf(fmaxf(ratio, 1.f - clipc), 1.f + clipc);
-        const float pg1 = -adv * ratio, pg2 = -adv * rc;
-        const float pg = fmaxf(pg1, pg2);
-        const float dpg = (pg1 >= pg2) ? -adv : ((ratio >= 1.f - clipc && ratio <= 1.f + clipc) ? -adv : 0.f);
-        const float gscale = dpg * ratio * hp.inv_nglobal / (float)nuse / sd * sc.c1 * (-sc.srm1);
+        const PpoRowPolicy p = ppo_row_policy(newm, oldm, advantages[r], advstats, ind, hp);
+        const float gscale = p.dnew / (float)nuse / sd * sc.c1 * (-sc.srm1);
 #pragma unroll
         for (int a = 0; a < 32; ++a) gout[a] = ((live >> a) & 1u) ? gscale * zs[a] : 0.f;
-        // value loss
-        const float v = newvalues[r], ret = returns[r];
-        float vl, dv;
-        if (hp.clip_v >= 0.f) {
-            const float ov = oldvalues[r];
-            const float un = (v - ret) * (v - ret);
-            const float dcl = v - ov;
-            const float vc = ov + fminf(fmaxf(dcl, -hp.clip_v), hp.clip_v);
-            const float cl = (vc - ret) * (vc - ret);
-            if (un >= cl) { vl = 0.5f * un; dv = (v - ret); }
-            else { vl = 0.5f * cl; dv = (dcl >= -hp.clip_v && dcl <= hp.clip_v) ? (vc - ret) : 0.f; }
-        } else { vl = 0.5f * (v - ret) * (v - ret); dv = (v - ret); }
-        dv_out = hp.vf_coef * dv * hp.inv_nglobal;
-        acc[0] = pg; acc[1] = vl; acc[2] = (fabsf(ratio - 1.f) > clipc) ? 1.0 : 0.0;
-        acc[3] = (ratio - 1.f) - logratio; acc[4] = ratio;
+        const PpoRowValue vr = ppo_row_value(newvalues[r], returns[r], oldvalues + r, hp);
+        dv_out = vr.seed;
+        ppo_row_metrics(acc, p, vr.vl);
         // padded bf16 rows: [deps (A) | 0..] and [dvalue | 0..]
         uint4* drow = reinterpret_cast<uint4*>(depsb + (size_t)r * 64);
 #pragma unroll
@@ -450,18 +429,8 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
 #pragma unroll
     for (int off = 1; off < LPR; off <<= 1) { newp += __shfl_xor_sync(0xffffffffu, newp, off); oldp += __shfl_xor_sync(0xffffffffu, oldp, off); }
     if (row_ok) {
-        const float newm = newp / (float)nuse, oldm = oldp / (float)nuse;
-        float adv = advantages[srow];
-        if (hp.norm_adv) adv = (adv - advstats[0]) / (advstats[1] + 1e-8f);
-        adv *= powf(hp.gamma_d, (float)(hp.K - ind - 1));
-        const float logratio = newm - oldm, ratio = expf(logratio);
-        const float tt = hp.K > 1 ? (float)ind / (float)(hp.K - 1) : (float)ind;
-        const float clipc = hp.K > 1 ? hp.clip_base + (hp.clip_coef - hp.clip_base) * (expf(hp.clip_rate * tt) - 1.f) / (expf(hp.clip_rate) - 1.f) : tt;
-        const float rc = fminf(fmaxf(ratio, 1.f - clipc), 1.f + clipc);
-        const float pg1 = -adv * ratio, pg2 = -adv * rc;
-        const float pg = fmaxf(pg1, pg2);
-        const float dpg = (pg1 >= pg2) ? -adv : ((ratio >= 1.f - clipc && ratio <= 1.f + clipc) ? -adv : 0.f);
-        const float gscale = dpg * ratio * hp.inv_nglobal / (float)nuse / sd * sc.c1 * (-sc.srm1);
+        const PpoRowPolicy p = ppo_row_policy(newp / (float)nuse, oldp / (float)nuse, advantages[srow], advstats, ind, hp);
+        const float gscale = p.dnew / (float)nuse / sd * sc.c1 * (-sc.srm1);
 #pragma unroll
         for (int e = 0; e < 4; ++e) gq[e] = ((live >> e) & 1u) ? gscale * z[e] : 0.f;
         // padded bf16 seed row [deps (A) | 0..]: this lane's 4 columns and 4 of the zero columns
@@ -477,20 +446,9 @@ __global__ void __launch_bounds__(256) tc_ppo_loss8_kernel(
             if (LPR == 8) lrow[8 + sub] = make_uint2(0u, 0u);
         }
         if (sub == 0) {
-            const float v = newvalues[r], ret = returns[srow];
-            float vl, dv;
-            if (hp.clip_v >= 0.f) {
-                const float ov = oldvalues[srow];
-                const float un = (v - ret) * (v - ret);
-                const float dcl = v - ov;
-                const float vc = ov + fminf(fmaxf(dcl, -hp.clip_v), hp.clip_v);
-                const float cl = (vc - ret) * (vc - ret);
-                if (un >= cl) { vl = 0.5f * un; dv = (v - ret); }
-                else { vl = 0.5f * cl; dv = (dcl >= -hp.clip_v && dcl <= hp.clip_v) ? (vc - ret) : 0.f; }
-            } else { vl = 0.5f * (v - ret) * (v - ret); dv = (v - ret); }
-            dv_out = hp.vf_coef * dv * hp.inv_nglobal;
-            acc[0] = pg; acc[1] = vl; acc[2] = (fabsf(ratio - 1.f) > clipc) ? 1.0 : 0.0;
-            acc[3] = (ratio - 1.f) - logratio; acc[4] = ratio;
+            const PpoRowValue vr = ppo_row_value(newvalues[r], returns[srow], oldvalues + srow, hp);
+            dv_out = vr.seed;
+            ppo_row_metrics(acc, p, vr.vl);
         }
         // padded bf16 seed row [dvalue | 0..]: 16 bytes per lane
         uint4* vrow = reinterpret_cast<uint4*>(dvalb + (size_t)r * 64);
@@ -986,29 +944,48 @@ static int tc_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, flo
 static int colsum(dppo_handle* h, cudaStream_t s, const float* D, int ld, int N, int ncols, const int* seg, int nseg,
                   float* part, float* out);   // dppo_api.cu
 
+// The layer-0 gradients of both tensor modes (dw0 [KP0][H] in h0's row order) into the flat gradient as separate launches: the actor's
+// rows [A+Do, A+Do+T) are the per-t column sums of du (the gradient of the bt table, through the time backward) and its x / obs rows
+// are dW_in; the critic's obs rows are its dW_in and the ones column collected its input-layer bias gradient.
+// dw0c == nullptr: no critic (pre-training).  gr = [actor net's gradient (nA) | critic's].
+static int tc_scatter_dw0(dppo_handle* h, cudaStream_t s, int net, const float* dw0a, const float* dw0c, float* gr) {
+    const Geom& g = h->g;
+    CUDA_TRY(launch_time_backward(h, s, net, dw0a + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
+    unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0a, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
+    if (!dw0c) return 0;
+    float* gc = gr + g.ao.n;
+    unpack_dw0_kernel<<<tc_nblk((size_t)g.Do * g.Hc, 256), 256, 0, s>>>(dw0c + (size_t)g.A * g.Hc, 0, 0, g.Do, g.Hc, gc + g.co.win); TC_KCHECK(h);
+    CUDA_TRY(cudaMemcpyAsync(gc + g.co.bin, dw0c + (size_t)(g.A + g.Do + g.T) * g.Hc, g.Hc * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return 0;
+}
+// advantage statistics of the whole minibatch (diffusion_ppo.py:74-75) into h->scalars: computed (adv_std < 0) from adv [N] or, with
+// iv != nullptr, from the rollout advantages through the index view; else the given ones
+static int launch_adv_stats(dppo_handle* h, cudaStream_t s, const float* adv, const TcIdxView* iv, int N, float adv_mean, float adv_std) {
+    if (adv_std < 0.f) adv_stats_kernel<<<1, 1024, 0, s>>>(iv ? iv->adv : adv, N, h->scalars, iv ? iv->flat : nullptr, iv ? iv->K : 1, iv ? iv->P : 0);
+    else set_scalars_kernel<<<1, 1, 0, s>>>(h->scalars, adv_mean, adv_std);
+    TC_KCHECK(h);
+    return 0;
+}
+// The loss8 kernels (tc_ppo_loss8_kernel) read rows as float4: A % 4 == 0, A <= max_a (32 for LPR = 8, 128 for a warp per row) and the
+// row arrays 16-byte aligned (the minibatch's prev / nxt / oldlogp, or the index view's chains / olp)
+static bool loss8_ok(int A, int max_a, const void* p0, const void* p1, const void* p2 = nullptr) {
+    return A % 4 == 0 && A <= max_a && (((uintptr_t)p0 | (uintptr_t)p1 | (uintptr_t)p2) & 15) == 0;
+}
+// the second stream of the overlapped tensor schedules and its three events (fork, join, the split-precision fold), made on first use
+static int ensure_aux_stream(dppo_handle* h) {
+    if (h->aux_stream) return 0;
+    CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
+    for (int i = 0; i < 3; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
+    return 0;
+}
+
 // actor backward from deps [N][A] fp32 (+ its padded bf16 copy): fills gnet[0 : nA]
 static int tc_actor_grads(dppo_handle* h, cudaStream_t s, int net, const TcMlp& m, const float* deps, const bf16* depsb, int N,
                           float* part, float* dw0, float* gnet) {
     const Geom& g = h->g;
     DPPO_TRY(tc_mlp_backward(h, s, m, depsb, N, part, gnet, g.ao.w1, g.ao.b1, g.ao.w2, g.ao.b2, g.ao.w3, dw0));
     if (deps) DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gnet + g.ao.b3));   // else: the loss kernel already reduced it
-    // dw0 rows [A+Do, A+Do+T) are the per-t column sums of du: the gradient of the bt table
-    CUDA_TRY(launch_time_backward(h, s, net, dw0 + (size_t)(g.A + g.Do) * g.H, gnet));
-    TC_KCHECK(h);
-    unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0, g.A, g.td, g.Do, g.H, gnet + g.ao.win);
-    TC_KCHECK(h);
-    return 0;
-}
-static int tc_critic_grads(dppo_handle* h, cudaStream_t s, const TcMlp& m, const float* dval, const bf16* dvalb, int N,
-                           float* part, float* dw0, float* gnet) {
-    const Geom& g = h->g;
-    DPPO_TRY(tc_mlp_backward(h, s, m, dvalb, N, part, gnet, g.co.w1, g.co.b1, g.co.w2, g.co.b2, g.co.w3, dw0));
-    if (dval) DPPO_TRY(colsum(h, s, dval, 1, N, 1, nullptr, 1, part, gnet + g.co.b3));
-    unpack_dw0_kernel<<<tc_nblk((size_t)g.Do * g.Hc, 256), 256, 0, s>>>(dw0 + (size_t)g.A * g.Hc, 0, 0, g.Do, g.Hc, gnet + g.co.win);
-    TC_KCHECK(h);
-    // the ones column of h0 collects the input-layer bias gradient
-    CUDA_TRY(cudaMemcpyAsync(gnet + g.co.bin, dw0 + (size_t)(g.A + g.Do + g.T) * g.Hc, g.Hc * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    return 0;
+    return tc_scatter_dw0(h, s, net, dw0, nullptr, gnet);
 }
 
 // PPODiffusion.c_loss + tape.gradient (diffusion_ppo.py:32-132, train_ppo_diffusion_agent.py:340-346) on the tensor path,
@@ -1076,35 +1053,21 @@ static int tc_ppo_begin(dppo_handle* h, cudaStream_t s, int N, int chunk_rows, i
         CUDA_TRY(cudaMemsetAsync(h->grads, 0, (nA + nC) * sizeof(float), s));
         CUDA_TRY(cudaMemsetAsync(P.dw0a, 0, acc_bytes, s));
     }
-    PpoHyper& hp = P.hp;
-    hp.A = g.A; hp.Da = h->cfg.action_dim; hp.K = g.K; hp.T = g.T; hp.reward_horizon = h->cfg.reward_horizon; hp.norm_adv = h->cfg.norm_adv;
-    hp.dcv = h->cfg.denoised_clip_value; hp.min_lp_std = h->cfg.min_logprob_denoising_std;
-    hp.lp_lo = h->cfg.logprob_clip_lo; hp.lp_hi = h->cfg.logprob_clip_hi; hp.gamma_d = h->cfg.gamma_denoising;
-    hp.clip_coef = h->cfg.clip_ploss_coef; hp.clip_base = h->cfg.clip_ploss_coef_base; hp.clip_rate = h->cfg.clip_ploss_coef_rate;
-    hp.clip_v = h->cfg.clip_vloss_coef; hp.vf_coef = h->cfg.vf_coef; hp.inv_nglobal = 1.0f / (float)N_global;
+    P.hp = ppo_hyper(h, N_global);
     return 0;
 }
-// advantage statistics for the whole minibatch (diffusion_ppo.py:74-75): given, or computed from the device array
+// advantage statistics for the whole minibatch: given, or computed from the device array
 static int tc_ppo_adv_stats(dppo_handle* h, cudaStream_t s, const float* advantages_all, int N, float adv_mean, float adv_std) {
     // only the loss kernel reads the statistics: with the two-stream schedule they are computed on the second stream, next to
     // pack_h0 and the forward chains (the join in front of the loss kernel orders them)
     TcPpoPlan& P = tc_plan(h);
     cudaStream_t st = s;
     if (P.ma.fused && P.mc.fused && !h->deterministic && !h->prof_on) {
-        if (!h->aux_stream) {
-            CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-            for (int i = 0; i < 2; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
-        }
+        DPPO_TRY(ensure_aux_stream(h));
         CUDA_TRY(cudaEventRecord(h->aux_ev[0], s)); CUDA_TRY(cudaStreamWaitEvent(h->aux_stream, h->aux_ev[0], 0));
         st = h->aux_stream;
     }
-    if (adv_std < 0.f) {
-        if (P.idx.flat) adv_stats_kernel<<<1, 1024, 0, st>>>(P.idx.adv, N, h->scalars, P.idx.flat, P.idx.K, P.idx.P);
-        else adv_stats_kernel<<<1, 1024, 0, st>>>(advantages_all, N, h->scalars);
-        TC_KCHECK(h);
-    }
-    else { set_scalars_kernel<<<1, 1, 0, st>>>(h->scalars, adv_mean, adv_std); TC_KCHECK(h); }
-    return 0;
+    return launch_adv_stats(h, st, advantages_all, P.idx.flat ? &P.idx : nullptr, N, adv_mean, adv_std);
 }
 // chunk size of the host pipeline: half waves of 128-row tiles (one tile per SM pair member), at most 7 chunks (+ the short lead
 // chunk); 0 = do not chunk.  Every chunk costs a start-up / drain of the four persistent chain kernels (~10 us each), so the
@@ -1124,8 +1087,7 @@ static int tc_ppo_chunk(dppo_handle* h, cudaStream_t s, int chunk, const float* 
     TcPpoPlan& P = tc_plan(h);
     if (n < 1 || n > P.chunk_rows || chunk < 0 || chunk >= P.nchunks) DPPO_FAIL(-1, "tc_ppo_chunk: bad chunk");
     const TcIdxView iv = P.idx;
-    const bool loss8 = (g.A % 4 == 0) && g.A <= 32 &&
-        (iv.flat ? ((((uintptr_t)iv.chains | (uintptr_t)iv.olp) & 15) == 0) : ((((uintptr_t)prev | (uintptr_t)nxt | (uintptr_t)oldlogp) & 15) == 0));   // float4 row reads
+    const bool loss8 = iv.flat ? loss8_ok(g.A, 32, iv.chains, iv.olp) : loss8_ok(g.A, 32, prev, nxt, oldlogp);
     if (iv.flat && (!loss8 || P.nchunks != 1)) DPPO_FAIL(-1, "tc_ppo_chunk: the index-driven minibatch needs A % 4 == 0, aligned buffers and a single chunk");
     const int nlb = loss8 ? tc_nblk(n, LOSS8_ROWS) : tc_nblk(n, 128);
     if (P.blocks_done + nlb > P.max_blocks) DPPO_FAIL(-1, "tc_ppo_chunk: partial-sum buffers exhausted");
@@ -1147,10 +1109,7 @@ static int tc_ppo_chunk(dppo_handle* h, cudaStream_t s, int chunk, const float* 
     // (391 row tiles on 148 SMs): the critic chain goes to a second stream so that its CTAs fill the actor chain's tail.
     // (not while the per-kernel profile is on: its event brackets are meant to time each kernel running alone)
     const bool overlap = defer && !h->prof_on;
-    if (overlap && !h->aux_stream) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-        for (int i = 0; i < 2; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
-    }
+    if (overlap) DPPO_TRY(ensure_aux_stream(h));
     auto fork = [&]() -> int { CUDA_TRY(cudaEventRecord(h->aux_ev[0], s)); CUDA_TRY(cudaStreamWaitEvent(h->aux_stream, h->aux_ev[0], 0)); return 0; };
     auto join = [&]() -> int { CUDA_TRY(cudaEventRecord(h->aux_ev[1], h->aux_stream)); CUDA_TRY(cudaStreamWaitEvent(s, h->aux_ev[1], 0)); return 0; };
     if (overlap) DPPO_TRY(fork());
@@ -1239,14 +1198,7 @@ static int tc_ppo_finish(dppo_handle* h, cudaStream_t s) {
     ppo_metrics_kernel<<<1, 256, 0, s>>>(P.bsum, P.blocks_done, P.hp.inv_nglobal, (float)((double)P.N / (double)P.N_global), gr + nA + nC); TC_KCHECK(h);
     // output-layer bias gradients = column sums of the seeds (per-block partials from the loss kernel)
     tc_reduce_cols_kernel<<<tc_nblk(g.A + 1, 8), 256, 0, s>>>(P.colb3, P.blocks_done, (size_t)(g.A + 1), g.A + 1, gr + g.ao.b3, g.A, gr + nA + g.co.b3); TC_KCHECK(h);
-    // actor: dw0 rows [A+Do, A+Do+T) are the per-t column sums of du = the gradient of the bt table
-    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR_FT, P.dw0a + (size_t)(g.A + g.Do) * g.H, gr));
-    TC_KCHECK(h);
-    unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(P.dw0a, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
-    // critic: obs rows of dw0 -> dW_in; the ones column of h0 collected the input-layer bias gradient
-    unpack_dw0_kernel<<<tc_nblk((size_t)g.Do * g.Hc, 256), 256, 0, s>>>(P.dw0c + (size_t)g.A * g.Hc, 0, 0, g.Do, g.Hc, gr + nA + g.co.win); TC_KCHECK(h);
-    CUDA_TRY(cudaMemcpyAsync(gr + nA + g.co.bin, P.dw0c + (size_t)(g.A + g.Do + g.T) * g.Hc, g.Hc * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    return 0;
+    return tc_scatter_dw0(h, s, DPPO_NET_ACTOR_FT, P.dw0a, P.dw0c, gr);
 }
 static int tc_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const float* prev, const float* nxt, const int32_t* inds,
                        const float* returns, const float* oldvalues, const float* advantages, const float* oldlogp,
@@ -1259,8 +1211,7 @@ static int tc_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
 
 // the same update with the minibatch given as flat (rollout row, denoising index) indices into the resident rollout buffers
 static bool tc_ppo_indexed_ok(const dppo_handle* h, const TcIdxView& v) {
-    return (h->g.A % 4 == 0) && h->g.A <= 32 && ((((uintptr_t)v.chains | (uintptr_t)v.olp) & 15) == 0) && !h->deterministic &&
-           fc_ok(h) && fc_critic_ok(h);
+    return loss8_ok(h->g.A, 32, v.chains, v.olp) && !h->deterministic && fc_ok(h) && fc_critic_ok(h);
 }
 static int tc_ppo_step_indexed(dppo_handle* h, cudaStream_t s, const TcIdxView& view, int N, int64_t N_global, float adv_mean, float adv_std) {
     DPPO_TRY(tc_ppo_begin(h, s, N, 0, N_global));

@@ -1153,30 +1153,6 @@ __global__ void ts_pad64_kernel(const float* __restrict__ src, int N, int ncols,
     *reinterpret_cast<uint4*>(hi + (size_t)r * ld + k0) = *reinterpret_cast<const uint4*>(oh);
     *reinterpret_cast<uint4*>(lo + (size_t)r * ld + k0) = *reinterpret_cast<const uint4*>(ol);
 }
-// column sums of a two-plane matrix [N][ncols] (ncols even, ncols/2 <= 256): part[blk][ncols]
-__global__ void __launch_bounds__(256) ts_colsum_kernel(const bf16* __restrict__ Dh, const bf16* __restrict__ Dl, int N, int ncols, int rows_per_block,
-                                                        float* __restrict__ part) {
-    __shared__ float2 red[256];
-    const int tpr = ncols / 2, groups = 256 / tpr;
-    const int cg = threadIdx.x % tpr, rg = threadIdx.x / tpr;
-    const int r0 = blockIdx.x * rows_per_block, r1 = min(N, r0 + rows_per_block);
-    float2 acc = make_float2(0.f, 0.f);
-    if (rg < groups) {
-        for (int r = r0 + rg; r < r1; r += groups) {
-            const float2 fh = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(Dh + (size_t)r * ncols + 2 * cg));
-            const float2 fl = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(Dl + (size_t)r * ncols + 2 * cg));
-            acc.x += fh.x + fl.x; acc.y += fh.y + fl.y;
-        }
-    }
-    red[threadIdx.x] = acc;
-    __syncthreads();
-    if (threadIdx.x < tpr) {
-        float2 sacc = red[threadIdx.x];
-        for (int g = 1; g < groups; ++g) { const float2 o = red[g * tpr + threadIdx.x]; sacc.x += o.x; sacc.y += o.y; }
-        part[(size_t)blockIdx.x * ncols + 2 * threadIdx.x] = sacc.x;
-        part[(size_t)blockIdx.x * ncols + 2 * threadIdx.x + 1] = sacc.y;
-    }
-}
 
 // the folded output layer (W2 W3, b2 W3 + b3; ActorDerived::w23 / b23) is rebuilt lazily: only forward-only programs read it, updates come in runs
 static int ensure_w23(dppo_handle* h, int net, cudaStream_t s) {
@@ -1518,7 +1494,6 @@ static ts::Operand ts_op(const bf16* const* p, size_t off, bool mn_major, int64_
     return o;
 }
 static ts::Operand tsK(const SplitT& t, int64_t mn, int64_t k, int64_t ld) { return ts_op(t.p, 0, false, mn, k, ld); }
-static ts::Operand tsMN(const SplitT& t, int64_t mn, int64_t k, int64_t ld) { return ts_op(t.p, 0, true, mn, k, ld); }
 static ts::Operand tswK(const TsW& w, size_t off, int64_t mn, int64_t k, int64_t ld) { return ts_op(w.p, off, false, mn, k, ld); }
 static ts::Operand tswMN(const TsW& w, size_t off, int64_t mn, int64_t k, int64_t ld) { return ts_op(w.p, off, true, mn, k, ld); }
 static ts::Gemm ts_gemm_of(ts::Operand A, ts::Operand B, int M, int N, int planes, int dual = 0) {
@@ -1569,28 +1544,6 @@ static int ts_mlp_forward(dppo_handle* h, cudaStream_t s, const TsMlp& m, int N,
     o.alg_flops = 2.0 * N * ((double)H * H + (double)H * m.NO);        // the algorithmic work it stands for
     if (m.fold_ev) CUDA_TRY(cudaStreamWaitEvent(s, m.fold_ev, 0));
     DPPO_TRY(ts_run(h, s, o));
-    return 0;
-}
-// dW[out_rows][out_cols] = X^T D (+ X^T D2)  (X [rows][M], D [rows][Nd], two planes each), split-K over the rows with a FIXED-order reduction
-static int ts_dw(dppo_handle* h, cudaStream_t s, const SplitT& X, int M, const SplitT& D, int Nd, int rows, float* part, float* out, int out_rows, int out_cols,
-                 int ld_out, int alg_rows, const SplitT* D2 = nullptr) {
-    ts::Gemm g = ts_gemm_of(tsMN(X, M, rows, M), tsMN(D, Nd, rows, Nd), M, Nd, 2);
-    if (D2) { g.A2 = g.A; g.B2 = tsMN(*D2, Nd, rows, Nd); }
-    g.splits = tc_splits_for(h, M, Nd, rows);
-    g.alg_flops = 2.0 * (double)rows * (double)alg_rows * (double)out_cols;
-    g.epi.out_f32 = part; g.epi.ld_f32 = Nd; g.epi.split_stride = (size_t)M * Nd;
-    const int S = ts::launch(h, s, g);
-    if (S < 0) return S;
-    tc_reduce2d_kernel<<<tc_nblk((size_t)out_rows * out_cols, 256), 256, 0, s>>>(part, S, (size_t)M * Nd, out_rows, out_cols, Nd, out, ld_out);
-    TC_KCHECK(h);
-    return 0;
-}
-static int ts_colsum(dppo_handle* h, cudaStream_t s, const SplitT& D, int N, int ncols, float* part, float* out) {
-    int nb = 2 * h->sm_count; if (nb > (N + 63) / 64) nb = (N + 63) / 64; if (nb < 1) nb = 1;
-    int rpb = (N + nb - 1) / nb; nb = (N + rpb - 1) / rpb;
-    if (ncols / 2 > 256 || (ncols & 1)) DPPO_FAIL(-7, "ts_colsum: %d columns unsupported", ncols);
-    ts_colsum_kernel<<<nb, 256, 0, s>>>(D.p[0], D.p[1], N, ncols, rpb, part); TC_KCHECK(h);
-    tc_reduce_cols_kernel<<<tc_nblk(ncols, 8), 256, 0, s>>>(part, nb, (size_t)ncols, ncols, out); TC_KCHECK(h);
     return 0;
 }
 // backward chain of the residual MLP from dout [N][NOP] (two planes, zero padded): dh1 = (dout (W2 W3)^T) . act'(h1),
@@ -1944,7 +1897,7 @@ static int ts_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, flo
 // h0 pack | folded output layers + adv-stats (second stream) | 3 + 3 forward | loss | 3 + 3 backward | grouped dW + reduce | tail || dW3 assembly.
 // shapes / alignment the index-driven variant needs (float4 row reads of the resident rollout buffers)
 static bool ts_ppo_indexed_ok(const dppo_handle* h, const TcIdxView& v) {
-    return (h->g.A % 4 == 0) && h->g.A <= 128 && ((((uintptr_t)v.chains | (uintptr_t)v.olp) & 15) == 0);
+    return loss8_ok(h->g.A, 128, v.chains, v.olp);
 }
 // idx (optional): the minibatch is given as flat (rollout row, denoising index) indices into the resident rollout buffers; the h0 pack,
 // the advantage statistics and the loss kernel address those buffers directly (no gathered copy), the row pointers are unused
@@ -1955,8 +1908,7 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     const size_t nA = g.ao.n, nC = g.co.n;
     float* gr = h->grads;
     const bool amish = h->cfg.actor_act == DPPO_ACT_MISH, cmish = h->cfg.critic_act == DPPO_ACT_MISH;
-    // float4 row reads (the indexed program is only taken when ts_ppo_indexed_ok holds)
-    const bool loss8 = (g.A % 4 == 0) && g.A <= 128 && (idx || ((((uintptr_t)prev | (uintptr_t)nxt | (uintptr_t)oldlogp) & 15) == 0));
+    const bool loss8 = idx ? loss8_ok(g.A, 128, idx->chains, idx->olp) : loss8_ok(g.A, 128, prev, nxt, oldlogp);
     const int NOP = ts_nop(g.A);                                  // the actor's seed width: 64 (A <= 32) or 128
     const bool wide = NOP > 64;                                   // the loss kernel takes a warp per row (tc_ppo_loss8_kernel<32>)
     const int NOg = g.A > 32 ? g.A : 32;                          // columns of the a1^T dout / h0^T dout scratch
@@ -1990,14 +1942,7 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     // (not while the per-kernel profile is on: its event brackets are meant to time each kernel running alone)
     const bool side = !h->prof_on;
     cudaStream_t sc = s;
-    if (side) {
-        if (!h->aux_stream) {
-            CUDA_TRY(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-            for (int i = 0; i < 2; ++i) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[i], cudaEventDisableTiming));
-        }
-        if (!h->aux_ev[2]) CUDA_TRY(cudaEventCreateWithFlags(&h->aux_ev[2], cudaEventDisableTiming));
-        sc = h->aux_stream;
-    }
+    if (side) { DPPO_TRY(ensure_aux_stream(h)); sc = h->aux_stream; }
     auto fork = [&]() -> int { if (side) { CUDA_TRY(cudaEventRecord(h->aux_ev[0], s)); CUDA_TRY(cudaStreamWaitEvent(sc, h->aux_ev[0], 0)); } return 0; };
     auto join = [&]() -> int { if (side) { CUDA_TRY(cudaEventRecord(h->aux_ev[1], sc)); CUDA_TRY(cudaStreamWaitEvent(s, h->aux_ev[1], 0)); } return 0; };
     // h0 straight from (prev, obs, K-1-inds): tconst = -(K) flags "t = K-1-trow[r]"; the critic reads the same tile (its x / one-hot rows of W0 are zero)
@@ -2019,21 +1964,11 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     // the folded output layers of the current weights (stale after every AdamW step): on the second stream, under the actor's L0 / L1
     DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR_FT, sc)); DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, sc));
     if (side) { CUDA_TRY(cudaEventRecord(h->aux_ev[2], sc)); ma.fold_ev = h->aux_ev[2]; }      // the actor's stream waits in front of its folded GEMM only
-    if (adv_std < 0.f) {
-        if (idx) adv_stats_kernel<<<1, 1024, 0, sc>>>(idx->adv, N, h->scalars, idx->flat, idx->K, idx->P);
-        else adv_stats_kernel<<<1, 1024, 0, sc>>>(advantages, N, h->scalars);
-        TC_KCHECK(h);
-    }
-    else { set_scalars_kernel<<<1, 1, 0, sc>>>(h->scalars, adv_mean, adv_std); TC_KCHECK(h); }
+    DPPO_TRY(launch_adv_stats(h, sc, advantages, idx, N, adv_mean, adv_std));
     DPPO_TRY(ts_mlp_forward(h, s, ma, N, side ? 2 : 0));
     DPPO_TRY(ts_mlp_forward(h, sc, mc, N));
     DPPO_TRY(join());
-    PpoHyper hp;
-    hp.A = g.A; hp.Da = h->cfg.action_dim; hp.K = g.K; hp.T = g.T; hp.reward_horizon = h->cfg.reward_horizon; hp.norm_adv = h->cfg.norm_adv;
-    hp.dcv = h->cfg.denoised_clip_value; hp.min_lp_std = h->cfg.min_logprob_denoising_std;
-    hp.lp_lo = h->cfg.logprob_clip_lo; hp.lp_hi = h->cfg.logprob_clip_hi; hp.gamma_d = h->cfg.gamma_denoising;
-    hp.clip_coef = h->cfg.clip_ploss_coef; hp.clip_base = h->cfg.clip_ploss_coef_base; hp.clip_rate = h->cfg.clip_ploss_coef_rate;
-    hp.clip_v = h->cfg.clip_vloss_coef; hp.vf_coef = h->cfg.vf_coef; hp.inv_nglobal = 1.0f / (float)N_global;
+    const PpoHyper hp = ppo_hyper(h, N_global);
     const float frac_local = (float)((double)N / (double)N_global);
     if (loss8) {
         // loss, metric partial sums, the two-plane padded gradient seeds and the output-bias column partials in one pass
@@ -2076,11 +2011,7 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     DPPO_TRY(colsum(h, s, dval, 1, N, 1, nullptr, 1, part, gr + nA + g.co.b3));
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, b2scr, g.H, gr + g.ao.b1); TC_KCHECK(h);
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.Hc, 8), 256, 0, s>>>(cpc, nrb, (size_t)2 * g.Hc, 2 * g.Hc, b2scr + g.H, g.Hc, gr + nA + g.co.b1); TC_KCHECK(h);
-    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR_FT, dw0a + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
-    unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0a, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
-    unpack_dw0_kernel<<<tc_nblk((size_t)g.Do * g.Hc, 256), 256, 0, s>>>(dw0c + (size_t)g.A * g.Hc, 0, 0, g.Do, g.Hc, gr + nA + g.co.win); TC_KCHECK(h);
-    CUDA_TRY(cudaMemcpyAsync(gr + nA + g.co.bin, dw0c + (size_t)(g.A + g.Do + g.T) * g.Hc, g.Hc * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    return 0;
+    return tc_scatter_dw0(h, s, DPPO_NET_ACTOR_FT, dw0a, dw0c, gr);
 }
 
 // DiffusionModel.c_loss / p_losses (diffusion.py:179-202) + tape.gradient: loss -> h->grads[nA], gradients -> h->grads[0 : nA]
@@ -2124,7 +2055,5 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     DPPO_TRY(ts_dw3_assemble(h, s, DPPO_NET_ACTOR, ga1, ga0, gr, dw0, nullptr, nullptr, nullptr, nullptr));
     tc_reduce_cols_kernel<<<tc_nblk(2 * g.H, 8), 256, 0, s>>>(cpa, nrb, (size_t)2 * g.H, 2 * g.H, ga1 + (size_t)(g.H + KP0) * NOg, g.H, gr + g.ao.b1); TC_KCHECK(h);
     DPPO_TRY(colsum(h, s, deps, g.A, N, g.A, nullptr, 1, part, gr + g.ao.b3));
-    CUDA_TRY(launch_time_backward(h, s, DPPO_NET_ACTOR, dw0 + (size_t)(g.A + g.Do) * g.H, gr)); TC_KCHECK(h);
-    unpack_dw0_kernel<<<tc_nblk((size_t)(g.A + g.Do) * g.H, 256), 256, 0, s>>>(dw0, g.A, g.td, g.Do, g.H, gr + g.ao.win); TC_KCHECK(h);
-    return 0;
+    return tc_scatter_dw0(h, s, DPPO_NET_ACTOR, dw0, nullptr, gr);
 }
