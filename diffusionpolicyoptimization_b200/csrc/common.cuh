@@ -154,8 +154,10 @@ struct ActorDerived {
 
 struct OptState { float* m; float* v; int64_t step; size_t n; };
 
+// A grow-only device buffer carved into 256-byte aligned slices by ws_take; ws_layout sizes it.  peak: the most bytes taken
+// since the layout began (a nested program gives its slices back, see ws_room).
 struct Workspace {
-    char* base = nullptr; size_t cap = 0, used = 0;
+    char* base = nullptr; size_t cap = 0, used = 0, peak = 0;
 };
 
 struct dppo_handle {
@@ -171,9 +173,7 @@ struct dppo_handle {
     float* grads;         // [nA + nC + 16]
     float* scalars;       // device scratch: [0..1] adv mean/std, [8..] metric sums
     Workspace ws;
-    // pinned + device staging for *_host calls
-    char* pin = nullptr; size_t pin_cap = 0;
-    char* dstage = nullptr; size_t dstage_cap = 0;
+    Workspace stage;      // device copies of the host arrays of the *_host calls
     cudaStream_t copy_stream = nullptr; cudaEvent_t copy_ev[9];   // chunked H2D / compute overlap of dppo_ppo_step_host
     // NCCL
     void* comm = nullptr; int rank = 0, world = 1;
@@ -212,14 +212,44 @@ struct dppo_handle {
     double prof_exec[4] = {0, 0, 0, 0};   // flops the tensor pipe executed (plane modes issue 3 or 6 products per algorithmic multiply-add)
 };
 
-int ws_reserve(dppo_handle* h, size_t bytes, cudaStream_t s);
 // profile bracket: call prof_begin before and prof_end after a GEMM-class launch
 void prof_begin(dppo_handle* h, cudaStream_t s);
 void prof_end(dppo_handle* h, cudaStream_t s, double flops, int cls, double exec_flops = -1.0);   // exec_flops: tensor-pipe flops actually issued (default: = flops)
-template <typename T> static inline T* ws_take(dppo_handle* h, size_t count) {
-    size_t bytes = (count * sizeof(T) + 255) / 256 * 256;
-    T* p = (T*)(h->ws.base + h->ws.used);
-    h->ws.used += bytes;
+
+// ------------------------------------------------------------------ workspace layout
+// A program describes its buffers once, as a layout: a function that only takes slices (ws_take) and computes pointers from them.
+// It launches nothing and reads nothing from the device.  ws_layout runs it twice: a counting pass whose high-water mark sizes
+// the buffer, then the pass whose pointers the program uses.
+template <typename T> static inline T* ws_take(Workspace& w, size_t count) {
+    T* p = (T*)((uintptr_t)w.base + w.used);      // not dereferenced during the counting pass, where base may be stale
+    w.used += (count * sizeof(T) + 255) / 256 * 256;
+    if (w.used > w.peak) w.peak = w.used;
     return p;
 }
-static inline size_t ws_bytes(size_t count, size_t elt) { return (count * elt + 255) / 256 * 256; }
+template <typename T> static inline T* ws_take(dppo_handle* h, size_t count) { return ws_take<T>(h->ws, count); }
+int ws_reserve(Workspace& w, size_t bytes, cudaStream_t s);   // grow-only; only ws_layout calls it
+static inline int ws_check(const Workspace& w) {
+    if (w.peak > w.cap) DPPO_FAIL(-7, "workspace layout takes %zu bytes, %zu reserved", w.peak, w.cap);
+    return 0;
+}
+template <typename F> static int ws_layout(Workspace& w, cudaStream_t s, F&& layout) {
+    w.used = w.peak = 0;
+    layout();
+    DPPO_TRY(ws_reserve(w, w.peak, s));
+    w.used = w.peak = 0;
+    layout();
+    return ws_check(w);
+}
+// A nested program (tc_actor_forward, ts_actor_forward) appends its slices above the caller's at call time and gives them back when
+// it returns; the caller holds pointers below w.used, so the buffer must not grow then.  The caller's layout makes room for it
+// with ws_room (the nested layout counts towards peak, nothing stays taken); the nested program takes its slices with ws_append.
+template <typename F> static void ws_room(Workspace& w, F&& layout) {
+    const size_t mark = w.used;
+    layout();
+    w.used = mark;
+}
+template <typename F> static int ws_append(Workspace& w, F&& layout) {
+    w.peak = w.used;
+    layout();
+    return ws_check(w);
+}

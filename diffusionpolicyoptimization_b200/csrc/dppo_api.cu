@@ -112,13 +112,13 @@ extern "C" size_t dppo_num_params(const dppo_cfg* cfg, int net) {
 }
 
 // ------------------------------------------------------------------ workspace
-int ws_reserve(dppo_handle* h, size_t bytes, cudaStream_t s) {
-    h->ws.used = 0;
-    if (bytes <= h->ws.cap) return 0;
-    if (h->ws.base) { CUDA_TRY(cudaStreamSynchronize(s)); CUDA_TRY(cudaDeviceSynchronize()); CUDA_TRY(cudaFree(h->ws.base)); h->ws.base = nullptr; h->ws.cap = 0; }
+// the old buffer may still be in use by queued work: synchronise before freeing it
+int ws_reserve(Workspace& w, size_t bytes, cudaStream_t s) {
+    if (bytes <= w.cap) return 0;
+    if (w.base) { CUDA_TRY(cudaStreamSynchronize(s)); CUDA_TRY(cudaDeviceSynchronize()); CUDA_TRY(cudaFree(w.base)); w.base = nullptr; w.cap = 0; }
     size_t cap = bytes + (bytes >> 3) + (1 << 20);
-    CUDA_TRY(cudaMalloc(&h->ws.base, cap));
-    h->ws.cap = cap;
+    CUDA_TRY(cudaMalloc(&w.base, cap));
+    w.cap = cap;
     return 0;
 }
 
@@ -331,8 +331,7 @@ extern "C" void dppo_destroy(dppo_handle* h) {
     if (h->ws.base) cudaFree(h->ws.base);
     if (h->copy_stream) { cudaStreamDestroy(h->copy_stream); for (int i = 0; i < 9; ++i) cudaEventDestroy(h->copy_ev[i]); }
     if (h->aux_stream) { cudaStreamDestroy(h->aux_stream); for (int i = 0; i < 3; ++i) if (h->aux_ev[i]) cudaEventDestroy(h->aux_ev[i]); }
-    if (h->pin) cudaFreeHost(h->pin);
-    if (h->dstage) cudaFree(h->dstage);
+    if (h->stage.base) cudaFree(h->stage.base);
     delete h;
 }
 
@@ -394,9 +393,6 @@ extern "C" int dppo_last_path(dppo_handle* h) { return h ? h->last_path : -1; }
 // ------------------------------------------------------------------ fp32 layer-by-layer forward
 struct FwdBufs { float *h0p, *u, *h1, *v, *out; };
 
-static size_t fwd_ws_bytes(int N, int KP, int H, int NO) {
-    return ws_bytes((size_t)N * KP, 4) + 3 * ws_bytes((size_t)N * H, 4) + ws_bytes((size_t)N * NO, 4);
-}
 static void fwd_take(dppo_handle* h, int N, int KP, int H, int NO, FwdBufs& b) {
     b.h0p = ws_take<float>(h, (size_t)N * KP);
     b.u = ws_take<float>(h, (size_t)N * H); b.h1 = ws_take<float>(h, (size_t)N * H); b.v = ws_take<float>(h, (size_t)N * H);
@@ -438,12 +434,6 @@ static int critic_fwd_fp32(dppo_handle* h, cudaStream_t s, const float* obs, int
 
 // ------------------------------------------------------------------ fp32 backward (shared by actor / critic)
 struct BwdBufs { float *dv, *dh1, *du, *part; size_t part_floats; };
-static size_t bwd_ws_bytes(const dppo_handle* h, int N, int KP, int H, int NO, int nseg) {
-    size_t colpart = (size_t)320 * (size_t)nseg * H;             // colsum partials
-    size_t gemm_part = (size_t)40 * (size_t)H * H;               // split-K partials
-    size_t pf = colpart > gemm_part ? colpart : gemm_part;
-    return 3 * ws_bytes((size_t)N * H, 4) + ws_bytes(pf, 4) + ws_bytes((size_t)nseg * H, 4) + ws_bytes((size_t)KP * H, 4);
-}
 static int colsum(dppo_handle* h, cudaStream_t s, const float* D, int ld, int N, int ncols, const int* seg, int nseg,
                   float* part, float* out) {
     int nb = (N + 127) / 128; if (nb > 320) nb = 320; if (nb < 1) nb = 1;
@@ -500,7 +490,7 @@ static int mlp_bwd_fp32(dppo_handle* h, cudaStream_t s, const float* w, size_t o
 }
 static void bwd_take(dppo_handle* h, int N, int KP, int H, int nseg, BwdBufs& b, float** Gseg, float** dw0p) {
     b.dv = ws_take<float>(h, (size_t)N * H); b.dh1 = ws_take<float>(h, (size_t)N * H); b.du = ws_take<float>(h, (size_t)N * H);
-    size_t colpart = (size_t)320 * (size_t)nseg * H, gemm_part = (size_t)40 * (size_t)H * H;
+    size_t colpart = (size_t)320 * (size_t)nseg * H, gemm_part = (size_t)40 * (size_t)H * H;   // colsum / split-K partials
     b.part_floats = colpart > gemm_part ? colpart : gemm_part;
     b.part = ws_take<float>(h, b.part_floats);
     *Gseg = ws_take<float>(h, (size_t)nseg * H);
@@ -528,24 +518,29 @@ static int critic_bwd_fp32(dppo_handle* h, cudaStream_t s, const FwdBufs& f, con
 // ------------------------------------------------------------------ forward-only entry points
 static const int ROW_CHUNK = 1 << 18;
 
+// room for the N-row actor forward of a tensor mode, which appends its buffers at call time (ts_actor_forward when split, else tc_actor_forward)
+static void tensor_forward_room(dppo_handle* h, bool split, int N) {
+    ws_room(h->ws, [&] {
+        if (split) { TsMlp m; ts_actor_forward_take(h, DPPO_NET_ACTOR, N, m); }
+        else { TcMlp m; tc_actor_forward_take(h, DPPO_NET_ACTOR, N, m); }
+    });
+}
+
 extern "C" int dppo_actor_forward(dppo_handle* h, int net, const float* x, const int32_t* t, const float* obs,
                                   int N, float* eps, dppo_stream_t st) {
     ENTER(h); cudaStream_t s = (cudaStream_t)st; const Geom& g = h->g;
     if (net < 0 || net > 3 || net == DPPO_NET_CRITIC || !x || !t || !obs || !eps || N < 0) DPPO_FAIL(-1, "dppo_actor_forward: bad arguments");
     for (int r0 = 0; r0 < N; r0 += ROW_CHUNK) {
         int n = N - r0 < ROW_CHUNK ? N - r0 : ROW_CHUNK;
-        if (tc_eligible(h, n)) {
-            DPPO_TRY(ws_reserve(h, tc_actor_forward_ws(h, n), s));
-            DPPO_TRY(tc_actor_forward(h, s, net, x + (size_t)r0 * g.A, obs + (size_t)r0 * g.Do, 1, n, t + r0, 0, eps + (size_t)r0 * g.A));
+        const bool split = ts_eligible(h, n);
+        if (tc_eligible(h, n) || split) {
+            DPPO_TRY(ws_layout(h->ws, s, [&] { tensor_forward_room(h, split, n); }));
+            if (split) DPPO_TRY(ts_actor_forward(h, s, net, x + (size_t)r0 * g.A, obs + (size_t)r0 * g.Do, 1, n, t + r0, 0, eps + (size_t)r0 * g.A));
+            else DPPO_TRY(tc_actor_forward(h, s, net, x + (size_t)r0 * g.A, obs + (size_t)r0 * g.Do, 1, n, t + r0, 0, eps + (size_t)r0 * g.A));
             continue;
         }
-        if (ts_eligible(h, n)) {
-            DPPO_TRY(ws_reserve(h, ts_actor_forward_ws(h, n), s));
-            DPPO_TRY(ts_actor_forward(h, s, net, x + (size_t)r0 * g.A, obs + (size_t)r0 * g.Do, 1, n, t + r0, 0, eps + (size_t)r0 * g.A));
-            continue;
-        }
-        DPPO_TRY(ws_reserve(h, fwd_ws_bytes(n, g.KP, g.H, g.A), s));
-        FwdBufs b; fwd_take(h, n, g.KP, g.H, g.A, b);
+        FwdBufs b;
+        DPPO_TRY(ws_layout(h->ws, s, [&] { fwd_take(h, n, g.KP, g.H, g.A, b); }));
         DPPO_TRY(actor_fwd_fp32(h, s, net, x + (size_t)r0 * g.A, obs + (size_t)r0 * g.Do, 1, n, t + r0, 0, b));
         CUDA_TRY(cudaMemcpyAsync(eps + (size_t)r0 * g.A, b.out, (size_t)n * g.A * sizeof(float), cudaMemcpyDeviceToDevice, s));
     }
@@ -558,8 +553,8 @@ extern "C" int dppo_value(dppo_handle* h, const float* obs, int N, float* v, dpp
         int n = N - r0 < ROW_CHUNK ? N - r0 : ROW_CHUNK;
         if (tc_eligible(h, n)) { DPPO_TRY(tc_value(h, s, obs + (size_t)r0 * g.Do, n, v + r0)); continue; }
         if (ts_eligible(h, n)) { DPPO_TRY(ts_value(h, s, obs + (size_t)r0 * g.Do, n, v + r0)); continue; }
-        DPPO_TRY(ws_reserve(h, fwd_ws_bytes(n, g.KPc, g.Hc, 1), s));
-        FwdBufs b; fwd_take(h, n, g.KPc, g.Hc, 1, b);
+        FwdBufs b;
+        DPPO_TRY(ws_layout(h->ws, s, [&] { fwd_take(h, n, g.KPc, g.Hc, 1, b); }));
         DPPO_TRY(critic_fwd_fp32(h, s, obs + (size_t)r0 * g.Do, n, b));
         CUDA_TRY(cudaMemcpyAsync(v + r0, b.out, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, s));
     }
@@ -578,13 +573,15 @@ static int logprobs_impl(dppo_handle* h, cudaStream_t s, const float* obs, const
         const bool split = ts_eligible(h, n);
         const bool tensor = tc_eligible(h, n) || split;
         const bool fusedlp = tensor && !split && fc_ok(h);
-        size_t need = (tensor ? ws_bytes((size_t)n * g.A, 4) + (split ? ts_actor_forward_ws(h, n) : tc_actor_forward_ws(h, n)) : fwd_ws_bytes(n, g.KP, g.H, g.A))
-                    + ws_bytes(n, 4) + ws_bytes((size_t)n * g.A, 4);
-        DPPO_TRY(ws_reserve(h, need, s));
         FwdBufs b; memset(&b, 0, sizeof(b));
-        if (tensor) b.out = ws_take<float>(h, (size_t)n * g.A); else fwd_take(h, n, g.KP, g.H, g.A, b);
-        int* trow = ws_take<int>(h, n);
-        float* pv = ws_take<float>(h, (size_t)n * g.A);
+        int* trow; float* pv; bf16* h0 = nullptr;
+        DPPO_TRY(ws_layout(h->ws, s, [&] {
+            if (tensor) b.out = ws_take<float>(h, (size_t)n * g.A); else fwd_take(h, n, g.KP, g.H, g.A, b);
+            trow = ws_take<int>(h, n);
+            pv = ws_take<float>(h, (size_t)n * g.A);
+            if (fusedlp) h0 = ws_take<bf16>(h, (size_t)n * h->tc->KP0);
+            else if (tensor) tensor_forward_room(h, split, n);
+        }));
         const float* xin; const float* ob; int obs_div;
         const float* ch = nullptr;
         if (chains) {
@@ -599,7 +596,6 @@ static int logprobs_impl(dppo_handle* h, cudaStream_t s, const float* obs, const
         const float* epsp;
         if (fusedlp) {
             // pack h0 straight from prev rows / the chains tensor, then forward + Gaussian log-prob in one fused launch
-            bf16* h0 = ws_take<bf16>(h, (size_t)n * h->tc->KP0);
             tc_pack_h0_kernel<<<nblk((size_t)n * (h->tc->KP0 / 8), 256), 256, 0, s>>>(chains ? ch : prev + (size_t)r0 * g.A, ob, trow, 0, n, g.A, g.Do, g.T,
                                                                                       h->tc->KP0, obs_div, h0, chains ? g.K : 0);
             KLAUNCH(h); KCHECK();
@@ -675,11 +671,13 @@ static int sample_layered_fp32(dppo_handle* h, cudaStream_t s, const float* obs,
                                float* actions, float* chains, bool tensor) {
     const Geom& g = h->g;
     const bool split = tensor && ts_eligible(h, B);
-    size_t need = (tensor ? ws_bytes((size_t)B * g.A, 4) + (split ? ts_actor_forward_ws(h, B) : tc_actor_forward_ws(h, B)) : fwd_ws_bytes(B, g.KP, g.H, g.A)) + ws_bytes((size_t)B * g.A, 4);
-    DPPO_TRY(ws_reserve(h, need, s));
     FwdBufs b; memset(&b, 0, sizeof(b));
-    if (tensor) b.out = ws_take<float>(h, (size_t)B * g.A); else fwd_take(h, B, g.KP, g.H, g.A, b);
-    float* x = ws_take<float>(h, (size_t)B * g.A);
+    float* x;
+    DPPO_TRY(ws_layout(h->ws, s, [&] {
+        if (tensor) b.out = ws_take<float>(h, (size_t)B * g.A); else fwd_take(h, B, g.KP, g.H, g.A, b);
+        x = ws_take<float>(h, (size_t)B * g.A);
+        if (tensor) tensor_forward_room(h, split, B);
+    }));
     sample_init_kernel<<<nblk((size_t)B * g.A, 256), 256, 0, s>>>(x, xT, B, g.A, seed, offset, row_offset, chains, g.K, g.K == g.T);
     KLAUNCH(h); KCHECK();
     for (int i = 0; i < g.T; ++i) {
@@ -798,31 +796,20 @@ static int sample_impl(dppo_handle* h, const float* obs, int B, int deterministi
     return env_tail();
 }
 
-static int stage_reserve(dppo_handle* h, size_t bytes) {
-    if (bytes <= h->dstage_cap) return 0;
-    if (h->dstage) { CUDA_TRY(cudaDeviceSynchronize()); CUDA_TRY(cudaFree(h->dstage)); h->dstage = nullptr; h->dstage_cap = 0; }
-    size_t cap = bytes + (bytes >> 2) + 4096;
-    CUDA_TRY(cudaMalloc(&h->dstage, cap));
-    h->dstage_cap = cap;
-    return 0;
-}
-static inline size_t a256(size_t b) { return (b + 255) / 256 * 256; }
-
 extern "C" int dppo_sample_host(dppo_handle* h, const float* obs, int B, int deterministic, int use_base_policy,
                                 float min_sampling_std, uint64_t seed, uint64_t offset, int64_t row_offset,
                                 const float* xT, const float* noise, float* actions, float* chains, dppo_stream_t st) {
     ENTER(h); cudaStream_t s = (cudaStream_t)st; const Geom& g = h->g;
     if (!obs || !actions || B < 0) DPPO_FAIL(-1, "dppo_sample_host: bad arguments");
     if (B == 0) return 0;
-    size_t b_obs = a256((size_t)B * g.Do * 4), b_x = a256((size_t)B * g.A * 4), b_nz = a256((size_t)g.T * B * g.A * 4);
-    size_t b_ch = a256((size_t)B * (g.K + 1) * g.A * 4);
-    DPPO_TRY(stage_reserve(h, b_obs + 2 * b_x + b_nz + b_ch));
-    char* p = h->dstage;
-    float* d_obs = (float*)p; p += b_obs;
-    float* d_xT = (float*)p; p += b_x;
-    float* d_act = (float*)p; p += b_x;
-    float* d_nz = (float*)p; p += b_nz;
-    float* d_ch = (float*)p;
+    float *d_obs, *d_xT, *d_act, *d_nz, *d_ch;
+    DPPO_TRY(ws_layout(h->stage, s, [&] {
+        Workspace& w = h->stage;
+        d_obs = ws_take<float>(w, (size_t)B * g.Do);
+        d_xT = ws_take<float>(w, (size_t)B * g.A); d_act = ws_take<float>(w, (size_t)B * g.A);
+        d_nz = ws_take<float>(w, (size_t)g.T * B * g.A);
+        d_ch = ws_take<float>(w, (size_t)B * (g.K + 1) * g.A);
+    }));
     CUDA_TRY(cudaMemcpyAsync(d_obs, obs, (size_t)B * g.Do * 4, cudaMemcpyHostToDevice, s));
     if (xT) CUDA_TRY(cudaMemcpyAsync(d_xT, xT, (size_t)B * g.A * 4, cudaMemcpyHostToDevice, s));
     if (noise) CUDA_TRY(cudaMemcpyAsync(d_nz, noise, (size_t)g.T * B * g.A * 4, cudaMemcpyHostToDevice, s));
@@ -1049,18 +1036,15 @@ extern "C" int dppo_ppo_step(dppo_handle* h, const float* obs, const float* prev
         DPPO_TRY(ts_ppo_step(h, s, obs, prev, nxt, inds, returns, oldvalues, advantages, oldlogp, N, N_global, adv_mean, adv_std));
     } else {
         const int nlb = nblk(N, 128);
-        size_t need = fwd_ws_bytes(N, g.KP, g.H, g.A) + fwd_ws_bytes(N, g.KPc, g.Hc, 1)
-                    + bwd_ws_bytes(h, N, g.KP, g.H, g.A, g.T) + bwd_ws_bytes(h, N, g.KPc, g.Hc, 1, 1)
-                    + ws_bytes(N, 4) + ws_bytes((size_t)N * g.A, 4) + ws_bytes(N, 4) + ws_bytes((size_t)nlb * 5, 8);
-        DPPO_TRY(ws_reserve(h, need, s));
-        FwdBufs fa, fc; fwd_take(h, N, g.KP, g.H, g.A, fa); fwd_take(h, N, g.KPc, g.Hc, 1, fc);
-        BwdBufs ba, bc; float *Ga, *Gc, *dw0a, *dw0c;
-        bwd_take(h, N, g.KP, g.H, g.T, ba, &Ga, &dw0a); bwd_take(h, N, g.KPc, g.Hc, 1, bc, &Gc, &dw0c);
-        int* trow = ws_take<int>(h, N);
-        float* deps = ws_take<float>(h, (size_t)N * g.A);
-        float* dval = ws_take<float>(h, N);
-        double* bsum = ws_take<double>(h, (size_t)nlb * 5);
-
+        FwdBufs fa, fc; BwdBufs ba, bc; float *Ga, *Gc, *dw0a, *dw0c, *deps, *dval; int* trow; double* bsum;
+        DPPO_TRY(ws_layout(h->ws, s, [&] {
+            fwd_take(h, N, g.KP, g.H, g.A, fa); fwd_take(h, N, g.KPc, g.Hc, 1, fc);
+            bwd_take(h, N, g.KP, g.H, g.T, ba, &Ga, &dw0a); bwd_take(h, N, g.KPc, g.Hc, 1, bc, &Gc, &dw0c);
+            trow = ws_take<int>(h, N);
+            deps = ws_take<float>(h, (size_t)N * g.A);
+            dval = ws_take<float>(h, N);
+            bsum = ws_take<double>(h, (size_t)nlb * 5);
+        }));
         make_trow_kernel<<<nblk(N, 256), 256, 0, s>>>(inds, N, g.K, 0, trow); KLAUNCH(h); KCHECK();
         DPPO_TRY(launch_adv_stats(h, s, advantages, nullptr, N, adv_mean, adv_std));
         DPPO_TRY(actor_fwd_fp32(h, s, DPPO_NET_ACTOR_FT, prev, obs, 1, N, trow, 0, fa));
@@ -1081,13 +1065,14 @@ extern "C" int dppo_ppo_step_host(dppo_handle* h, const float* obs, const float*
                                   float adv_mean, float adv_std, float lr, int apply, float* metrics8_host, dppo_stream_t st) {
     ENTER(h); cudaStream_t s = (cudaStream_t)st; const Geom& g = h->g;
     if (N < 1) DPPO_FAIL(-1, "dppo_ppo_step_host: bad arguments");
-    size_t b_obs = a256((size_t)N * g.Do * 4), b_x = a256((size_t)N * g.A * 4), b_n = a256((size_t)N * 4);
-    DPPO_TRY(stage_reserve(h, b_obs + 3 * b_x + 4 * b_n + 256));
-    char* p = h->dstage;
-    float* d_obs = (float*)p; p += b_obs;
-    float* d_prev = (float*)p; p += b_x; float* d_next = (float*)p; p += b_x; float* d_olp = (float*)p; p += b_x;
-    int* d_inds = (int*)p; p += b_n; float* d_ret = (float*)p; p += b_n; float* d_val = (float*)p; p += b_n; float* d_adv = (float*)p; p += b_n;
-    float* d_met = (float*)p;
+    float *d_obs, *d_prev, *d_next, *d_olp, *d_ret, *d_val, *d_adv, *d_met; int* d_inds;
+    DPPO_TRY(ws_layout(h->stage, s, [&] {
+        Workspace& w = h->stage;
+        d_obs = ws_take<float>(w, (size_t)N * g.Do);
+        d_prev = ws_take<float>(w, (size_t)N * g.A); d_next = ws_take<float>(w, (size_t)N * g.A); d_olp = ws_take<float>(w, (size_t)N * g.A);
+        d_inds = ws_take<int>(w, N); d_ret = ws_take<float>(w, N); d_val = ws_take<float>(w, N); d_adv = ws_take<float>(w, N);
+        d_met = ws_take<float>(w, 8);
+    }));
     // tensor mode: chunked pipeline - the H2D copy of chunk c+1 (copy stream) overlaps the compute of chunk c
     const int chunk_rows = (tc_eligible(h, N) && fc_ok(h) && fc_critic_ok(h) && !h->deterministic) ? tc_ppo_pipeline_chunk_rows(h, N) : 0;
     if (chunk_rows > 0) {
@@ -1159,14 +1144,15 @@ static int ppo_indexed_impl(dppo_handle* h, cudaStream_t s, const float* obs_buf
         DPPO_FAIL(-1, "dppo_ppo_step_indexed: bad arguments");
     if (g.K < 1) DPPO_FAIL(-1, "dppo_ppo_step_indexed: ft_denoising_steps must be >= 1");
     if (P * g.K > 2000000000LL) DPPO_FAIL(-1, "dppo_ppo_step_indexed: rollout buffer too large for int32 flat indices");
-    size_t b_obs = a256((size_t)N * g.Do * 4), b_x = a256((size_t)N * g.A * 4), b_n = a256((size_t)N * 4);
-    DPPO_TRY(stage_reserve(h, b_obs + 3 * b_x + 5 * b_n + 512));
-    char* p = h->dstage;
-    float* d_obs = (float*)p; p += b_obs;
-    float* d_prev = (float*)p; p += b_x; float* d_next = (float*)p; p += b_x; float* d_olp = (float*)p; p += b_x;
-    int* d_dind = (int*)p; p += b_n; float* d_ret = (float*)p; p += b_n; float* d_val = (float*)p; p += b_n; float* d_adv = (float*)p; p += b_n;
-    int* d_inds = (int*)p; p += b_n;
-    float* d_met = (float*)p; int* d_bad = (int*)(p + 256);
+    float *d_obs, *d_prev, *d_next, *d_olp, *d_ret, *d_val, *d_adv, *d_met; int *d_dind, *d_inds, *d_bad;
+    DPPO_TRY(ws_layout(h->stage, s, [&] {
+        Workspace& w = h->stage;
+        d_obs = ws_take<float>(w, (size_t)N * g.Do);
+        d_prev = ws_take<float>(w, (size_t)N * g.A); d_next = ws_take<float>(w, (size_t)N * g.A); d_olp = ws_take<float>(w, (size_t)N * g.A);
+        d_dind = ws_take<int>(w, N); d_ret = ws_take<float>(w, N); d_val = ws_take<float>(w, N); d_adv = ws_take<float>(w, N);
+        d_inds = ws_take<int>(w, N);
+        d_met = ws_take<float>(w, 8); d_bad = ws_take<int>(w, 1);
+    }));
     if (inds_host) { CUDA_TRY(cudaMemcpyAsync(d_inds, inds_host, (size_t)N * 4, cudaMemcpyHostToDevice, s)); inds_dev = d_inds; }
     CUDA_TRY(cudaMemsetAsync(d_bad, 0, sizeof(int), s));
     // tensor mode: no materialised minibatch - the h0 pack and loss kernels read the rollout buffers through the flat indices
@@ -1248,14 +1234,14 @@ extern "C" int dppo_pretrain_step(dppo_handle* h, const float* actions, const fl
     } else {
         const size_t ne = (size_t)N * g.A;
         const int nlb = nblk(ne, 256);
-        size_t need = fwd_ws_bytes(N, g.KP, g.H, g.A) + bwd_ws_bytes(h, N, g.KP, g.H, g.A, g.T)
-                    + ws_bytes(N, 4) + 3 * ws_bytes(ne, 4) + ws_bytes(nlb, 8);
-        DPPO_TRY(ws_reserve(h, need, s));
-        FwdBufs fa; fwd_take(h, N, g.KP, g.H, g.A, fa);
-        BwdBufs ba; float *Ga, *dw0a; bwd_take(h, N, g.KP, g.H, g.T, ba, &Ga, &dw0a);
-        int* trow = ws_take<int>(h, N);
-        float* noise = ws_take<float>(h, ne); float* xn = ws_take<float>(h, ne); float* deps = ws_take<float>(h, ne);
-        double* bsum = ws_take<double>(h, nlb);
+        FwdBufs fa; BwdBufs ba; float *Ga, *dw0a, *noise, *xn, *deps; int* trow; double* bsum;
+        DPPO_TRY(ws_layout(h->ws, s, [&] {
+            fwd_take(h, N, g.KP, g.H, g.A, fa);
+            bwd_take(h, N, g.KP, g.H, g.T, ba, &Ga, &dw0a);
+            trow = ws_take<int>(h, N);
+            noise = ws_take<float>(h, ne); xn = ws_take<float>(h, ne); deps = ws_take<float>(h, ne);
+            bsum = ws_take<double>(h, nlb);
+        }));
         pretrain_prep_kernel<<<nblk(ne, 256), 256, 0, s>>>(actions, t_in, noise_in, N, g.A, g.T, h->sched, seed, offset, row_offset, trow, noise, xn);
         KLAUNCH(h); KCHECK();
         DPPO_TRY(actor_fwd_fp32(h, s, DPPO_NET_ACTOR, xn, obs, 1, N, trow, 0, fa));

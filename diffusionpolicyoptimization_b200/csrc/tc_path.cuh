@@ -724,10 +724,6 @@ static TcMlp tc_mlp_at(const TcMlp& m, size_t r0) {
     if (o.m0) o.m0 += r0 * (size_t)(m.H / 32); if (o.m1) o.m1 += r0 * (size_t)(m.H / 32);
     return o;
 }
-static size_t tc_mlp_ws_bytes(int N, int H, bool mish, bool bwd) {
-    size_t one = ws_bytes((size_t)N * H, sizeof(bf16));
-    return one * (3 + (mish ? 2 : 0) + (bwd ? 3 : 0)) + 2 * ws_bytes((size_t)N * (H / 32), 4);
-}
 static void tc_mlp_take(dppo_handle* h, int N, TcMlp& m, bool bwd) {
     const size_t n = (size_t)N * m.H;
     m.a0 = ws_take<bf16>(h, n); m.a1 = ws_take<bf16>(h, n); m.v = ws_take<bf16>(h, n);
@@ -894,44 +890,33 @@ static void tc_critic_mlp(const dppo_handle* h, TcMlp& m) {
 }
 
 // ------------------------------------------------------------------ forward-only: eps[N][A] = actor(x, t, obs)
+// the buffers tc_actor_forward appends for N rows: h0, and the layer activations unless the fused chain runs the forward
+static bf16* tc_actor_forward_take(dppo_handle* h, int net, int N, TcMlp& m) {
+    tc_actor_mlp(h, net, m);
+    bf16* h0 = ws_take<bf16>(h, (size_t)N * h->tc->KP0);
+    if (!fc_ok(h)) tc_mlp_take(h, N, m, false);
+    m.h0 = h0;
+    return h0;
+}
 static int tc_actor_forward(dppo_handle* h, cudaStream_t s, int net, const float* x, const float* obs, int obs_div, int N,
                             const int* trow, int tconst, float* eps) {
     const Geom& g = h->g; const int KP0 = h->tc->KP0;
-    if (fc_ok(h)) {
-        const size_t need = h->ws.used + ws_bytes((size_t)N * KP0, 2);
-        if (need > h->ws.cap) DPPO_FAIL(-7, "tc_actor_forward: workspace too small (%zu > %zu)", need, h->ws.cap);
-        const size_t mark = h->ws.used;
-        bf16* h0 = ws_take<bf16>(h, (size_t)N * KP0);
-        tc_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(x, obs, trow, tconst, N, g.A, g.Do, g.T, KP0, obs_div, h0);
-        TC_KCHECK(h);
-        int r = fc_actor_infer(h, s, net, h0, N, fc::FINAL_EPS, eps, nullptr, nullptr, nullptr, nullptr);
-        h->ws.used = mark;
-        return r;
-    }
     // the caller may hold workspace pointers (eps, trow) below ws.used: only append
-    const size_t need = h->ws.used + ws_bytes((size_t)N * KP0, 2) + tc_mlp_ws_bytes(N, g.H, h->cfg.actor_act == DPPO_ACT_MISH, false);
-    if (need > h->ws.cap) DPPO_FAIL(-7, "tc_actor_forward: workspace too small (%zu > %zu)", need, h->ws.cap);
     const size_t mark = h->ws.used;
-    TcMlp m; tc_actor_mlp(h, net, m);
-    bf16* h0 = ws_take<bf16>(h, (size_t)N * KP0);
-    tc_mlp_take(h, N, m, false);
-    m.h0 = h0; m.out = eps;
+    TcMlp m; bf16* h0;
+    DPPO_TRY(ws_append(h->ws, [&] { h0 = tc_actor_forward_take(h, net, N, m); }));
+    m.out = eps;
     tc_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(x, obs, trow, tconst, N, g.A, g.Do, g.T, KP0, obs_div, h0);
     TC_KCHECK(h);
-    int r = tc_mlp_forward(h, s, m, N);
+    const int r = fc_ok(h) ? fc_actor_infer(h, s, net, h0, N, fc::FINAL_EPS, eps, nullptr, nullptr, nullptr, nullptr) : tc_mlp_forward(h, s, m, N);
     h->ws.used = mark;
     return r;
 }
-// extra workspace bytes tc_actor_forward appends for N rows
-static size_t tc_actor_forward_ws(const dppo_handle* h, int N) {
-    return ws_bytes((size_t)N * h->tc->KP0, 2) + tc_mlp_ws_bytes(N, h->g.H, h->cfg.actor_act == DPPO_ACT_MISH, false);
-}
 static int tc_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, float* v) {
     const Geom& g = h->g; const int KP0 = h->tc->KP0;
-    DPPO_TRY(ws_reserve(h, ws_bytes((size_t)N * KP0, 2) + tc_mlp_ws_bytes(N, g.Hc, h->cfg.critic_act == DPPO_ACT_MISH, false), s));
     TcMlp m; tc_critic_mlp(h, m);
-    bf16* h0 = ws_take<bf16>(h, (size_t)N * KP0);
-    tc_mlp_take(h, N, m, false);
+    bf16* h0;
+    DPPO_TRY(ws_layout(h->ws, s, [&] { h0 = ws_take<bf16>(h, (size_t)N * KP0); tc_mlp_take(h, N, m, false); }));
     m.h0 = h0; m.out = v;
     // the critic only reads the obs block (the x / one-hot rows of its W0 are zero)
     tc_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(nullptr, obs, nullptr, -1, N, g.A, g.Do, g.T, KP0, 1, h0);
@@ -1026,25 +1011,20 @@ static int tc_ppo_begin(dppo_handle* h, cudaStream_t s, int N, int chunk_rows, i
     P.full_rows = nchunks > 1 ? 1 : 0; P.rows_done = 0; P.dw_done = 0; P.dw_flush_chunk = nchunks / 2 - 1;
     const int NC = P.full_rows ? N : (P.chunk_rows < N ? P.chunk_rows : N);
     P.max_blocks = tc_nblk(N, LOSS8_ROWS) + nchunks;
-    const bool amish = h->cfg.actor_act == DPPO_ACT_MISH, cmish = h->cfg.critic_act == DPPO_ACT_MISH;
-    const size_t pf = tc_part_floats(h, g.H);
     const size_t n_cpa = (size_t)nchunks * h->sm_count * 2 * g.H, n_cpc = (size_t)nchunks * h->sm_count * 2 * g.Hc;
-    size_t need = ws_bytes((size_t)NC * KP0, 2) + tc_mlp_ws_bytes(NC, g.H, amish, true) + tc_mlp_ws_bytes(NC, g.Hc, cmish, true)
-                + ws_bytes((size_t)NC * g.A, 4) + ws_bytes(NC, 4) + 2 * ws_bytes((size_t)NC * 64, 2)
-                + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes((size_t)KP0 * g.Hc, 4)
-                + ws_bytes((size_t)P.max_blocks * 5, 8) + ws_bytes((size_t)P.max_blocks * (g.A + 1), 4) + ws_bytes(n_cpa, 4) + ws_bytes(n_cpc, 4);
-    DPPO_TRY(ws_reserve(h, need, s));
     tc_actor_mlp(h, DPPO_NET_ACTOR_FT, P.ma); tc_critic_mlp(h, P.mc);
-    P.h0 = ws_take<bf16>(h, (size_t)NC * KP0);
-    tc_mlp_take(h, NC, P.ma, true); tc_mlp_take(h, NC, P.mc, true);
-    P.eps = ws_take<float>(h, (size_t)NC * g.A); P.val = ws_take<float>(h, NC);
-    P.depsb = ws_take<bf16>(h, (size_t)NC * 64); P.dvalb = ws_take<bf16>(h, (size_t)NC * 64);
-    P.part = ws_take<float>(h, pf);
-    P.bsum = ws_take<double>(h, (size_t)P.max_blocks * 5);
-    P.colb3 = ws_take<float>(h, (size_t)P.max_blocks * (g.A + 1));
-    // the four accumulators below are adjacent so that one memset clears them
-    P.dw0a = ws_take<float>(h, (size_t)KP0 * g.H); P.dw0c = ws_take<float>(h, (size_t)KP0 * g.Hc);
-    P.cpa = ws_take<float>(h, n_cpa); P.cpc = ws_take<float>(h, n_cpc);
+    DPPO_TRY(ws_layout(h->ws, s, [&] {
+        P.h0 = ws_take<bf16>(h, (size_t)NC * KP0);
+        tc_mlp_take(h, NC, P.ma, true); tc_mlp_take(h, NC, P.mc, true);
+        P.eps = ws_take<float>(h, (size_t)NC * g.A); P.val = ws_take<float>(h, NC);
+        P.depsb = ws_take<bf16>(h, (size_t)NC * 64); P.dvalb = ws_take<bf16>(h, (size_t)NC * 64);
+        P.part = ws_take<float>(h, tc_part_floats(h, g.H));
+        P.bsum = ws_take<double>(h, (size_t)P.max_blocks * 5);
+        P.colb3 = ws_take<float>(h, (size_t)P.max_blocks * (g.A + 1));
+        // the four accumulators below are adjacent so that one memset clears them
+        P.dw0a = ws_take<float>(h, (size_t)KP0 * g.H); P.dw0c = ws_take<float>(h, (size_t)KP0 * g.Hc);
+        P.cpa = ws_take<float>(h, n_cpa); P.cpc = ws_take<float>(h, n_cpc);
+    }));
     const size_t acc_bytes = (size_t)((char*)(P.cpc + n_cpc) - (char*)P.dw0a);
     P.ma.h0 = P.h0; P.mc.h0 = P.h0; P.ma.out = P.eps; P.mc.out = P.val;
     const bool defer = P.ma.fused && P.mc.fused && !h->deterministic;
@@ -1230,20 +1210,18 @@ static int tc_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     const size_t nA = g.ao.n; float* gr = h->grads;
     const size_t ne = (size_t)N * g.A;
     const int nlb = tc_nblk(ne, 256);
-    const size_t pf = tc_part_floats(h, g.H);
-    size_t need = ws_bytes((size_t)N * KP0, 2) + tc_mlp_ws_bytes(N, g.H, h->cfg.actor_act == DPPO_ACT_MISH, true)
-                + 4 * ws_bytes(ne, 4) + ws_bytes(N, 4) + ws_bytes((size_t)N * 64, 2) + ws_bytes(pf, 4)
-                + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes(nlb, 8);
-    DPPO_TRY(ws_reserve(h, need, s));
     TcMlp ma; tc_actor_mlp(h, DPPO_NET_ACTOR, ma);
-    bf16* h0 = ws_take<bf16>(h, (size_t)N * KP0);
-    tc_mlp_take(h, N, ma, true);
-    float* eps = ws_take<float>(h, ne); float* deps = ws_take<float>(h, ne); float* noise = ws_take<float>(h, ne); float* xn = ws_take<float>(h, ne);
-    int* trow = ws_take<int>(h, N);
-    bf16* depsb = ws_take<bf16>(h, (size_t)N * 64);
-    float* part = ws_take<float>(h, pf);
-    float* dw0 = ws_take<float>(h, (size_t)KP0 * g.H);
-    double* bsum = ws_take<double>(h, nlb);
+    bf16 *h0, *depsb; float *eps, *deps, *noise, *xn, *part, *dw0; int* trow; double* bsum;
+    DPPO_TRY(ws_layout(h->ws, s, [&] {
+        h0 = ws_take<bf16>(h, (size_t)N * KP0);
+        tc_mlp_take(h, N, ma, true);
+        eps = ws_take<float>(h, ne); deps = ws_take<float>(h, ne); noise = ws_take<float>(h, ne); xn = ws_take<float>(h, ne);
+        trow = ws_take<int>(h, N);
+        depsb = ws_take<bf16>(h, (size_t)N * 64);
+        part = ws_take<float>(h, tc_part_floats(h, g.H));
+        dw0 = ws_take<float>(h, (size_t)KP0 * g.H);
+        bsum = ws_take<double>(h, nlb);
+    }));
     ma.h0 = h0; ma.out = eps;
     if (!h->deterministic) {
         CUDA_TRY(cudaMemsetAsync(gr, 0, nA * sizeof(float), s));

@@ -1470,22 +1470,19 @@ static void ts_critic_mlp(const dppo_handle* h, TsMlp& m) {
     m.fp = h->cfg.critic_act == DPPO_ACT_RELU ? 4 : 2;                               // Mish is smooth
     m.b0 = w + g.co.bin; m.b1 = w + g.co.b1;
 }
-static size_t ts_mlp_ws_bytes(int N, int H, int KP0, bool mish, bool bwd) {
-    return 2 * (2 * ws_bytes((size_t)N * KP0, 2) + 2 * ws_bytes((size_t)N * H, 2)) + 2 * ws_bytes((size_t)N * H, 2) * (size_t)((mish ? 2 : 0) + (bwd ? 4 : 0))
-         + 2 * ws_bytes((size_t)N * (H / 32), 4);
-}
 static SplitT ts_take(dppo_handle* h, size_t n, int planes) {
     SplitT t = split_null();
     for (int pl = 0; pl < planes; ++pl) t.p[pl] = ws_take<bf16>(h, n);
     return t;
 }
-static void ts_mlp_take(dppo_handle* h, int N, TsMlp& m, bool bwd) {
+// own_h0 = false: the net reads another net's input planes (h0, h0b), which the caller points it at
+static void ts_mlp_take(dppo_handle* h, int N, TsMlp& m, bool bwd, bool own_h0 = true) {
     const size_t n = (size_t)N * m.H;
-    m.h0 = ts_take(h, (size_t)N * m.KP0, 2);
+    if (own_h0) m.h0 = ts_take(h, (size_t)N * m.KP0, 2);
     m.a0 = ts_take(h, n, 2); m.a1 = ts_take(h, n, 2);
     if (m.act1 == 2) { m.g0 = ts_take(h, n, 2); m.g1 = ts_take(h, n, 2); }
     if (bwd) { m.dh1 = ts_take(h, n, 2); m.du = ts_take(h, n, 2); }
-    if (bwd && m.fp == 4) { m.h0b = ts_take(h, (size_t)N * m.KP0, 2); m.a0b = ts_take(h, n, 2); m.a1b = ts_take(h, n, 2); }
+    if (bwd && m.fp == 4) { if (own_h0) m.h0b = ts_take(h, (size_t)N * m.KP0, 2); m.a0b = ts_take(h, n, 2); m.a1b = ts_take(h, n, 2); }
     m.m0 = ws_take<uint32_t>(h, (size_t)N * (m.H / 32)); m.m1 = ws_take<uint32_t>(h, (size_t)N * (m.H / 32));
 }
 static ts::Operand ts_op(const bf16* const* p, size_t off, bool mn_major, int64_t mn, int64_t k, int64_t ld) {
@@ -1858,16 +1855,18 @@ static size_t ts_part_floats(const dppo_handle* h, int H) {
     return a > b ? a : b;
 }
 // ------------------------------------------------------------------ forward-only programs
-static size_t ts_actor_forward_ws(const dppo_handle* h, int N) { return ts_mlp_ws_bytes(N, h->g.H, h->ts->KP0, h->cfg.actor_act == DPPO_ACT_MISH, false); }
+// the buffers ts_actor_forward appends for N rows
+static void ts_actor_forward_take(dppo_handle* h, int net, int N, TsMlp& m) {
+    ts_actor_mlp(h, net, m);
+    ts_mlp_take(h, N, m, false);
+}
 // eps[N][A] = actor(x, t, obs); appends to the workspace (the caller may hold pointers below ws.used)
 static int ts_actor_forward(dppo_handle* h, cudaStream_t s, int net, const float* x, const float* obs, int obs_div, int N,
                             const int* trow, int tconst, float* eps, int chainK = 0) {
     const Geom& g = h->g; const int KP0 = h->ts->KP0;
-    const size_t need = h->ws.used + ts_actor_forward_ws(h, N);
-    if (need > h->ws.cap) DPPO_FAIL(-7, "ts_actor_forward: workspace too small (%zu > %zu)", need, h->ws.cap);
     const size_t mark = h->ws.used;
-    TsMlp m; ts_actor_mlp(h, net, m);
-    ts_mlp_take(h, N, m, false);
+    TsMlp m;
+    DPPO_TRY(ws_append(h->ws, [&] { ts_actor_forward_take(h, net, N, m); }));
     m.out = eps;
     // every program of this mode folds, so that the log-prob forward and the update's forward are the same arithmetic and the PPO
     // ratio of unchanged weights is exactly 1 (the full-size parity tests assert it)
@@ -1880,9 +1879,8 @@ static int ts_actor_forward(dppo_handle* h, cudaStream_t s, int net, const float
 }
 static int ts_value(dppo_handle* h, cudaStream_t s, const float* obs, int N, float* v) {
     const Geom& g = h->g; const int KP0 = h->ts->KP0;
-    DPPO_TRY(ws_reserve(h, ts_mlp_ws_bytes(N, g.Hc, KP0, h->cfg.critic_act == DPPO_ACT_MISH, false), s));
     TsMlp m; ts_critic_mlp(h, m);
-    ts_mlp_take(h, N, m, false);
+    DPPO_TRY(ws_layout(h->ws, s, [&] { ts_mlp_take(h, N, m, false); }));
     m.out = v;
     DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, s));
     ts_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(nullptr, obs, nullptr, -1, N, g.A, g.Do, g.T, KP0, 1,
@@ -1907,7 +1905,6 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     const Geom& g = h->g; const int KP0 = h->ts->KP0;
     const size_t nA = g.ao.n, nC = g.co.n;
     float* gr = h->grads;
-    const bool amish = h->cfg.actor_act == DPPO_ACT_MISH, cmish = h->cfg.critic_act == DPPO_ACT_MISH;
     const bool loss8 = idx ? loss8_ok(g.A, 128, idx->chains, idx->olp) : loss8_ok(g.A, 128, prev, nxt, oldlogp);
     const int NOP = ts_nop(g.A);                                  // the actor's seed width: 64 (A <= 32) or 128
     const bool wide = NOP > 64;                                   // the loss kernel takes a warp per row (tc_ppo_loss8_kernel<32>)
@@ -1916,24 +1913,21 @@ static int ts_ppo_step(dppo_handle* h, cudaStream_t s, const float* obs, const f
     const int nlb = loss8 ? tc_nblk(N, wide ? 256 / 32 : LOSS8_ROWS) : tc_nblk(N, 128);
     const int nrb = (N + 31) / 32;
     const size_t pf = ts_part_floats(h, g.H);
-    const size_t need = ts_mlp_ws_bytes(N, g.H, KP0, amish, true) + ts_mlp_ws_bytes(N, g.Hc, KP0, cmish, true)
-                      + 2 * ws_bytes((size_t)N * g.A, 4) + 2 * ws_bytes(N, 4) + 2 * ws_bytes((size_t)N * NOP, 2) + 2 * ws_bytes((size_t)N * 64, 2)
-                      + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes((size_t)KP0 * g.Hc, 4) + ws_bytes((size_t)nlb * 5, 8) + ws_bytes(16, 4)
-                      + ws_bytes((size_t)nlb * (g.A + 1), 4) + ws_bytes((size_t)nrb * 2 * g.H, 4) + ws_bytes((size_t)nrb * 2 * g.Hc, 4)
-                      + ws_bytes((size_t)(g.H + g.Hc + 2 * KP0) * NOg + g.H + g.Hc, 4);
-    DPPO_TRY(ws_reserve(h, need, s));
     TsMlp ma, mc; ts_actor_mlp(h, DPPO_NET_ACTOR_FT, ma); ts_critic_mlp(h, mc);
-    ts_mlp_take(h, N, ma, true); ts_mlp_take(h, N, mc, true);
-    float* eps = ws_take<float>(h, (size_t)N * g.A); float* deps = ws_take<float>(h, (size_t)N * g.A);
-    float* val = ws_take<float>(h, N); float* dval = ws_take<float>(h, N);
-    SplitT depsb = ts_take(h, (size_t)N * NOP, 2), dvalb = ts_take(h, (size_t)N * 64, 2);
-    float* part = ws_take<float>(h, pf);
-    float* dw0a = ws_take<float>(h, (size_t)KP0 * g.H); float* dw0c = ws_take<float>(h, (size_t)KP0 * g.Hc);
-    double* bsum = ws_take<double>(h, (size_t)nlb * 5);
-    int* ebeg = ws_take<int>(h, 16);
-    float* colb3 = ws_take<float>(h, (size_t)nlb * (g.A + 1));
-    float* cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H); float* cpc = ws_take<float>(h, (size_t)nrb * 2 * g.Hc);
-    float* gfold = ws_take<float>(h, (size_t)(g.H + g.Hc + 2 * KP0) * NOg + g.H + g.Hc);      // a1^T dout / h0^T dout of both nets (folded output layer) + scratch
+    float *eps, *deps, *val, *dval, *part, *dw0a, *dw0c, *colb3, *cpa, *cpc, *gfold; SplitT depsb, dvalb; double* bsum; int* ebeg;
+    DPPO_TRY(ws_layout(h->ws, s, [&] {
+        ts_mlp_take(h, N, ma, true); ts_mlp_take(h, N, mc, true, false);
+        eps = ws_take<float>(h, (size_t)N * g.A); deps = ws_take<float>(h, (size_t)N * g.A);
+        val = ws_take<float>(h, N); dval = ws_take<float>(h, N);
+        depsb = ts_take(h, (size_t)N * NOP, 2); dvalb = ts_take(h, (size_t)N * 64, 2);
+        part = ws_take<float>(h, pf);
+        dw0a = ws_take<float>(h, (size_t)KP0 * g.H); dw0c = ws_take<float>(h, (size_t)KP0 * g.Hc);
+        bsum = ws_take<double>(h, (size_t)nlb * 5);
+        ebeg = ws_take<int>(h, 16);
+        colb3 = ws_take<float>(h, (size_t)nlb * (g.A + 1));
+        cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H); cpc = ws_take<float>(h, (size_t)nrb * 2 * g.Hc);
+        gfold = ws_take<float>(h, (size_t)(g.H + g.Hc + 2 * KP0) * NOg + g.H + g.Hc);      // a1^T dout / h0^T dout of both nets (folded output layer) + scratch
+    }));
     float* ga1 = gfold; float* ga0 = ga1 + (size_t)g.H * g.A; float* gc1 = ga0 + (size_t)KP0 * g.A; float* gc0 = gc1 + g.Hc;
     ma.out = eps; mc.out = val;
     // The critic's GEMMs are independent of the actor's until the loss (and again until the weight gradients) and their tiles are
@@ -2024,22 +2018,22 @@ static int ts_pretrain_grads(dppo_handle* h, cudaStream_t s, const float* action
     const int nrb = (N + 31) / 32;
     const int NOP = ts_nop(g.A), NOg = g.A > 32 ? g.A : 32;
     const size_t pf = ts_part_floats(h, g.H);
-    const size_t need = ts_mlp_ws_bytes(N, g.H, KP0, h->cfg.actor_act == DPPO_ACT_MISH, true) + 4 * ws_bytes(ne, 4) + ws_bytes(N, 4)
-                      + 2 * ws_bytes((size_t)N * NOP, 2) + ws_bytes(pf, 4) + ws_bytes((size_t)KP0 * g.H, 4) + ws_bytes(nlb, 8) + ws_bytes(16, 4)
-                      + ws_bytes((size_t)nrb * 2 * g.H, 4) + ws_bytes((size_t)(g.H + KP0) * NOg + g.H, 4);
-    DPPO_TRY(ws_reserve(h, need, s));
     TsMlp ma; ts_actor_mlp(h, DPPO_NET_ACTOR, ma);
-    ts_mlp_take(h, N, ma, true);
-    float* ga1 = ws_take<float>(h, (size_t)(g.H + KP0) * NOg + g.H); float* ga0 = ga1 + (size_t)g.H * g.A;    // + scratch for the unwritten slot-0 sums
+    float *ga1, *eps, *deps, *noise, *xn, *part, *dw0, *cpa; int *trow, *ebeg; SplitT depsb; double* bsum;
+    DPPO_TRY(ws_layout(h->ws, s, [&] {
+        ts_mlp_take(h, N, ma, true);
+        ga1 = ws_take<float>(h, (size_t)(g.H + KP0) * NOg + g.H);    // + scratch for the unwritten slot-0 sums
+        eps = ws_take<float>(h, ne); deps = ws_take<float>(h, ne); noise = ws_take<float>(h, ne); xn = ws_take<float>(h, ne);
+        trow = ws_take<int>(h, N);
+        depsb = ts_take(h, (size_t)N * NOP, 2);
+        part = ws_take<float>(h, pf);
+        dw0 = ws_take<float>(h, (size_t)KP0 * g.H);
+        bsum = ws_take<double>(h, nlb);
+        ebeg = ws_take<int>(h, 16);
+        cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H);
+    }));
+    float* ga0 = ga1 + (size_t)g.H * g.A;
     DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR, s));
-    float* eps = ws_take<float>(h, ne); float* deps = ws_take<float>(h, ne); float* noise = ws_take<float>(h, ne); float* xn = ws_take<float>(h, ne);
-    int* trow = ws_take<int>(h, N);
-    SplitT depsb = ts_take(h, (size_t)N * NOP, 2);
-    float* part = ws_take<float>(h, pf);
-    float* dw0 = ws_take<float>(h, (size_t)KP0 * g.H);
-    double* bsum = ws_take<double>(h, nlb);
-    int* ebeg = ws_take<int>(h, 16);
-    float* cpa = ws_take<float>(h, (size_t)nrb * 2 * g.H);
     ma.out = eps;
     pretrain_prep_kernel<<<tc_nblk(ne, 256), 256, 0, s>>>(actions, t_in, noise_in, N, g.A, g.T, h->sched, seed, offset, row_offset, trow, noise, xn); TC_KCHECK(h);
     ts_pack_h0_kernel<<<tc_nblk((size_t)N * (KP0 / 8), 256), 256, 0, s>>>(xn, obs, trow, 0, N, g.A, g.Do, g.T, KP0, 1, ma.h0, ma.h0b, 0); TC_KCHECK(h);
