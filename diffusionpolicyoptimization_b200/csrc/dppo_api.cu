@@ -628,10 +628,16 @@ extern "C" int dppo_logprobs_subsample(dppo_handle* h, const float* obs, const f
 }
 
 // ------------------------------------------------------------------ sampling
+// AP <= 32: every CTA computes all 512 layer-0 columns; wider chunks: each CTA its own 32, all-gathered (sample_cluster.cuh)
+template <int AP, int R>
+static auto cluster_kernel() {
+    if constexpr (AP > 32) return sample_cluster_wide_kernel<AP, R>;
+    else return sample_cluster_kernel<AP, R>;
+}
 template <int AP, int R>
 static int launch_cluster(dppo_handle* h, cudaStream_t s, ClusterSampleP& p, int B, bool probe_only, int* max_clusters) {
-    auto kern = sample_cluster_kernel<AP, R>;
-    size_t smem = cluster_sample_smem_floats<AP, R>() * sizeof(float);
+    auto kern = cluster_kernel<AP, R>();
+    size_t smem = (AP > 32 ? cluster_sample_wide_smem_floats<AP, R>() : cluster_sample_smem_floats<AP, R>()) * sizeof(float);
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
@@ -765,10 +771,10 @@ static int sample_impl(dppo_handle* h, const float* obs, int B, int deterministi
     hp.deterministic = deterministic;
     const bool split = ts_eligible(h, B);
     const bool tensor = tc_eligible(h, B) || split;
-    const bool cluster_shape = (g.H == CS_H && g.A <= 32 && h->cfg.actor_act == DPPO_ACT_RELU && h->force_path != 2);
+    const bool cluster_shape = (g.H == CS_H && g.A <= 128 && h->cfg.actor_act == DPPO_ACT_RELU && h->force_path != 2);
     // the persistent cluster kernel wins while the chain is latency bound; beyond that rows are
-    // plentiful enough for real GEMM tiles
-    const int cluster_limit = h->cfg.precision == DPPO_PREC_BF16 ? 1024 : 4096;
+    // plentiful enough for real GEMM tiles.  Wide chunks cross over earlier (measured, DESIGN.md §5.3)
+    const int cluster_limit = h->cfg.precision == DPPO_PREC_BF16 ? 1024 : g.A <= 32 ? 4096 : g.A <= 64 ? 2048 : 1024;
     if (cluster_shape && !tensor && (B <= cluster_limit || h->force_path == 1) && h->cluster_max != 0) {
         ClusterSampleP p; memset(&p, 0, sizeof(p));
         p.w[0] = h->net_w[DPPO_NET_ACTOR]; p.w[1] = h->net_w[DPPO_NET_ACTOR_FT];
@@ -780,7 +786,8 @@ static int sample_impl(dppo_handle* h, const float* obs, int B, int deterministi
         p.B = B; p.A = g.A; p.Do = g.Do; p.T = g.T; p.K = g.K; p.td = g.td; p.use_base_policy = use_base_policy;
         p.hp = hp; p.seed = seed; p.offset = offset; p.row_offset = row_offset;
         if (env) { p.raw_actions = env->raw_actions; p.act_min = amin; p.act_max = amax; p.act_cols = env->act_steps * ad_; p.Da = ad_; }
-        int r = g.A <= 12 ? cluster_dispatch<12>(h, s, p, B) : (g.A <= 24 ? cluster_dispatch<24>(h, s, p, B) : cluster_dispatch<32>(h, s, p, B));
+        int r = g.A <= 12 ? cluster_dispatch<12>(h, s, p, B) : g.A <= 24 ? cluster_dispatch<24>(h, s, p, B)
+              : g.A <= 32 ? cluster_dispatch<32>(h, s, p, B) : g.A <= 64 ? cluster_dispatch<64>(h, s, p, B) : cluster_dispatch<128>(h, s, p, B);
         if (r == 0) { h->last_path = 1; return 0; }
         if (h->force_path == 1) return r;
         h->cluster_max = 0;   // not launchable here: remember and fall through to the layered path
