@@ -628,16 +628,29 @@ extern "C" int dppo_logprobs_subsample(dppo_handle* h, const float* obs, const f
 }
 
 // ------------------------------------------------------------------ sampling
-// AP <= 32: every CTA computes all 512 layer-0 columns; wider chunks: each CTA its own 32, all-gathered (sample_cluster.cuh)
-template <int AP, int R>
+// H = 512, AP <= 32: every CTA computes all 512 layer-0 columns; H = 512, wider chunks: each CTA its own 32, all-gathered;
+// H in {256, 768, 1024}: each CTA its own H / 16, all-gathered, with a partly resident W1 slice (sample_cluster.cuh)
+template <int H, int AP, int R>
 static auto cluster_kernel() {
-    if constexpr (AP > 32) return sample_cluster_wide_kernel<AP, R>;
+    if constexpr (H != CS_H) return sample_cluster_width_kernel<H, AP, R>;
+    else if constexpr (AP > 32) return sample_cluster_wide_kernel<AP, R>;
     else return sample_cluster_kernel<AP, R>;
 }
-template <int AP, int R>
+template <int H, int AP, int R>
+static constexpr size_t cluster_smem_floats() {
+    if constexpr (H != CS_H) return ClusterWidthPlan<H, AP, R>::floats;
+    else if constexpr (AP > 32) return cluster_sample_wide_smem_floats<AP, R>();
+    else return cluster_sample_smem_floats<AP, R>();
+}
+template <int H, int AP>
+static constexpr int cluster_rmax() {
+    if constexpr (H != CS_H) return cluster_width_rmax<H, AP>();
+    else return 8;
+}
+template <int H, int AP, int R>
 static int launch_cluster(dppo_handle* h, cudaStream_t s, ClusterSampleP& p, int B, bool probe_only, int* max_clusters) {
-    auto kern = cluster_kernel<AP, R>();
-    size_t smem = (AP > 32 ? cluster_sample_wide_smem_floats<AP, R>() : cluster_sample_smem_floats<AP, R>()) * sizeof(float);
+    auto kern = cluster_kernel<H, AP, R>();
+    size_t smem = cluster_smem_floats<H, AP, R>() * sizeof(float);
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
@@ -657,19 +670,37 @@ static int launch_cluster(dppo_handle* h, cudaStream_t s, ClusterSampleP& p, int
     KLAUNCH(h);
     return 0;
 }
-template <int AP>
+// rows per cluster pass: the fewest that cover B in one pass of the resident clusters, capped at what the width's
+// shared-memory plan allows (more rows than that loop over the chunks)
+template <int H, int AP>
 static int cluster_dispatch(dppo_handle* h, cudaStream_t s, ClusterSampleP& p, int B) {
+    constexpr int RMAX = cluster_rmax<H, AP>();
     int nc = h->cluster_max;
     if (nc < 0) {
-        DPPO_TRY((launch_cluster<AP, 8>(h, s, p, B, true, &nc)));
+        DPPO_TRY((launch_cluster<H, AP, RMAX>(h, s, p, B, true, &nc)));
         h->cluster_max = nc;
     }
     if (nc < 1) DPPO_FAIL(-5, "cluster sampler unavailable on this device");
-    int per = (B + nc - 1) / nc;
-    if (per <= 2) return launch_cluster<AP, 2>(h, s, p, B, false, nullptr);
-    if (per <= 4) return launch_cluster<AP, 4>(h, s, p, B, false, nullptr);
-    if (per <= 6) return launch_cluster<AP, 6>(h, s, p, B, false, nullptr);
-    return launch_cluster<AP, 8>(h, s, p, B, false, nullptr);
+    const int per = std::min((B + nc - 1) / nc, RMAX);
+    if (per <= 2) return launch_cluster<H, AP, 2>(h, s, p, B, false, nullptr);
+    if (per <= 4) return launch_cluster<H, AP, std::min(4, RMAX)>(h, s, p, B, false, nullptr);
+    if (per <= 6) return launch_cluster<H, AP, std::min(6, RMAX)>(h, s, p, B, false, nullptr);
+    return launch_cluster<H, AP, std::min(8, RMAX)>(h, s, p, B, false, nullptr);
+}
+// fp32 rows up to which the cluster sampler beats the layered path (the measured crossovers of DESIGN.md §5.3)
+static int cluster_row_limit(int H, int A) {
+    if (H == 1024) return 1024;
+    if (H != CS_H) return A <= 64 ? 2048 : 1024;     // 256, 768
+    return A <= 32 ? 4096 : A <= 64 ? 2048 : 1024;
+}
+template <int H>
+static int cluster_dispatch_width(dppo_handle* h, cudaStream_t s, ClusterSampleP& p, int B) {
+    const int A = p.A;
+    if constexpr (H == CS_H)
+        return A <= 12 ? cluster_dispatch<H, 12>(h, s, p, B) : A <= 24 ? cluster_dispatch<H, 24>(h, s, p, B)
+             : A <= 32 ? cluster_dispatch<H, 32>(h, s, p, B) : A <= 64 ? cluster_dispatch<H, 64>(h, s, p, B) : cluster_dispatch<H, 128>(h, s, p, B);
+    else
+        return A <= 32 ? cluster_dispatch<H, 32>(h, s, p, B) : A <= 64 ? cluster_dispatch<H, 64>(h, s, p, B) : cluster_dispatch<H, 128>(h, s, p, B);
 }
 
 static int sample_layered_fp32(dppo_handle* h, cudaStream_t s, const float* obs, int B, int use_base, SampleHyper hp,
@@ -771,10 +802,11 @@ static int sample_impl(dppo_handle* h, const float* obs, int B, int deterministi
     hp.deterministic = deterministic;
     const bool split = ts_eligible(h, B);
     const bool tensor = tc_eligible(h, B) || split;
-    const bool cluster_shape = (g.H == CS_H && g.A <= 128 && h->cfg.actor_act == DPPO_ACT_RELU && h->force_path != 2);
+    const bool cluster_width = g.H == 256 || g.H == 512 || g.H == 768 || g.H == 1024;
+    const bool cluster_shape = (cluster_width && g.A <= 128 && h->cfg.actor_act == DPPO_ACT_RELU && h->force_path != 2);
     // the persistent cluster kernel wins while the chain is latency bound; beyond that rows are
-    // plentiful enough for real GEMM tiles.  Wide chunks cross over earlier (measured, DESIGN.md §5.3)
-    const int cluster_limit = h->cfg.precision == DPPO_PREC_BF16 ? 1024 : g.A <= 32 ? 4096 : g.A <= 64 ? 2048 : 1024;
+    // plentiful enough for real GEMM tiles.  Wide chunks and other widths cross over earlier (measured, DESIGN.md §5.3)
+    const int cluster_limit = h->cfg.precision == DPPO_PREC_BF16 ? 1024 : cluster_row_limit(g.H, g.A);
     if (cluster_shape && !tensor && (B <= cluster_limit || h->force_path == 1) && h->cluster_max != 0) {
         ClusterSampleP p; memset(&p, 0, sizeof(p));
         p.w[0] = h->net_w[DPPO_NET_ACTOR]; p.w[1] = h->net_w[DPPO_NET_ACTOR_FT];
@@ -786,8 +818,8 @@ static int sample_impl(dppo_handle* h, const float* obs, int B, int deterministi
         p.B = B; p.A = g.A; p.Do = g.Do; p.T = g.T; p.K = g.K; p.td = g.td; p.use_base_policy = use_base_policy;
         p.hp = hp; p.seed = seed; p.offset = offset; p.row_offset = row_offset;
         if (env) { p.raw_actions = env->raw_actions; p.act_min = amin; p.act_max = amax; p.act_cols = env->act_steps * ad_; p.Da = ad_; }
-        int r = g.A <= 12 ? cluster_dispatch<12>(h, s, p, B) : g.A <= 24 ? cluster_dispatch<24>(h, s, p, B)
-              : g.A <= 32 ? cluster_dispatch<32>(h, s, p, B) : g.A <= 64 ? cluster_dispatch<64>(h, s, p, B) : cluster_dispatch<128>(h, s, p, B);
+        int r = g.H == 256 ? cluster_dispatch_width<256>(h, s, p, B) : g.H == 512 ? cluster_dispatch_width<512>(h, s, p, B)
+              : g.H == 768 ? cluster_dispatch_width<768>(h, s, p, B) : cluster_dispatch_width<1024>(h, s, p, B);
         if (r == 0) { h->last_path = 1; return 0; }
         if (h->force_path == 1) return r;
         h->cluster_max = 0;   // not launchable here: remember and fall through to the layered path

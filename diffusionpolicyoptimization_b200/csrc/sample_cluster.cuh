@@ -456,3 +456,288 @@ __global__ void __launch_bounds__(CS_THREADS, 1) sample_cluster_wide_kernel(cons
     // no CTA may exit while peers can still write into its shared memory
     cluster.sync();
 }
+
+// ---- other hidden widths: sample_cluster_width_kernel<H, AP, R>, H in {256, 768, 1024}, AP in {32, 64, 128}
+// The wide kernel's scheme for every chunk width: each CTA computes its own COLS = H / 16 columns of layer 0 from a resident
+// [AP][COLS] slice of W_in's x-rows, relu(u) is all-gathered over DSMEM behind a cluster barrier, then the L1 slice, the partial
+// folded output layer and the posterior update follow as in the wide kernel.  What changes with COLS:
+//   * products over COLS columns (layer 0 and the L1 slice): lane & 15 picks a column, the thread owns the NC = COLS / 16 columns
+//     c, c + 16, ... and lane >> 4 picks half of the R rows.  The two half-warps read the same weight address (broadcast) and two
+//     relu(u) rows; actA rows are padded by 4 floats so those two float4 reads fall in different banks.  The K rows are split over
+//     the 16 warps (H / 16 rows each) and reduced across warps in shared memory, as at H = 512;
+//   * the W1 slice is partly resident: of each warp's H / 16 k-rows the first KRW stay in shared memory and the rest are read
+//     from L2 (coalesced, one 64-byte segment per column group and half-warp) every denoising step.  KRW is the largest multiple
+//     of 4 that the (H, AP, R) plan leaves room for (ClusterWidthPlan).  Which rows are resident does not change the order of
+//     the sums, so the results do not depend on R.
+// The H = 512 kernels above are left as they are (their A <= 32 and A > 32 instantiations keep their code instruction for
+// instruction); a fix to the shared phases belongs in all three.
+constexpr size_t CS_SMEM_FLOATS = 227 * 1024 / sizeof(float);   // the most dynamic shared memory a block can have (sm_100)
+
+template <int H, int AP, int R>
+struct ClusterWidthPlan {
+    static constexpr int COLS = H / CS_C;
+    static constexpr size_t fixed = (size_t)3 * COLS * AP          // W3s, W23s, Wxs
+                                  + (size_t)R * (H + 4) + (size_t)R * H   // actA (rows padded by 4), red
+                                  + (size_t)3 * R * COLS           // cobs, uown, out1
+                                  + (size_t)R * AP * (1 + CS_C)    // xs, part[16]
+                                  + COLS + AP;                     // b1s, b3s
+    static constexpr bool fits = fixed <= CS_SMEM_FLOATS;
+    // resident k-rows of W1 per warp: what is left, in multiples of 4, at most the warp's H / 16
+    static constexpr size_t room = fits ? (CS_SMEM_FLOATS - fixed) / ((size_t)CS_C * COLS) / 4 * 4 : 0;
+    static constexpr int krw = room < (size_t)(H / CS_C) ? (int)room : H / CS_C;
+    static constexpr size_t floats = fixed + (size_t)krw * CS_C * COLS;
+};
+// the most rows per cluster pass whose plan fits
+template <int H, int AP>
+constexpr int cluster_width_rmax() {
+    return ClusterWidthPlan<H, AP, 8>::fits ? 8 : ClusterWidthPlan<H, AP, 6>::fits ? 6 : ClusterWidthPlan<H, AP, 4>::fits ? 4 : 2;
+}
+
+template <int H, int AP, int R>
+__global__ void __launch_bounds__(CS_THREADS, 1) sample_cluster_width_kernel(const ClusterSampleP p) {
+    constexpr int COLS = H / CS_C;          // hidden columns per CTA
+    constexpr int NC = COLS / 16;           // columns per thread in the products
+    constexpr int RH = R / 2;               // rows per half-warp
+    constexpr int LDA = H + 4;              // actA row stride
+    constexpr int KPW = H / CS_C;           // k-rows of W1 per warp
+    constexpr int KRW = ClusterWidthPlan<H, AP, R>::krw;   // of which resident
+    constexpr int KW = AP / 16;             // x-rows of W_in per warp in layer 0
+    constexpr int NE = (R * AP + CS_THREADS - 1) / CS_THREADS;
+    static_assert(H % 256 == 0 && H != CS_H && H <= 1024, "widths other than 512, multiples of 256");
+    static_assert(AP % 16 == 0 && R % 2 == 0 && R * COLS <= CS_THREADS, "thread mapping");
+    static_assert(ClusterWidthPlan<H, AP, R>::fits && KRW % 4 == 0 && ClusterWidthPlan<H, AP, R>::floats <= CS_SMEM_FLOATS,
+                  "shared-memory plan exceeds 227 KB");
+    cg::cluster_group cluster = cg::this_cluster();
+    const int crank = (int)cluster.block_rank();
+    const int cid = blockIdx.x / CS_C, nclusters = gridDim.x / CS_C;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int c16 = lane & 15, half = lane >> 4;
+    const int col0 = crank * COLS;
+    const int A = p.A, T = p.T, K = p.K, B = p.B;
+
+    extern __shared__ __align__(16) float smem[];
+    float* W3s = smem;                         // [COLS][AP]
+    float* W23s = W3s + COLS * AP;             // [COLS][AP]
+    float* Wxs = W23s + COLS * AP;             // [AP][COLS]  W_in[a][col0 + j], rows a >= A zeroed
+    float* actA = Wxs + AP * COLS;             // [R][LDA]    relu(u), all-gathered
+    float* red = actA + R * LDA;               // [16][R][COLS] cross-warp partials (layer 0, then L1)
+    float* cobs = red + R * H;                 // [R][COLS]   obs[r] @ W_in[A+td:, col0 + j]
+    float* uown = cobs + R * COLS;             // [R][COLS]   raw u, own columns (residual)
+    float* out1 = uown + R * COLS;             // [R][COLS]   relu(h1), own columns
+    float* xs = out1 + R * COLS;               // [R][AP]     current x
+    float* part = xs + R * AP;                 // [16][R][AP] partial eps of every CTA
+    float* b1s = part + CS_C * R * AP;         // [COLS]
+    float* b3s = b1s + COLS;                   // [AP]
+    float* W1s = b3s + AP;                     // [16][KRW][COLS] resident k-rows of every warp's share of the W1 slice
+
+    for (int chunk = cid; chunk < p.nchunks; chunk += nclusters) {
+        const int row0 = chunk * R;
+        // ---- initialise x (x_T injected or Philox slot 0)
+#pragma unroll
+        for (int q = 0; q < NE; ++q) {
+            const int e = tid + q * CS_THREADS;
+            if (e < R * AP) {
+                const int r = e / AP, a = e % AP;
+                float v = 0.f;
+                if (a < A && row0 + r < B) {
+                    v = p.xT ? p.xT[(size_t)(row0 + r) * A + a]
+                             : philox_normal(p.seed, p.offset, p.row_offset + row0 + r, 0, a);
+                    if (crank == 0 && p.chains && K == T) p.chains[((size_t)(row0 + r) * (K + 1)) * A + a] = v;
+                }
+                xs[e] = v;
+            }
+        }
+        __syncthreads();
+        int cur_net = -1;
+
+        for (int i = 0; i < T; ++i) {
+            const int t = T - 1 - i;
+            const int net = (t < K && !p.use_base_policy) ? 1 : 0;
+            const float* w = p.w[net];
+            if (net != cur_net) {
+                // ---- (re)load this net's resident slices and recompute its obs term
+                for (int idx = tid; idx < CS_C * KRW * COLS; idx += CS_THREADS) {
+                    const int wk = idx / (KRW * COLS), rem = idx % (KRW * COLS);
+                    W1s[idx] = w[p.o.w1 + (size_t)(wk * KPW + rem / COLS) * H + col0 + rem % COLS];
+                }
+                for (int idx = tid; idx < COLS * AP; idx += CS_THREADS) {
+                    int k = idx / AP, a = idx % AP;
+                    W3s[idx] = a < A ? w[p.o.w3 + (size_t)(col0 + k) * A + a] : 0.f;
+                    W23s[idx] = a < A ? p.w23[net][(size_t)(col0 + k) * A + a] : 0.f;
+                }
+                if (tid < COLS) b1s[tid] = w[p.o.b1 + col0 + tid];
+                if (tid < AP) b3s[tid] = tid < A ? p.b23[net][tid] : 0.f;
+                for (int idx = tid; idx < AP * COLS; idx += CS_THREADS) {
+                    const int a = idx / COLS, j = idx % COLS;
+                    Wxs[idx] = a < A ? w[p.o.win + (size_t)a * H + col0 + j] : 0.f;
+                }
+                if (tid < R * COLS) {
+                    const int r = tid / COLS, j = tid % COLS;
+                    float c = 0.f;
+                    for (int jo = 0; jo < p.Do; ++jo) {
+                        const float ov = (row0 + r < B) ? p.obs[(size_t)(row0 + r) * p.Do + jo] : 0.f;
+                        c = fmaf(ov, w[p.o.win + (size_t)(A + p.td + jo) * H + col0 + j], c);
+                    }
+                    cobs[tid] = c;
+                }
+                cur_net = net;
+                __syncthreads();
+            }
+            // the bias row of this step's own columns and this step's noise do not depend on the products: fetch them first
+            const float btv = tid < R * COLS ? p.bt[net][(size_t)t * H + col0 + tid % COLS] : 0.f;
+            float nz[NE];
+#pragma unroll
+            for (int q = 0; q < NE; ++q) {
+                const int e = tid + q * CS_THREADS;
+                nz[q] = 0.f;
+                if (e < R * AP) {
+                    const int r = e / AP, a = e % AP;
+                    if (a < A && row0 + r < B) {
+                        const int64_t row = row0 + r;
+                        nz[q] = p.noise ? p.noise[((size_t)i * B + row) * A + a] : philox_normal(p.seed, p.offset, p.row_offset + row, 1 + i, a);
+                    }
+                }
+            }
+            // ---- L0, own columns: u[:, cols] = x @ W_in[0:AP, cols] (K split over the warps) + obs term + bt[t]
+            {
+                float acc[RH][NC];
+#pragma unroll
+                for (int rr = 0; rr < RH; ++rr)
+#pragma unroll
+                    for (int m = 0; m < NC; ++m) acc[rr][m] = 0.f;
+#pragma unroll
+                for (int kk = 0; kk < KW; ++kk) {
+                    const int a = warp * KW + kk;
+                    float wv[NC];
+#pragma unroll
+                    for (int m = 0; m < NC; ++m) wv[m] = Wxs[a * COLS + c16 + 16 * m];
+#pragma unroll
+                    for (int rr = 0; rr < RH; ++rr) {
+                        const float xv = xs[(2 * rr + half) * AP + a];
+#pragma unroll
+                        for (int m = 0; m < NC; ++m) acc[rr][m] = fmaf(xv, wv[m], acc[rr][m]);
+                    }
+                }
+#pragma unroll
+                for (int rr = 0; rr < RH; ++rr)
+#pragma unroll
+                    for (int m = 0; m < NC; ++m) red[(warp * R + 2 * rr + half) * COLS + c16 + 16 * m] = acc[rr][m];
+            }
+            __syncthreads();
+            if (tid < R * COLS) {
+                const int r = tid / COLS, j = tid % COLS;
+                float u = cobs[tid] + btv;
+#pragma unroll
+                for (int wr = 0; wr < 16; ++wr) u += red[(wr * R + r) * COLS + j];
+                uown[tid] = u;
+                const float v = fmaxf(u, 0.f);
+#pragma unroll 1
+                for (int dst = 0; dst < CS_C; ++dst) cluster.map_shared_rank(actA, dst)[r * LDA + col0 + j] = v;
+            }
+            cluster.sync();    // relu(u) of all H columns is in every CTA's actA
+            // ---- L1 slice: h1[:, cols] = relu(u) @ W1[:, cols] + b1; this warp's k-rows warp * KPW .. + KPW, the first KRW resident
+            {
+                float acc[RH][NC];
+#pragma unroll
+                for (int rr = 0; rr < RH; ++rr)
+#pragma unroll
+                    for (int m = 0; m < NC; ++m) acc[rr][m] = 0.f;
+                const float* ap = actA + half * LDA + warp * KPW;
+                const float* Ws = W1s + warp * KRW * COLS + c16;
+#pragma unroll 4
+                for (int kk = 0; kk < KRW; kk += 4) {
+                    float wv[4][NC];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+#pragma unroll
+                        for (int m = 0; m < NC; ++m) wv[q][m] = Ws[(kk + q) * COLS + 16 * m];
+#pragma unroll
+                    for (int rr = 0; rr < RH; ++rr) {
+                        const float4 a = *reinterpret_cast<const float4*>(ap + 2 * rr * LDA + kk);
+#pragma unroll
+                        for (int m = 0; m < NC; ++m) {
+                            acc[rr][m] = fmaf(a.x, wv[0][m], acc[rr][m]); acc[rr][m] = fmaf(a.y, wv[1][m], acc[rr][m]);
+                            acc[rr][m] = fmaf(a.z, wv[2][m], acc[rr][m]); acc[rr][m] = fmaf(a.w, wv[3][m], acc[rr][m]);
+                        }
+                    }
+                }
+                const float* Wg = w + p.o.w1 + (size_t)(warp * KPW) * H + col0 + c16;
+#pragma unroll 2
+                for (int kk = KRW; kk < KPW; kk += 4) {
+                    float wv[4][NC];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+#pragma unroll
+                        for (int m = 0; m < NC; ++m) wv[q][m] = __ldg(Wg + (size_t)(kk + q) * H + 16 * m);
+#pragma unroll
+                    for (int rr = 0; rr < RH; ++rr) {
+                        const float4 a = *reinterpret_cast<const float4*>(ap + 2 * rr * LDA + kk);
+#pragma unroll
+                        for (int m = 0; m < NC; ++m) {
+                            acc[rr][m] = fmaf(a.x, wv[0][m], acc[rr][m]); acc[rr][m] = fmaf(a.y, wv[1][m], acc[rr][m]);
+                            acc[rr][m] = fmaf(a.z, wv[2][m], acc[rr][m]); acc[rr][m] = fmaf(a.w, wv[3][m], acc[rr][m]);
+                        }
+                    }
+                }
+#pragma unroll
+                for (int rr = 0; rr < RH; ++rr)
+#pragma unroll
+                    for (int m = 0; m < NC; ++m) red[(warp * R + 2 * rr + half) * COLS + c16 + 16 * m] = acc[rr][m];
+            }
+            __syncthreads();
+            if (tid < R * COLS) {
+                const int r = tid / COLS, j = tid % COLS;
+                float s = b1s[j];
+#pragma unroll
+                for (int wr = 0; wr < 16; ++wr) s += red[(wr * R + r) * COLS + j];
+                out1[tid] = fmaxf(s, 0.f);
+            }
+            __syncthreads();
+            // ---- partial output layer over this CTA's columns, written straight into the 16 CTAs' partial buffers
+#pragma unroll
+            for (int q = 0; q < NE; ++q) {
+                const int e = tid + q * CS_THREADS;
+                if (e < R * AP) {
+                    const int r = e / AP, a = e % AP;
+                    float s = 0.f;
+#pragma unroll 16
+                    for (int k = 0; k < COLS; ++k) s = fmaf(out1[r * COLS + k], W23s[k * AP + a], s);
+                    float s2 = 0.f;
+#pragma unroll 16
+                    for (int k = 0; k < COLS; ++k) s2 = fmaf(uown[r * COLS + k], W3s[k * AP + a], s2);
+                    s += s2;
+#pragma unroll 1
+                    for (int dst = 0; dst < CS_C; ++dst) cluster.map_shared_rank(part, dst)[crank * (R * AP) + e] = s;
+                }
+            }
+            cluster.sync();
+            // ---- posterior mean / clipped noise / x update (identical in all 16 CTAs)
+#pragma unroll
+            for (int q = 0; q < NE; ++q) {
+                const int e = tid + q * CS_THREADS;
+                if (e < R * AP) {
+                    const int r = e / AP, a = e % AP;
+                    if (a < A && row0 + r < B) {
+                        float ev = b3s[a];
+#pragma unroll
+                        for (int src = 0; src < CS_C; ++src) ev += part[src * (R * AP) + e];
+                        const int64_t row = row0 + r;
+                        const float xn = ddpm_step_elem(xs[e], ev, nz[q], t, p.sch, T, p.hp, t == 0);
+                        xs[e] = xn;
+                        if (crank == 0) {
+                            if (p.chains && t <= K) p.chains[((size_t)row * (K + 1) + (K - t)) * A + a] = xn;
+                            if (t == 0) {
+                                p.actions[(size_t)row * A + a] = xn;
+                                if (p.raw_actions && a < p.act_cols)
+                                    p.raw_actions[(size_t)row * p.act_cols + a] = env_unnormalize_action(xn, p.act_min[a % p.Da], p.act_max[a % p.Da]);
+                            }
+                        }
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    // no CTA may exit while peers can still write into its shared memory
+    cluster.sync();
+}

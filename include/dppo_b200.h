@@ -254,8 +254,9 @@ int64_t dppo_tc_launch_count(dppo_handle* h);
 /* Of those, launches of the fused layer-chain kernel (whole MLP forward / backward / T-step sampler per launch). */
 int64_t dppo_fused_launch_count(dppo_handle* h);
 /* Which sampler the last dppo_sample used: 1 = persistent cluster kernel (one launch, T steps on
- * chip, fp32 FFMA), 2 = layer-by-layer fp32, 3 = layer-by-layer tcgen05, 4 = fused tcgen05 chain
- * (one launch, T steps on chip).  Test / bench introspection. */
+ * chip, fp32 FFMA; ReLU actors of width 256, 512, 768 or 1024 with chunks A <= 128 - other widths,
+ * a Mish actor and wider chunks take 2), 2 = layer-by-layer fp32, 3 = layer-by-layer tcgen05,
+ * 4 = fused tcgen05 chain (one launch, T steps on chip).  Test / bench introspection. */
 int dppo_last_path(dppo_handle* h);
 /* Test hook: 0 = automatic dispatch, 1 = force the cluster sampler, 2 = forbid it,
  * 3 = forbid the fused tcgen05 chain (the tensor path then runs one GEMM launch per layer). */

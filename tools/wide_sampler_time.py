@@ -1,12 +1,14 @@
-"""What the small-batch rollout sampler costs for wide action chunks: the persistent cluster kernel (path 1) against the
-layer-by-layer fp32 sampler (path 2, forced), alternating block by block, at A = horizon_steps x action_dim in {24, 56, 112, 128}
-(walker2d's chunk, robomimic-transport-sized ones, the widest the cluster kernel covers), H = 512, T = 20, K = 10:
+"""What the small-batch rollout sampler costs for wide action chunks and other actor widths: the persistent cluster kernel
+(path 1) against the layer-by-layer fp32 sampler (path 2, forced), alternating block by block, at A = horizon_steps x action_dim
+in {24, 56, 112, 128} (walker2d's chunk, robomimic-transport-sized ones, the widest the cluster kernel covers) and actor width
+H = 512 by default, T = 20, K = 10:
   * `sample` and `rollout_step` (normalise kernel + sampler with the un-normalising epilogue) for B in {40, 50} env rows
     (the gym configs' n_envs, robomimic's), in the fp32 and bf16x3 modes (below 2048 rows both sample with the same fp32 kernels);
   * `sample` in the fp32 mode for B up to 4096 rows (dppo_sample's row limit for the cluster path), where the layered path's
     SGEMM tiles fill up.
 Median and min of 7 timed blocks of 20 calls (CUDA events), after warm-up; the card's name and power limit are printed with them.
-    python tools/wide_sampler_time.py [output.json]"""
+    python tools/wide_sampler_time.py [output.json] [--widths 256,768,1024] [--chunks 24,56,128]"""
+import argparse
 import json
 import os
 import subprocess
@@ -60,21 +62,28 @@ def alternate(e, fn, iters):
 
 
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("output", nargs="?")
+    ap.add_argument("--widths", default="512", help="actor hidden widths, comma-separated")
+    ap.add_argument("--chunks", default=",".join(str(a) for a in SHAPES), help="chunk widths A, comma-separated")
+    args = ap.parse_args()
+    widths = [int(v) for v in args.widths.split(",")]
+    chunks = [int(v) for v in args.chunks.split(",")]
     if not torch.cuda.is_available():
         sys.exit("wide_sampler_time.py: no CUDA device")
     out = {"card": card(), "iters": ITERS, "blocks": BLOCKS, "results": []}
     print(f"card, power limit: {out['card']}", flush=True)
 
-    def report(A, mode, call, B, r, T):
+    def report(H, A, mode, call, B, r, T):
         (c_med, c_min), (l_med, l_min) = r[1], r[2]
-        row = dict(A=A, mode=mode, call=call, B=B, cluster_med_us=c_med, cluster_min_us=c_min, layered_med_us=l_med,
+        row = dict(H=H, A=A, mode=mode, call=call, B=B, cluster_med_us=c_med, cluster_min_us=c_min, layered_med_us=l_med,
                    layered_min_us=l_min, speedup=l_med / c_med, cluster_us_per_denoising_step=c_med / T)
         out["results"].append(row)
-        print(f"A={A:3d} {mode:6s} {call:12s} B={B:4d}: cluster {c_med:8.1f} us (min {c_min:8.1f})  layered {l_med:8.1f} us "
+        print(f"H={H:4d} A={A:3d} {mode:6s} {call:12s} B={B:4d}: cluster {c_med:8.1f} us (min {c_min:8.1f})  layered {l_med:8.1f} us "
               f"(min {l_min:8.1f})  speed-up {l_med / c_med:5.2f}x  cluster per denoising step {c_med / T:5.2f} us", flush=True)
 
-    for A, dims in SHAPES.items():
-        o = O.make_oracle("hopper", seed=0, **dims)
+    for H, A in [(H, A) for H in widths for A in chunks]:
+        o = O.make_oracle("hopper", seed=0, actor_hidden=H, **SHAPES[A])
         d, T = o.d, o.d.denoising_steps
         for mode, prec in MODES.items():
             e = make_engine(o, prec)
@@ -87,16 +96,16 @@ def main():
             for B in ENVS + (SWEEP if mode == "fp32" else ()):
                 obs, act, ch = obs_all[:B], act_all[:B], ch_all[:B]
                 r = alternate(e, lambda: e.sample(obs, seed=1, offset=2, actions_out=act, chains_out=ch), ITERS if B <= 1024 else 5)
-                report(A, mode, "sample", B, r, T)
+                report(H, A, mode, "sample", B, r, T)
                 if B in ENVS:
                     raw_obs = torch.from_numpy(rng.uniform(-2, 3, (B, d.obs_dim))).pin_memory()
                     raw_act = torch.zeros(B, d.action_dim).pin_memory()
                     obs_out = torch.empty(B, d.obs_dim, device="cuda")
                     r = alternate(e, lambda: e.rollout_step(raw_obs, obs_out, act, ch, raw_act, 1, seed=1, offset=2), ITERS)
-                    report(A, mode, "rollout_step", B, r, T)
+                    report(H, A, mode, "rollout_step", B, r, T)
             e.close()
-    if len(sys.argv) > 1:
-        with open(sys.argv[1], "w") as f:
+    if args.output:
+        with open(args.output, "w") as f:
             json.dump(out, f, indent=1)
 
 
