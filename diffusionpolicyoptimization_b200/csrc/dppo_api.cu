@@ -79,12 +79,17 @@ extern "C" int dppo_ddpm_schedule(int T, float* out) {
 }
 
 // ------------------------------------------------------------------ geometry
+// the accepted configurations (include/dppo_b200.h); a refusal leaves its reason in dppo_last_error
 static int make_geom(const dppo_cfg* c, Geom* g) {
-    if (c->obs_dim < 1 || c->action_dim < 1 || c->horizon_steps < 1 || c->cond_steps < 1) return -1;
-    if (c->denoising_steps < 1 || c->denoising_steps > 255 || c->ft_denoising_steps < 0 || c->ft_denoising_steps > c->denoising_steps) return -1;
-    if (c->time_dim < 4 || (c->time_dim & 1) || c->time_dim > 64) return -1;
-    if (c->actor_hidden < 16 || c->actor_hidden > 1024 || c->critic_hidden < 16 || c->critic_hidden > 1024) return -1;
-    if ((c->actor_hidden % 4) || (c->critic_hidden % 4)) return -1;
+    if (c->obs_dim < 1 || c->action_dim < 1 || c->horizon_steps < 1 || c->cond_steps < 1) DPPO_FAIL(-1, "obs_dim, action_dim, horizon_steps and cond_steps must be >= 1");
+    if (c->denoising_steps < 1 || c->denoising_steps > 255 || c->ft_denoising_steps < 0 || c->ft_denoising_steps > c->denoising_steps)
+        DPPO_FAIL(-1, "denoising_steps must be in [1, 255] and ft_denoising_steps in [0, denoising_steps] (got %d, %d)", c->denoising_steps, c->ft_denoising_steps);
+    if (c->time_dim < 4 || (c->time_dim & 1) || c->time_dim > 64) DPPO_FAIL(-1, "time_dim must be even and in [4, 64] (got %d)", c->time_dim);
+    // the time-embedding backward keeps 5 T time_dim floats in shared memory (time_backward_smem): at most 160 KB
+    if (c->denoising_steps * c->time_dim > 8192)
+        DPPO_FAIL(-1, "denoising_steps x time_dim must be <= 8192 (got %d x %d)", c->denoising_steps, c->time_dim);
+    if (c->actor_hidden < 16 || c->actor_hidden > 1024 || c->critic_hidden < 16 || c->critic_hidden > 1024 || (c->actor_hidden % 4) || (c->critic_hidden % 4))
+        DPPO_FAIL(-1, "actor_hidden and critic_hidden must be multiples of 4 in [16, 1024] (got %d, %d)", c->actor_hidden, c->critic_hidden);
     g->Do = c->obs_dim * c->cond_steps; g->A = c->action_dim * c->horizon_steps;
     g->T = c->denoising_steps; g->K = c->ft_denoising_steps; g->td = c->time_dim;
     g->H = c->actor_hidden; g->Hc = c->critic_hidden;
@@ -251,7 +256,7 @@ extern "C" int dppo_create(const dppo_cfg* cfg, int device, dppo_handle** out) {
 }
 static int dppo_create_impl(const dppo_cfg* cfg, int device, dppo_handle** out, dppo_handle** partial) {
     Geom g;
-    if (make_geom(cfg, &g)) DPPO_FAIL(-1, "dppo_create: invalid configuration");
+    if (make_geom(cfg, &g)) { const std::string why = dppo_last_error(); DPPO_FAIL(-1, "dppo_create: invalid configuration: %s", why.c_str()); }
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0) DPPO_FAIL(-4, "dppo_create: no CUDA device (%s); this library has no CPU fallback", cudaGetErrorString(e));
@@ -438,12 +443,14 @@ static int colsum(dppo_handle* h, cudaStream_t s, const float* D, int ld, int N,
                   float* part, float* out) {
     int nb = (N + 127) / 128; if (nb > 320) nb = 320; if (nb < 1) nb = 1;
     int rpb = (N + nb - 1) / nb; nb = (N + rpb - 1) / rpb;
-    size_t sm = (size_t)nseg * ncols * sizeof(float);
-    if (sm > 48 * 1024) {
-        if (sm > 200 * 1024) DPPO_FAIL(-1, "colsum: %d segments x %d columns does not fit in shared memory", nseg, ncols);
-        CUDA_TRY(cudaFuncSetAttribute(colsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    }
-    colsum_kernel<<<nb, 256, sm, s>>>(D, ld, N, ncols, seg, nseg, rpb, part); KLAUNCH(h); KCHECK();
+    // a block sums a slice of the columns for every segment: [nseg][slice] in shared memory, at most 200 KB (T = 255 segments of
+    // H = 1024 columns are 1 MB: four or more slices, blockIdx.y)
+    const int max_cols = (int)((200 * 1024) / ((size_t)nseg * sizeof(float)));
+    if (max_cols < 1) DPPO_FAIL(-1, "colsum: %d segments do not fit in shared memory", nseg);
+    const int nslice = (ncols + max_cols - 1) / max_cols, slice = (ncols + nslice - 1) / nslice;
+    size_t sm = (size_t)nseg * slice * sizeof(float);
+    if (sm > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(colsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    colsum_kernel<<<dim3(nb, nslice), 256, sm, s>>>(D, ld, N, ncols, slice, seg, nseg, rpb, part); KLAUNCH(h); KCHECK();
     size_t n = (size_t)nseg * ncols;
     tc_reduce_cols_kernel<<<nblk(n, 8), 256, 0, s>>>(part, nb, n, (int)n, out); KLAUNCH(h); KCHECK();
     return 0;

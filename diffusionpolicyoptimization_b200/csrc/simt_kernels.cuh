@@ -667,23 +667,26 @@ __global__ void sum_blocks_kernel(const double* __restrict__ block_sums, int nbl
 // =====================================================================================
 // Column sums (bias gradients) and per-t column sums (time-embedding gradient)
 //   part[blk][seg][n] = sum over this block's rows with seg(row)==seg of D[row][n]
+// Block (x, y) takes row block x and the columns [y * slice, (y + 1) * slice) of every segment (shared memory [nseg][slice]).
 // =====================================================================================
-__global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ D, int ld, int N, int ncols,
+__global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ D, int ld, int N, int ncols, int slice,
                                                      const int* __restrict__ seg, int nseg, int rows_per_block,
                                                      float* __restrict__ part) {
-    extern __shared__ float sm[];   // [nseg][ncols]
-    for (int i = threadIdx.x; i < nseg * ncols; i += blockDim.x) sm[i] = 0.f;
+    extern __shared__ float sm[];   // [nseg][slice]
+    const int c0 = blockIdx.y * slice, nc = min(slice, ncols - c0);
+    for (int i = threadIdx.x; i < nseg * slice; i += blockDim.x) sm[i] = 0.f;
     __syncthreads();
     const int r0 = blockIdx.x * rows_per_block, r1 = min(N, r0 + rows_per_block);
-    // each thread owns columns c = tid, tid+256, ... and walks the rows: no atomics needed
-    for (int c = threadIdx.x; c < ncols; c += blockDim.x) {
+    // each thread owns columns c = tid, tid+256, ... of the slice and walks the rows: no atomics needed
+    for (int c = threadIdx.x; c < nc; c += blockDim.x) {
         for (int r = r0; r < r1; ++r) {
             int s = seg ? seg[r] : 0;
-            sm[s * ncols + c] += D[(size_t)r * ld + c];
+            sm[s * slice + c] += D[(size_t)r * ld + c0 + c];
         }
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < nseg * ncols; i += blockDim.x) part[(size_t)blockIdx.x * nseg * ncols + i] = sm[i];
+    float* out = part + (size_t)blockIdx.x * nseg * ncols + c0;
+    for (int i = threadIdx.x; i < nseg * nc; i += blockDim.x) out[(size_t)(i / nc) * ncols + i % nc] = sm[(i / nc) * slice + i % nc];
 }
 
 // time-MLP + layer-0 bias backward from G[T][H] = per-t column sums of du, on time_backward_grid() blocks of 512 threads
@@ -807,13 +810,14 @@ static inline int time_backward_grid(const Geom& g) { return g.T + (g.H + 31) / 
 static inline size_t time_backward_smem(const Geom& g) { return (size_t)5 * g.T * g.td * sizeof(float); }
 // the time-MLP / layer-0 bias backward of actor `net` from G [T][H] into its gradient slice gnet
 static cudaError_t launch_time_backward(const dppo_handle* h, cudaStream_t s, int net, const float* G, float* gnet) {
-    static bool attr_set_dev[64] = {};
+    // the attribute is per device and shared by every handle on it: raised whenever a handle needs more than is set
+    static size_t attr_dev[64] = {};
     const Geom& g = h->g; const ActorDerived& d = h->ad[net];
     const size_t sm = time_backward_smem(g);
-    if (sm > 48 * 1024 && !attr_set_dev[h->device & 63]) {
+    if (sm > 48 * 1024 && sm > attr_dev[h->device & 63]) {
         const cudaError_t e = cudaFuncSetAttribute(time_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         if (e != cudaSuccess) return e;
-        attr_set_dev[h->device & 63] = true;
+        attr_dev[h->device & 63] = sm;
     }
     time_backward_kernel<<<time_backward_grid(g), 512, sm, s>>>(h->net_w[net], g.ao, g.A, g.td, g.H, g.T, G, d.sinemb, d.thpre, d.temb, d.dte, gnet);
     return cudaGetLastError();

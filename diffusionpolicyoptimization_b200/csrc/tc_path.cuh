@@ -164,27 +164,32 @@ __global__ void tc_pad64_kernel(const float* __restrict__ src, int N, int ncols,
     for (int j = 0; j < 8; ++j) o[j] = __float2bfloat16(k0 + j < ncols ? src[(size_t)r * ncols + k0 + j] : 0.f);
     *reinterpret_cast<uint4*>(dst + (size_t)r * 64 + k0) = *reinterpret_cast<const uint4*>(o);
 }
-// column sums of a bf16 matrix D[N][ncols] (ncols even, ncols/2 <= 256): part[blk][ncols]
+// column sums of a bf16 matrix D[N][ncols] (ncols even): part[blk][ncols].  Up to 512 columns one pass, `groups` row groups of
+// ncols / 2 threads (a thread per column pair); wider matrices take passes of 256 column pairs, one row group.
 __global__ void __launch_bounds__(256) tc_colsum_kernel(const bf16* __restrict__ D, int N, int ncols, int rows_per_block, float* __restrict__ part) {
     __shared__ float2 red[256];
-    const int tpr = ncols / 2, groups = 256 / tpr;
+    const int npair = ncols / 2, tpr = npair < 256 ? npair : 256, groups = 256 / tpr;
     const int cg = threadIdx.x % tpr, rg = threadIdx.x / tpr;
     const int r0 = blockIdx.x * rows_per_block, r1 = min(N, r0 + rows_per_block);
-    float2 acc = make_float2(0.f, 0.f);
-    if (rg < groups) {
-        for (int r = r0 + rg; r < r1; r += groups) {
-            __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(D + (size_t)r * ncols + 2 * cg);
-            float2 f = __bfloat1622float2(v);
-            acc.x += f.x; acc.y += f.y;
+    for (int p0 = 0; p0 < npair; p0 += tpr) {
+        const int p = p0 + cg;
+        float2 acc = make_float2(0.f, 0.f);
+        if (rg < groups && p < npair) {
+            for (int r = r0 + rg; r < r1; r += groups) {
+                __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(D + (size_t)r * ncols + 2 * p);
+                float2 f = __bfloat1622float2(v);
+                acc.x += f.x; acc.y += f.y;
+            }
         }
-    }
-    red[threadIdx.x] = acc;
-    __syncthreads();
-    if (threadIdx.x < tpr) {
-        float2 s = red[threadIdx.x];
-        for (int g = 1; g < groups; ++g) { float2 o = red[g * tpr + threadIdx.x]; s.x += o.x; s.y += o.y; }
-        part[(size_t)blockIdx.x * ncols + 2 * threadIdx.x] = s.x;
-        part[(size_t)blockIdx.x * ncols + 2 * threadIdx.x + 1] = s.y;
+        red[threadIdx.x] = acc;
+        __syncthreads();
+        if (threadIdx.x < tpr && p < npair) {
+            float2 s = red[threadIdx.x];
+            for (int g = 1; g < groups; ++g) { float2 o = red[g * tpr + threadIdx.x]; s.x += o.x; s.y += o.y; }
+            part[(size_t)blockIdx.x * ncols + 2 * p] = s.x;
+            part[(size_t)blockIdx.x * ncols + 2 * p + 1] = s.y;
+        }
+        __syncthreads();
     }
 }
 // out[r][c] = sum_s part[s*stride + r*ld_in + c]   for r < rows, c < cols   (deterministic split-K reduction)

@@ -1253,6 +1253,7 @@ static int ts_alloc_w(TsW& w, size_t n) {
     w.p[1] = w.p[0] + n; w.p[2] = nullptr;
     return 0;
 }
+static bool ts_dw3_fits(const Geom& g);
 static int ts_init(dppo_handle* h) {
     if (h->cfg.precision != DPPO_PREC_BF16X3) return 0;
     const Geom& g = h->g;
@@ -1260,7 +1261,8 @@ static int ts_init(dppo_handle* h) {
     memset(st, 0, sizeof(*st));
     h->ts = st;
     st->KP0 = round_up(g.A + g.Do + g.T + 1, 64);
-    if ((g.H % 64) || (g.Hc % 64) || g.A > 128) return 0;    // shapes this path does not cover: stays on FFMA
+    // shapes this path does not cover (the widths of the plane GEMMs, the output-layer gradient assembly): stays on FFMA
+    if ((g.H % 64) || (g.Hc % 64) || !ts_dw3_fits(g)) return 0;
     for (int net = 0; net < 4; ++net) {
         TsNetW& w = st->net[net];
         const size_t H = net == DPPO_NET_CRITIC ? g.Hc : g.H;
@@ -1786,6 +1788,24 @@ __global__ void __launch_bounds__(512) ts_dw3_assemble_kernel(const TsDw3Args fa
     if (b < rank_c) ts_rank_rows_body(fc, b, dw3_sm, rc0, rc1);
 }
 static inline int tsDW3KS() { return DW3_KS; }
+// the assembly's k slice of one net (rows of [W2 ; layer-0 rows] per block) and its dynamic shared memory: the larger of the dW3 body's
+// [kper][NO] + [16][32][NC] and the rank-rows body's [DW3_RB][NO] + [H][N3 + 1] (WIDE, NO > 32: NC = DW3_WC, N3 = 32)
+static int ts_dw3_kper(const Geom& g, int H) { return (H + g.A + g.Do + g.T + DW3_KS - 1) / DW3_KS; }
+static size_t ts_dw3_net_smem(const Geom& g, int H, int NO) {
+    const bool w = NO > 32;
+    const int nc = w ? DW3_WC : NO, n3 = w ? 32 : NO;
+    const size_t a = (size_t)ts_dw3_kper(g, H) * NO + 16 * 32 * nc, b = (size_t)DW3_RB * NO + (size_t)H * (n3 + 1);
+    return (a > b ? a : b) * sizeof(float);
+}
+static size_t ts_dw3_smem(const Geom& g) {
+    const size_t a = ts_dw3_net_smem(g, g.H, g.A), c = ts_dw3_net_smem(g, g.Hc, 1);
+    return a > c ? a : c;
+}
+// the shapes the assembly covers, for ts_init (a handle outside them runs this mode on FFMA) and the launch: a block's 16 warps hold
+// at most 8 k rows each, shared memory up to 100 KB.  (The 256 chunk counters cover any accepted width: H, Hc <= 1024.)
+static bool ts_dw3_fits(const Geom& g) {
+    return g.A <= 128 && ts_dw3_kper(g, g.H) <= 128 && ts_dw3_kper(g, g.Hc) <= 128 && ts_dw3_smem(g) <= 100 * 1024;
+}
 // gnet: this net's slice of the flat gradient; dw0: its [KP0][H] layer-0 staging buffer
 static TsDw3Args ts_dw3_args(const dppo_handle* h, int net, const float* g1, const float* g0, float* gnet, float* dw0) {
     const Geom& g = h->g; const float* w = h->net_w[net];
@@ -1821,23 +1841,16 @@ static int ts_dw3_assemble(dppo_handle* h, cudaStream_t s, int actor_net, const 
     }
     const int nba = tc_nblk((size_t)g.H, 32) * tsDW3KS();
     const bool wide = fa.NO > 32;
-    auto smf = [&](const TsDw3Args& f, bool w) {
-        const int K = f.H + f.A + f.Do + f.T, nc = w ? DW3_WC : f.NO, n3 = w ? 32 : f.NO;
-        const size_t a = (size_t)(((K + DW3_KS - 1) / DW3_KS) * f.NO + 16 * 32 * nc), b = (size_t)(DW3_RB * f.NO + f.H * (n3 + 1));
-        return (a > b ? a : b) * sizeof(float);
-    };
-    auto kper = [&](const TsDw3Args& f) { return (f.H + f.A + f.Do + f.T + DW3_KS - 1) / DW3_KS; };
-    // (without the critic fc is a copy of fa: size it as the actor)
-    const size_t sm = smf(fa, wide) > smf(fc, fc.NO > 32) ? smf(fa, wide) : smf(fc, fc.NO > 32);
+    // (sized for both nets also when the critic is absent)
+    const size_t sm = ts_dw3_smem(g);
     auto kern = wide ? ts_dw3_assemble_kernel<true> : ts_dw3_assemble_kernel<false>;
     static bool attr_set_dev[2][64] = {};
     if (!attr_set_dev[wide][h->device & 63]) { CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024)); attr_set_dev[wide][h->device & 63] = true; }
-    if (sm > 100 * 1024 || g.A > 128 || kper(fa) > 128 || kper(fc) > 128) DPPO_FAIL(-7, "ts_dw3_assemble: shape not covered");
+    if (!ts_dw3_fits(g)) DPPO_FAIL(-7, "ts_dw3_assemble: shape not covered (ts_init routes it to FFMA)");
     TsState* st = h->ts;
     // buffer: [256 chunk counters (always at the front: launches with and without the critic share them, every launch leaves them zero)
     //          | partial tiles]
     const size_t need = 1024 + ((size_t)nba * 32 * g.A + (size_t)nbc * 32) * sizeof(float);
-    if ((nba + nbc) / DW3_KS > 256) DPPO_FAIL(-7, "ts_dw3_assemble: too many column chunks");
     if (st->dw3_bytes < need) {
         CUDA_TRY(cudaStreamSynchronize(s));
         if (st->dw3_buf) cudaFree(st->dw3_buf);

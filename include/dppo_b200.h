@@ -54,7 +54,11 @@ enum { DPPO_OPT_PRETRAIN = 0 /* actor */, DPPO_OPT_FINETUNE = 1 /* actor_ft ++ c
 
 /* Hyper-parameters = cfg.model.* / cfg.train.* of cfg/gym/finetune/hopper-v2/ft_ppo_diffusion_mlp.yaml
  * and cfg/gym/pretrain/hopper-medium-v2/pre_diffusion_mlp.yaml.  dppo_cfg_default() fills the
- * hopper fine-tune values. */
+ * hopper fine-tune values.
+ * Accepted shapes (dppo_create refuses any other, naming the limit; dppo_num_params returns 0 for it):
+ *   obs_dim, action_dim, horizon_steps, cond_steps >= 1;  1 <= denoising_steps <= 255;  0 <= ft_denoising_steps <= denoising_steps;
+ *   time_dim even, 4 ... 64;  denoising_steps * time_dim <= 8192 (the time-embedding backward keeps 5 T time_dim floats in
+ *   shared memory: 160 KB);  actor_hidden, critic_hidden multiples of 4, 16 ... 1024. */
 typedef struct dppo_cfg {
     int32_t obs_dim, action_dim, horizon_steps, cond_steps;   /* yaml:16-22                        */
     int32_t denoising_steps, ft_denoising_steps;              /* yaml:18-19                        */
