@@ -212,6 +212,12 @@ struct dppo_handle {
     double prof_exec[4] = {0, 0, 0, 0};   // flops the tensor pipe executed (plane modes issue 3 or 6 products per algorithmic multiply-add)
 };
 
+// Every weight change of a net (set_weights, an applied PPO or pre-training step, ema_update, a skipped update) calls this: it marks
+// every lazily rebuilt table of that net stale - w0p, w23 / b23 and the split-precision folded layers - so that the next reader
+// rebuilds it.  The eagerly rebuilt copies (time tables, bf16 / plane operands) are rewritten by the same call that changed the
+// weights.  A lazy table added later is listed here, once.
+static void mark_weights_changed(dppo_handle* h, int net);
+
 // profile bracket: call prof_begin before and prof_end after a GEMM-class launch
 void prof_begin(dppo_handle* h, cudaStream_t s);
 void prof_end(dppo_handle* h, cudaStream_t s, double flops, int cls, double exec_flops = -1.0);   // exec_flops: tensor-pipe flops actually issued (default: = flops)

@@ -232,7 +232,7 @@ static int ensure_w0p(dppo_handle* h, int net, cudaStream_t s) {
 }
 static int prep_net(dppo_handle* h, int net, cudaStream_t s) {
     const Geom& g = h->g;
-    h->w0p_dirty[net] = 1; h->w23_dirty[net] = 1;
+    mark_weights_changed(h, net);
     if (net != DPPO_NET_CRITIC) {
         ActorDerived& d = h->ad[net];
         int threads = g.H < 64 ? 64 : (g.H > 512 ? 512 : round_up(g.H, 32));

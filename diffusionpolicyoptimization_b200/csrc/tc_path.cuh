@@ -545,7 +545,7 @@ static int tc_prep_pack_ft_critic(dppo_handle* h, cudaStream_t s) {
     a.sinemb = d.sinemb; a.thpre = d.thpre; a.temb = d.temb; a.bt = d.bt;
     a.a_w2w0 = wa.w2w0; a.a_w1 = wa.w1; a.a_w3t = wa.w3t; a.a_w3p = wa.w3p; a.a_w1t = wa.w1t; a.a_w2t = wa.w2t;
     a.c_w2w0 = wc.w2w0; a.c_w1 = wc.w1; a.c_w3t = wc.w3t; a.c_w3p = wc.w3p; a.c_w1t = wc.w1t; a.c_w2t = wc.w2t; a.c_bias2 = wc.bias2;
-    h->w0p_dirty[DPPO_NET_ACTOR_FT] = 1; h->w0p_dirty[DPPO_NET_CRITIC] = 1;
+    mark_weights_changed(h, DPPO_NET_ACTOR_FT); mark_weights_changed(h, DPPO_NET_CRITIC);
     tc_prep_pack_kernel<<<g.T + a.na + a.nc, 256, 4 * g.td * sizeof(float), s>>>(a);
     h->launches++;
     cudaError_t e = cudaGetLastError();

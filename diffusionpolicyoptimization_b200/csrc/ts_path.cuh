@@ -1071,6 +1071,11 @@ struct TsState { TsNetW net[4]; int KP0; int fold_dirty[4]; char* dw3_buf; size_
 // outputs; an actor with a wider action chunk (up to 128) takes 128.  The critic (one output) keeps 64.
 static inline int ts_nop(int NO) { return NO <= 32 ? 64 : 128; }
 
+static void mark_weights_changed(dppo_handle* h, int net) {
+    h->w0p_dirty[net] = 1; h->w23_dirty[net] = 1;
+    if (h->ts) h->ts->fold_dirty[net] = 1;
+}
+
 __device__ __forceinline__ void ts_put(const TsW& W, size_t i, float v) {
     bf16 a, b; ts::split_bf16(v, a, b);
     W.p[0][i] = a; W.p[1][i] = b;
@@ -1286,7 +1291,6 @@ static void ts_destroy(dppo_handle* h) {
 static int ts_refresh_net(dppo_handle* h, int net, cudaStream_t s) {
     if (h->cfg.precision != DPPO_PREC_BF16X3 || !ts_shapes_ok(h)) return 0;
     const Geom& g = h->g; const TsNetW& w = h->ts->net[net];
-    h->ts->fold_dirty[net] = 1;
     if (net == DPPO_NET_CRITIC) ts_pack_critic_kernel<<<128, 256, 0, s>>>(h->net_w[net], g.co, g.A, g.Do, g.Hc, h->ts->KP0, w);
     else ts_pack_actor_kernel<<<256, 256, 0, s>>>(h->net_w[net], g.ao, g.A, g.td, g.Do, g.T, g.H, h->ts->KP0, h->ad[net].bt, w);
     TC_KCHECK(h);
@@ -1413,7 +1417,7 @@ static int ts_apply_update(dppo_handle* h, cudaStream_t s, const float* g, float
     a.sinemb = d.sinemb; a.thpre = d.thpre; a.temb = d.temb; a.bt = d.bt;
     a.done = reinterpret_cast<int*>(d.dte + (size_t)gm.T * gm.td) + 1;
     CUDA_TRY(launch_pdl(ts_update_kernel, dim3(a.elem_blocks + gm.T), dim3(512), ts_update_smem(gm), s, a)); TC_KCHECK(h);
-    for (int net : {DPPO_NET_ACTOR_FT, DPPO_NET_CRITIC}) { h->w0p_dirty[net] = 1; h->w23_dirty[net] = 1; h->ts->fold_dirty[net] = 1; }
+    mark_weights_changed(h, DPPO_NET_ACTOR_FT); mark_weights_changed(h, DPPO_NET_CRITIC);
     // the folded output layers of the new weights, here rather than lazily at the next update's start: there they ran on the second
     // stream but got SMs only when the actor's persistent L1 drained, and the actor's folded GEMM waited for them
     DPPO_TRY(ts_ensure_fold(h, DPPO_NET_ACTOR_FT, s)); DPPO_TRY(ts_ensure_fold(h, DPPO_NET_CRITIC, s));

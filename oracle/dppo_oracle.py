@@ -210,7 +210,7 @@ def residual_mlp(p: Sequence[torch.Tensor], x: torch.Tensor, act) -> torch.Tenso
 def time_embedding(p: Sequence[torch.Tensor], t: torch.Tensor, time_dim: int) -> torch.Tensor:
     """mlp_diffusion.py:40-45: SinusoidalPosEmb -> Dense(2*td, mish) -> Dense(td)."""
     tw1, tb1, tw2, tb2 = p
-    e = sinusoidal_pos_emb(t, time_dim)
+    e = sinusoidal_pos_emb(t, time_dim).to(tw1.dtype)       # float64 parameters evaluate the whole net in float64
     return mish(e @ tw1 + tb1) @ tw2 + tb2
 
 
